@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--precision fp32|bf16|bf16x3|bf16x6] [--utterances U]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): the default framewise conv model
 (80 mels, 6 layers, sum pooling at the intermediate location, random init)
@@ -67,7 +68,11 @@ def kernel_metrics():
 def parse_args():
     parser = argparse.ArgumentParser()
     parser.add_argument('--gpus', type=int, default=1)
-    parser.add_argument('--steps', type=int, default=20)
+    parser.add_argument(
+        '--steps', type=int, default=20,
+        help='timed steps of the headline kernel-only loop (the value, ms_per_step and '
+             '--dump-outputs); the pinned-host end-to-end legs run max(3, min(K, 10)), '
+             'the other legs their own fixed or --transformer-steps counts')
     parser.add_argument('--warmup', type=int, default=3)
     parser.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     parser.add_argument(
@@ -89,7 +94,17 @@ def parse_args():
     parser.add_argument(
         '--no-list-api', dest='list_api', action='store_false',
         help='skip the list-of-tensors end-to-end leg')
-    return parser.parse_args()
+    parser.add_argument(
+        '--dump-outputs', metavar='DIR',
+        help='after the timed steps, write the word scores and logits of the last '
+             'timed step as DIR/scores.npy and DIR/logits.npy (float32, one value '
+             'per word in corpus order; rank r of N > 1 writes scores.rank<r>.npy)')
+    args = parser.parse_args()
+    if args.steps < 1:
+        parser.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        parser.error('--dump-outputs writes the GPU path\'s outputs; not with --impl reference')
+    return args
 
 
 ###############################################################################
@@ -642,6 +657,17 @@ def time_single_utterance(emphases, model, gpu, calls=200):
         'api': 'emphases_b200.from_alignment_and_audio (host audio in, scores on the host out)'}
 
 
+def dump_outputs(directory, result, plan, rank, world):
+    """The word rows of a forward_packed result (separator rows dropped) as
+    float32 .npy files, so that two builds can be compared output for output"""
+    os.makedirs(directory, exist_ok=True)
+    rows = torch.from_numpy(np.flatnonzero(plan.word_seq >= 0)).to(result['scores'].device)
+    suffix = '' if world == 1 else f'.rank{rank}'
+    for name in ('scores', 'logits'):
+        values = result[name].reshape(-1).index_select(0, rows).float().cpu().numpy()
+        np.save(os.path.join(directory, f'{name}{suffix}.npy'), values)
+
+
 def workload_config(args):
     return {
         'workload': (
@@ -716,7 +742,7 @@ def main():
         torch.cuda.synchronize(device)
 
     for _ in range(max(args.warmup, 3)):
-        step()
+        result = step()
     barrier()
     clocks = ClockSampler(local_rank)
     clocks.start()
@@ -726,11 +752,14 @@ def main():
     start.record()
     for _ in range(args.steps):
         timers.append({})
-        step(timers[-1])
+        result = step(timers[-1])
     end.record()
     barrier()
     elapsed_ms = start.elapsed_time(end)
     clock_summary = clocks.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result, plan, rank, world)
+    del result
     launches_per_step = sum(entry[2] for entry in timers[0].values())
     kernel_ms = {
         name: statistics.mean(t[name][0].elapsed_time(t[name][1]) for t in timers)

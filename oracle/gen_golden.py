@@ -18,7 +18,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, 'tests'))
 
+from golden_util import save_golden  # noqa: E402
 from oracle import ref_stubs  # noqa: E402
 from oracle import emphases_oracle as oracle  # noqa: E402
 
@@ -127,7 +129,7 @@ def gen_c1():
                 alignment, audio, 16000, checkpoint=path)
         out['full.scores_autocast'] = result.float().numpy()
         out['full.scores_autocast_dtype'] = np.array(str(result.dtype))
-    np.savez_compressed(os.path.join(GOLDEN, 'c1.npz'), **out)
+    save_golden('c1', out)
     print('c1', {k: v.shape for k, v in out.items() if 'state' not in k})
 
 
@@ -183,7 +185,7 @@ def gen_sweep():
                         batch
                     ):
                         out[f'b2.{name}'] = value.numpy()
-    np.savez_compressed(os.path.join(GOLDEN, 'sweep.npz'), **out)
+    save_golden('sweep', out)
     print('sweep', len(out))
 
 
@@ -224,7 +226,7 @@ def gen_pool():
                 out['segment.segments'] = segments.numpy()
                 out['segment.bounds'] = seg_bounds.numpy()
                 out['segment.lengths'] = seg_lengths.numpy()
-    np.savez_compressed(os.path.join(GOLDEN, 'pool.npz'), **out)
+    save_golden('pool', out)
     print('pool', {k: (v.shape if v.ndim else str(v)) for k, v in out.items()})
 
 
@@ -266,7 +268,7 @@ def gen_transformer():
             ):
                 out[f'b2.{name}'] = value.numpy()
             out['b2.logits'] = model(*batch).numpy()
-    np.savez_compressed(os.path.join(GOLDEN, 'transformer.npz'), **out)
+    save_golden('transformer', out)
     print('transformer', len(out))
 
 
@@ -308,7 +310,7 @@ def gen_transformer_input():
             ):
                 out[f'b2.{name}'] = value.numpy()
             out['b2.logits'] = model(*batch).numpy()
-    np.savez_compressed(os.path.join(GOLDEN, 'transformer_input.npz'), **out)
+    save_golden('transformer_input', out)
     print('transformer_input', len(out))
 
 
@@ -325,7 +327,7 @@ def gen_loss():
             out[loss_fn] = emphases.loss(
                 scores, targets, None, None, word_lengths,
                 loss_fn=loss_fn).numpy()
-    np.savez_compressed(os.path.join(GOLDEN, 'loss.npz'), **out)
+    save_golden('loss', out)
     print('loss', out['bce'], out['mse'])
 
 
@@ -360,7 +362,7 @@ def gen_upsample():
                 out[f'{method}.loss.{loss_fn}'] = emphases.loss(
                     scores, xs, frame_lengths, bounds, word_lengths,
                     training=True, loss_fn=loss_fn).numpy()
-    np.savez_compressed(os.path.join(GOLDEN, 'upsample.npz'), **out)
+    save_golden('upsample', out)
     print('upsample', {k: v.shape for k, v in out.items()})
 
 
@@ -418,7 +420,7 @@ def gen_sampler():
         ):
             if key is not None:
                 out[f'collate/{key}'] = value.numpy()
-    np.savez_compressed(os.path.join(GOLDEN, 'sampler.npz'), **out)
+    save_golden('sampler', out)
     print('sampler.npz', len(out))
 
 
@@ -463,7 +465,7 @@ def gen_evaluate():
                 [[g[k] for k in keys] for g in granular], dtype=np.float64)
             out[f'{loss_fn}/stats'] = np.array(
                 [*predicted_stats(), *target_stats()], dtype=np.float64)
-    np.savez_compressed(os.path.join(GOLDEN, 'evaluate.npz'), **out)
+    save_golden('evaluate', out)
     print('evaluate.npz', len(out))
 
 

@@ -38,8 +38,6 @@ def padded_batch(seed=0, items=3):
 @pytest.mark.parametrize('method', ['sum', 'average', 'max', 'center'])
 @pytest.mark.parametrize('loss_fn', ['bce', 'mse'])
 def test_gradients_match_autograd(emphases, golden, method, loss_fn):
-    if loss_fn == 'mse' and method != 'sum':
-        pytest.skip('loss variants are covered with sum pooling')
     emphases.configure(DOWNSAMPLE_METHOD=method, LOSS=loss_fn)
     data = golden('sweep')
     state = state_from_golden(data)
