@@ -10,7 +10,8 @@
 // The convolutions run through emph_conv_stack one layer at a time (so every
 // layer's output is kept for the backward pass) in `precision`: the fp32 FFMA
 // kernel, or the split-bf16 tensor-core kernel (bf16x3 / bf16x6, fp32-grade)
-// for the forward and the input-gradient passes.  Weight gradients are fp32.
+// for the forward and the input-gradient passes.  Weight gradients run on the
+// split-bf16 mma.sync kernel in every mode (16-bit operands, fp32 accumulate).
 #include <vector>
 
 #include "common.cuh"
@@ -89,14 +90,24 @@ static bool keeps_pre(int act) { return act == EMPH_ACT_GELU || act == EMPH_ACT_
 
 // Rows kept per item.  The reference convolves all `frames` padded columns of
 // every item (emphases/model/layers/convolution.py:36-37 ignores the lengths),
-// but a word only pools frames below its item's length, and the value of the
-// last frame layer at row t depends on layer-i rows up to t + (layers - 1 - i):
-// rows beyond length + n_frame_layers * (k - 1) / 2 cannot reach the loss or
-// any gradient, so they are not computed (the kept rows are bit-identical).
+// and the value of the last frame layer at row t depends on layer-i rows up to
+// t + (layers - 1 - i): with `lengths` at least one past the last frame any
+// word reads (the caller's duty: a word may end past the audio), rows beyond
+// length + n_frame_layers * (k - 1) / 2 cannot reach the loss or any
+// gradient, so they are not computed (the rows words read are bit-identical).
 static int kept_rows(const emph_train_model& m, int frames, const int64_t* lengths, int b) {
     if (!lengths) return frames;
     const long long reach = lengths[b] + (long long)m.n_frame_layers * ((kTrainKernel - 1) / 2);
     return (int)(reach < frames ? (reach < 1 ? 1 : reach) : frames);
+}
+
+// Separator rows between the word rows of two items: the output projection
+// (kernel up to 7) reads (head_kernel - 1) / 2 rows on each side of a word, and
+// must see zeros there, not the next item's words (a word decoder layer, k = 3,
+// needs one)
+static int word_gap(const emph_train_model& m) {
+    const int half = (m.head_kernel - 1) / 2;
+    return half > 1 ? half : 1;
 }
 
 static TrainLayout make_layout(
@@ -105,7 +116,7 @@ static TrainLayout make_layout(
     l.batch = batch; l.frames = frames; l.wmax = wmax;
     l.total = 1;
     for (int b = 0; b < batch; ++b) l.total += kept_rows(m, frames, lengths, b) + 1;
-    l.total_words = batch * (wmax + 1) + 1;
+    l.total_words = batch * (wmax + word_gap(m)) + word_gap(m);
     l.n_frame = m.n_frame_layers; l.n_word = m.n_word_layers;
     size_t cursor = 0;
     auto take = [&](size_t bytes) { size_t at = cursor; cursor += up(bytes); return at; };
@@ -246,7 +257,7 @@ extern "C" int emph_train_forward(
         row_start[b] = next_row;
         n_rows[b] = kept_rows(m, frames, frame_lengths_host, b);
         next_row += n_rows[b] + 1;
-        word_row_start[b] = 1 + b * (wmax + 1);
+        word_row_start[b] = word_gap(m) + b * (wmax + word_gap(m));
         n_words[b] = wmax;
         const int64_t count = word_lengths_host[b];
         for (int j = 0; j < wmax; ++j) {

@@ -273,8 +273,9 @@ class _ConvModelFunction(torch.autograd.Function):
 # 'bf16x3' (hi/lo split, 1e-5 class logits) leaves 2e-3 on the gradient of the
 # first layer, and so does 'bf16x3+bf16x6' (x3 forward, x6 input gradients:
 # the forward's 1e-5 is what the deep gradients amplify); 2.01 instead of
-# 2.10 ms per step.  'fp32': the FFMA kernels, 4.1 ms.  Weight gradients are
-# always fp32.
+# 2.10 ms per step.  'fp32': the FFMA kernels, 4.1 ms.  In every mode the
+# weight gradients run on mma.sync with split bf16 operands (hi*hi + lo*hi +
+# hi*lo: 16-bit operands, fp32 accumulation), ~2^-16 relative per product.
 TRAIN_PRECISION = os.environ.get('EMPHASES_B200_TRAIN_PRECISION', 'bf16x6')
 _TRAIN_PRECISIONS = {
     'fp32': (_lib.PREC_FP32, _lib.PREC_FP32),
@@ -382,7 +383,16 @@ class _NativeConvFunction(torch.autograd.Function):
         wmax = int(word_bounds.shape[2])
         bounds = word_bounds.detach().to('cpu', torch.int64).contiguous()
         lengths = word_lengths.detach().to('cpu', torch.int64).contiguous()
-        frame_lengths = frame_lengths.detach().to('cpu', torch.int64).contiguous()
+        # Rows kept per item (see csrc/train_step.cu, kept_rows): a word may end
+        # past its item's length (an alignment running past the audio), and the
+        # rows it pools must be computed over all padded columns as the
+        # reference does, so an item reaches to the last frame any word reads
+        # (hi - 1, or the center (lo + hi) // 2)
+        lo, hi = bounds[:, 0].numpy(), bounds[:, 1].numpy()
+        real = np.arange(wmax)[None] < lengths.numpy()[:, None]
+        reach = np.where(real, np.maximum(hi, (lo + hi) // 2 + 1), 0).max(axis=1)
+        frame_lengths = torch.from_numpy(np.maximum(
+            frame_lengths.detach().to('cpu', torch.int64).numpy(), reach))
         descriptor = state.descriptor
         descriptor.pool_method = _lib.POOL[emphases.DOWNSAMPLE_METHOD]
         descriptor.forward_precision, descriptor.precision = _TRAIN_PRECISIONS[TRAIN_PRECISION]
@@ -457,6 +467,17 @@ class _NativeConvFunction(torch.autograd.Function):
 
 def forward_with_grad(model, features, frame_lengths, word_bounds, word_lengths):
     """Model.forward in training mode (gradients flow to model.parameters())"""
+    if model.location in ('intermediate', 'loss'):
+        # raise where the reference's downsample raises; it slices the padded
+        # (B, C, T) tensor, so a word may reach any of the T columns
+        method = emphases.DOWNSAMPLE_METHOD
+        if method in ('max', 'center'):
+            bounds = word_bounds.detach().to('cpu', torch.int64).numpy()
+            lengths = word_lengths.detach().to('cpu', torch.int64).numpy()
+            valid = np.arange(bounds.shape[2])[None] < lengths[:, None]
+            engine.validate_bounds(
+                np.stack([bounds[:, 0][valid], bounds[:, 1][valid]], axis=1),
+                features.shape[2], method)
     if native_step_supported(model, features):
         return _NativeConvFunction.apply(
             model, features, frame_lengths, word_bounds, word_lengths,

@@ -515,14 +515,21 @@ int emph_masked_loss(
  *             both calls re-pack what they need); acts[i] the EMPH_ACT_* code
  *             after layer i.  forward_precision / precision: EMPH_PREC_FP32,
  *             EMPH_PREC_BF16X3_TC or _BF16X6_TC for the forward / the
- *             input-gradient convolutions (weight gradients are always fp32).
+ *             input-gradient convolutions.  The weight gradients run on
+ *             mma.sync in every mode: bf16 hi + lo operands (16 bits each),
+ *             hi*hi + lo*hi + hi*lo with fp32 accumulation, ~2^-16 relative
+ *             per product.
  *   features  (B, 80, T) fp32 device; word_bounds (B, 2, Wmax) / word_lengths
  *             (B) int64 HOST arrays (emphases/data/collate.py:72-78).
  *             frame_lengths (B) int64 host, or NULL: the reference convolves
- *             all T padded columns of every item; rows further than one row
- *             per frame layer beyond an item's length cannot reach a word, so
- *             with the lengths given they are skipped (same logits, same
- *             gradients).  Pass the same array to both calls.
+ *             all T padded columns of every item.  With lengths given, rows
+ *             further than one row per frame layer beyond frame_lengths[b] are
+ *             skipped, which keeps the last frame layer exact up to row
+ *             frame_lengths[b] only: same logits and gradients as long as no
+ *             word of item b reads a frame at or past frame_lengths[b].  A word
+ *             may end past the audio, so pass per item max(length, 1 + the
+ *             last frame any word reads: hi - 1, or (lo + hi) / 2 for
+ *             `center`), and the same array to both calls.
  *   workspace device scratch of emph_train_workspace(...) bytes: it carries the
  *             kept activations from emph_train_forward to emph_train_backward
  *   logits    (B, 1, Wmax) fp32 device out (padded slots included, as
