@@ -409,43 +409,21 @@ def downsample(xs, word_bounds, word_lengths):
         raise ValueError(f'Interpolation method {method} is not defined')
     device = emphases.resolve_device(None, xs)
     eng = emphases.get_engine(device)
-    batch, channels, frames = xs.shape
+    batch, _, frames = xs.shape
     with torch.cuda.device(device):
-        starts, total = engine.packed_starts([frames] * batch)
-        meta = torch.from_numpy(np.concatenate([
-            starts.astype(np.int32), np.full(batch, frames, dtype=np.int32)])
-        ).to(device)
-        row_start, n_rows = meta[:batch], meta[batch:]
-        row_seq = eng.row_index(row_start, n_rows, batch, total)
-        rows = torch.empty(
-            (total, channels), dtype=torch.float32, device=device)
-        xs32 = xs.detach().to(device, torch.float32).contiguous()
-        _lib.call(
-            'emph_pack_rows', _lib.ptr(xs32), batch, channels, frames,
-            _lib.ptr(row_start), _lib.ptr(n_rows), _lib.ptr(row_seq), total,
-            _lib.ptr(rows), _lib.stream_ptr())
-        views, word_starts, total_words, bounds, lengths = \
+        rows, _, row_start, n_rows, _, _ = model_module.pack_batch(eng, xs)
+        views, word_starts, _, bounds, lengths = \
             model_module.word_rows(word_bounds, word_lengths, device)
-        wmax = word_bounds.shape[2]
-        if method != 'center':
-            wmax_out = int(lengths.max())
-        else:
-            wmax_out = wmax
+        if method == 'center':
             # center gathers every slot, padded ones included (core.py:458-466)
             views['word_lo'].clamp_(min=0)
             views['word_hi'].clamp_(min=0)
-        valid = np.arange(wmax)[None] < (
-            lengths[:, None] if method != 'center'
-            else np.full((batch, 1), wmax))
-        engine.validate_bounds(
-            np.stack([bounds[:, 0][valid], bounds[:, 1][valid]], axis=1),
-            np.full(int(valid.sum()), frames), method)
+            lengths = np.full(batch, word_bounds.shape[2])
+        model_module.check_word_bounds(bounds, lengths, frames, method)
         pooled = eng.pool(
             rows, row_start, n_rows, views['word_seq'], views['word_lo'],
             views['word_hi'], method)
-        index = torch.from_numpy(
-            (word_starts[:, None] + np.arange(wmax_out)[None]).astype(np.int64)
-        ).to(device)
+        index = model_module.slot_index(word_starts, int(lengths.max()), device)
         return pooled[index].transpose(1, 2).contiguous().to(xs.dtype)
 
 

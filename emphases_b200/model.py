@@ -136,36 +136,103 @@ class Model(torch.nn.Module):
                 self, features, frame_lengths, word_bounds, word_lengths)
 
 
-def word_rows(word_bounds, word_lengths, device):
-    """Packed word-row arrays for padded (B, 2, Wmax) bounds: every item gets
-    Wmax slots; slots j >= word_lengths[i] are marked (-1, -1)"""
-    batch, _, wmax = word_bounds.shape
-    starts, total = engine.packed_starts([wmax] * batch)
-    bounds = word_bounds.detach().to('cpu', torch.int64).numpy()
-    lengths = word_lengths.detach().to('cpu', torch.int64).numpy()
-    word_seq = np.full(total, -1, dtype=np.int32)
-    word_lo = np.zeros(total, dtype=np.int32)
-    word_hi = np.zeros(total, dtype=np.int32)
-    for b in range(batch):
-        s = int(starts[b])
-        word_seq[s:s + wmax] = b
-        word_lo[s:s + wmax] = bounds[b, 0]
-        word_hi[s:s + wmax] = bounds[b, 1]
-        word_lo[s + int(lengths[b]):s + wmax] = -1
-        word_hi[s + int(lengths[b]):s + wmax] = -1
+def pack_batch(eng, xs):
+    """Packed rows of a padded (B, C, T) batch: every item is a sequence of
+    all T columns, padding included.  One H2D copy of (row_start, n_rows),
+    then emph_row_index and emph_pack_rows.  Returns (rows, row_seq, device
+    row_start, device n_rows, host starts, total rows)."""
+    batch, channels, frames = xs.shape
+    device = eng.device
+    starts, total = engine.packed_starts([frames] * batch)
+    meta = torch.from_numpy(np.concatenate([
+        starts.astype(np.int32), np.full(batch, frames, dtype=np.int32)])
+    ).to(device)
+    row_start, n_rows = meta[:batch], meta[batch:]
+    row_seq = eng.row_index(row_start, n_rows, batch, total)
+    rows = torch.empty((total, channels), dtype=torch.float32, device=device)
+    xs = xs.detach().to(device, torch.float32).contiguous()
+    _lib.call(
+        'emph_pack_rows', _lib.ptr(xs), batch, channels, frames,
+        _lib.ptr(row_start), _lib.ptr(n_rows), _lib.ptr(row_seq), total,
+        _lib.ptr(rows), _lib.stream_ptr())
+    return rows, row_seq, row_start, n_rows, starts, total
+
+
+def slot_index(starts, width, device):
+    """(B, width) int64 device index of the packed rows of every item's
+    `width` slots: row starts[b] + j"""
+    return torch.from_numpy(
+        (starts[:, None] + np.arange(width)[None]).astype(np.int64)).to(device)
+
+
+def check_word_bounds(bounds, lengths, frames, method):
+    """Raise where the reference's downsample raises, for the slots j <
+    lengths[b] of host bounds (B, 2, W) over a padded batch of `frames`
+    columns"""
+    valid = np.arange(bounds.shape[2])[None] < lengths[:, None]
+    engine.validate_bounds(
+        np.stack([bounds[:, 0][valid], bounds[:, 1][valid]], axis=1),
+        frames, method)
+
+
+def slot_views(word_seq, word_lo, word_hi, device):
+    """Device word-row arrays of a padded batch from (B, W) host arrays: every
+    item gets W slots, separator rows read (-1, 0, 0).  One H2D copy.
+    Returns (views, host word starts, total word rows)."""
+    batch, width = word_seq.shape
+    starts, total = engine.packed_starts([width] * batch)
+    rows = np.zeros((3, total), dtype=np.int32)
+    rows[0] = -1
+    for b, s in enumerate(starts):
+        rows[:, s:s + width] = word_seq[b], word_lo[b], word_hi[b]
     blob = torch.from_numpy(np.concatenate([
-        starts.astype(np.int32), np.full(batch, wmax, dtype=np.int32),
-        word_seq, word_lo, word_hi])).to(device)
+        starts.astype(np.int32), np.full(batch, width, dtype=np.int32),
+        rows.reshape(-1)])).to(device)
     views = {
         'word_row_start': blob[:batch],
         'n_words': blob[batch:2 * batch],
         'word_seq': blob[2 * batch:2 * batch + total],
         'word_lo': blob[2 * batch + total:2 * batch + 2 * total],
         'word_hi': blob[2 * batch + 2 * total:]}
+    return views, starts, total
+
+
+def word_rows(word_bounds, word_lengths, device):
+    """Packed word-row arrays for padded (B, 2, Wmax) bounds: every item gets
+    Wmax slots; slots j >= word_lengths[i] are marked (-1, -1)"""
+    batch, _, wmax = word_bounds.shape
+    bounds = word_bounds.detach().to('cpu', torch.int64).numpy()
+    lengths = word_lengths.detach().to('cpu', torch.int64).numpy()
+    masked = np.arange(wmax)[None] >= lengths[:, None]
+    views, starts, total = slot_views(
+        np.repeat(np.arange(batch)[:, None], wmax, axis=1),
+        np.where(masked, -1, bounds[:, 0]), np.where(masked, -1, bounds[:, 1]),
+        device)
     return views, starts, total, bounds, lengths
 
 
+def conv_encoders(eng, weights, precision):
+    """(encode, decode) of the convolution architecture: the frame and word
+    conv stacks.  Every packed row is a query and a key alike
+    (convolution.py:36-37 ignores the lengths), so the counts go unread."""
+
+    def encode(rows, row_seq, row_start, n_queries, n_keys):
+        return eng.conv_stack(
+            rows, row_seq, weights.frame,
+            engine.frame_precision(precision, weights.frame))
+
+    def decode(pooled, word_row_seq, word_start, n_queries, n_keys):
+        return eng.conv_stack(
+            pooled, word_row_seq, weights.word,
+            engine.word_precision(precision, weights.word))
+
+    return encode, decode
+
+
 def run_forward(model, features, frame_lengths, word_bounds, word_lengths):
+    """Model.forward on packed rows, for both architectures.  The encoder pair
+    takes (rows, row_seq, device row_start, host n_queries, n_keys): every
+    sequence has n_queries rows, of which the first n_keys are valid keys."""
     eng = emphases.get_engine(features.device)
     weights = model.packed_weights()
     method = emphases.DOWNSAMPLE_METHOD
@@ -174,63 +241,40 @@ def run_forward(model, features, frame_lengths, word_bounds, word_lengths):
     precision = emphases.precision_code()
     if model.architecture == 'transformer':
         from . import transformer
-        return transformer.run_forward(
-            model, eng, weights, features, frame_lengths, word_bounds,
-            word_lengths)
+        encode, decode = transformer.encoders(eng, weights)
+    else:
+        encode, decode = conv_encoders(eng, weights, precision)
+    device = features.device
+    batch, _, frames = features.shape
+    wmax = word_bounds.shape[2]
     if model.location == 'input':
         from . import segments
-        return segments.run_forward_input(
-            model, eng, weights, features, word_bounds, word_lengths,
-            method, precision)
-
-    batch, channels, frames = features.shape
-    device = features.device
-    # Convolution ignores frame_lengths (convolution.py:36-37): every item
-    # is a sequence of all `frames` columns, padding included
-    starts, total = engine.packed_starts([frames] * batch)
-    rows_meta = torch.from_numpy(np.concatenate([
-        starts.astype(np.int32), np.full(batch, frames, dtype=np.int32)])
-    ).to(device)
-    row_start, n_rows = rows_meta[:batch], rows_meta[batch:]
-    row_seq = eng.row_index(row_start, n_rows, batch, total)
-    rows = torch.empty((total, channels), dtype=torch.float32, device=device)
-    features = features.detach().to(torch.float32).contiguous()
-    _lib.call(
-        'emph_pack_rows', _lib.ptr(features), batch, channels, frames,
-        _lib.ptr(row_start), _lib.ptr(n_rows), _lib.ptr(row_seq), total,
-        _lib.ptr(rows), _lib.stream_ptr())
-    frame_rows = eng.conv_stack(
-        rows, row_seq, weights.frame,
-        engine.frame_precision(precision, weights.frame))
-
-    if model.location == 'inference' and model.training:
-        # frame-resolution logits (model/core.py:119-122)
-        logits, _ = eng.head(
-            frame_rows, row_seq, weights, _lib.HEAD_LOGITS, want_scores=False)
-        index = torch.from_numpy(
-            (starts[:, None] + np.arange(frames)[None]).astype(np.int64)
-        ).to(device)
-        return logits[index][:, None, :]
-
-    views, word_starts, total_words, bounds, lengths = word_rows(
-        word_bounds, word_lengths, device)
-    wmax = word_bounds.shape[2]
-    valid = np.arange(wmax)[None] < lengths[:, None]
-    engine.validate_bounds(
-        np.stack([bounds[:, 0][valid], bounds[:, 1][valid]], axis=1),
-        np.full(int(valid.sum()), frames), method)
-    pooled = eng.pool(
-        frame_rows, row_start, n_rows, views['word_seq'], views['word_lo'],
-        views['word_hi'], method)
-    word_row_seq = eng.row_index(
-        views['word_row_start'], views['n_words'], batch, total_words)
-    if model.location == 'intermediate':
-        pooled = eng.conv_stack(
-            pooled, word_row_seq, weights.word,
-            engine.word_precision(precision, weights.word))
+        words, word_row_seq, word_starts = segments.run_forward_input(
+            eng, features, word_bounds, word_lengths, method, encode, decode)
+    else:
+        rows, row_seq, row_start, n_rows, starts, _ = pack_batch(eng, features)
+        # frame_lengths goes in as given: only the Transformer reads it on the
+        # host (a device tensor costs a sync)
+        frame_rows = encode(
+            rows, row_seq, row_start, np.full(batch, frames), frame_lengths)
+        if model.location == 'inference' and model.training:
+            # frame-resolution logits (model/core.py:119-122)
+            logits, _ = eng.head(
+                frame_rows, row_seq, weights, _lib.HEAD_LOGITS,
+                want_scores=False)
+            return logits[slot_index(starts, frames, device)][:, None, :]
+        views, word_starts, total_words, bounds, lengths = word_rows(
+            word_bounds, word_lengths, device)
+        check_word_bounds(bounds, lengths, frames, method)
+        words = eng.pool(
+            frame_rows, row_start, n_rows, views['word_seq'], views['word_lo'],
+            views['word_hi'], method)
+        word_row_seq = eng.row_index(
+            views['word_row_start'], views['n_words'], batch, total_words)
+        if model.location == 'intermediate':
+            words = decode(
+                words, word_row_seq, views['word_row_start'],
+                np.full(batch, wmax), lengths)
     logits, _ = eng.head(
-        pooled, word_row_seq, weights, _lib.HEAD_LOGITS, want_scores=False)
-    index = torch.from_numpy(
-        (word_starts[:, None] + np.arange(wmax)[None]).astype(np.int64)
-    ).to(device)
-    return logits[index][:, None, :]
+        words, word_row_seq, weights, _lib.HEAD_LOGITS, want_scores=False)
+    return logits[slot_index(word_starts, wmax, device)][:, None, :]

@@ -12,6 +12,7 @@ import torch
 
 import emphases_b200 as emphases
 from . import _lib, engine
+from .model import slot_views
 
 
 def _segment_plan(word_bounds, word_lengths, frames):
@@ -101,86 +102,44 @@ def input_word_rows(batch, wmax, lengths, count, max_length, method, device):
     out as B sequences of Wmax word slots; row w pools segment word_seq[w] over
     its padded length (model/core.py:55-63), masked slots are (-2, -2).
     Returns (device views, host word_starts, total_words)."""
-    word_starts, total_words = engine.packed_starts([wmax] * batch)
-    word_seq = np.full(total_words, -1, dtype=np.int32)
-    word_lo = np.zeros(total_words, dtype=np.int32)
-    word_hi = np.zeros(total_words, dtype=np.int32)
-    for b in range(batch):
-        s = int(word_starts[b])
-        word_seq[s:s + wmax] = b * wmax + np.arange(wmax)
-        if method == 'center':
-            # downsample(frame_embeddings, [0, frames], ones): (0 + frames) // 2
-            word_lo[s:s + wmax] = 0
-            word_hi[s:s + wmax] = count[b]
-        else:
-            # reduction over the whole padded segment (model/core.py:55-63)
-            word_lo[s:s + wmax] = 0
-            word_hi[s:s + wmax] = max_length
-        word_lo[s + int(lengths[b]):s + wmax] = -2         # word mask (:77-82)
-        word_hi[s + int(lengths[b]):s + wmax] = -2
     if method == 'max' and max_length == 0:
         raise IndexError('max(): Expected reduction dim 2 to have non-zero size')
+    masked = np.arange(wmax)[None] >= lengths[:, None]          # word mask (:77-82)
     if method == 'center':
-        valid = np.arange(wmax)[None] < lengths[:, None]
-        if np.any((count // 2)[valid] >= max(max_length, 1)):
+        if np.any((count // 2)[~masked] >= max(max_length, 1)):
             raise IndexError('center frame index out of range for a word')
-    meta = torch.from_numpy(np.concatenate([
-        word_starts.astype(np.int32), np.full(batch, wmax, dtype=np.int32),
-        word_seq, word_lo, word_hi])).to(device)
-    views = {
-        'word_row_start': meta[:batch],
-        'n_words': meta[batch:2 * batch],
-        'word_seq': meta[2 * batch:2 * batch + total_words],
-        'word_lo': meta[2 * batch + total_words:2 * batch + 2 * total_words],
-        'word_hi': meta[2 * batch + 2 * total_words:]}
-    return views, word_starts, total_words
+        # downsample(frame_embeddings, [0, frames], ones): (0 + frames) // 2
+        hi = count
+    else:
+        # reduction over the whole padded segment (model/core.py:55-63)
+        hi = np.full_like(count, max_length)
+    return slot_views(
+        np.arange(batch * wmax).reshape(batch, wmax), np.where(masked, -2, 0),
+        np.where(masked, -2, hi), device)
 
 
-def run_forward_input(
-    model, eng, weights, features, word_bounds, word_lengths, method, precision,
-    encode=None, decode=None
-):
-    """Model.forward for DOWNSAMPLE_LOCATION == 'input'.
-
-    `encode(segments, seg_row_seq, seg_start, max_length, counts)` and
-    `decode(pooled, word_row_seq, word_start, wmax, lengths)` replace the
-    convolutional frame encoder / word decoder (the Transformer variant
-    attends within each word segment: keys are the segment's own `counts`
-    frames, queries all `max_length` rows)."""
-    device = features.device
-    batch, channels, frames = features.shape
+def run_forward_input(eng, features, word_bounds, word_lengths, method, encode, decode):
+    """Model.forward for DOWNSAMPLE_LOCATION == 'input' up to the output head,
+    with model.run_forward's encoder pair: every word segment is a sequence of
+    max_length queries whose keys are the segment's own frames (the Transformer
+    attends within each segment).  Returns (decoded word rows, word_row_seq,
+    host word starts)."""
+    batch, _, frames = features.shape
     wmax = word_bounds.shape[2]
     _, lengths, max_length, lo, count = _segment_plan(
         word_bounds, word_lengths, frames)
-    n_seg = batch * wmax
     segments, seg_row_seq, d_seg_start, d_seg_rows, _, _ = _gather(
         eng, features, lo, count, max_length)
-    if encode is not None:
-        frame_rows = encode(
-            segments, seg_row_seq, d_seg_start, max_length, count.reshape(-1))
-    else:
-        frame_rows = eng.conv_stack(
-            segments, seg_row_seq, weights.frame,
-            engine.frame_precision(precision, weights.frame))
-
+    frame_rows = encode(
+        segments, seg_row_seq, d_seg_start, np.full(lo.size, max_length),
+        count.reshape(-1))
     views, word_starts, total_words = input_word_rows(
-        batch, wmax, lengths, count, max_length, method, device)
-    d_word_start, d_n_words = views['word_row_start'], views['n_words']
-    d_word_seq, d_word_lo, d_word_hi = (
-        views['word_seq'], views['word_lo'], views['word_hi'])
+        batch, wmax, lengths, count, max_length, method, eng.device)
     pooled = eng.pool(
-        frame_rows, d_seg_start, d_seg_rows, d_word_seq, d_word_lo, d_word_hi,
-        method)
-    word_row_seq = eng.row_index(d_word_start, d_n_words, batch, total_words)
-    if decode is not None:
-        words = decode(pooled, word_row_seq, d_word_start, wmax, lengths)
-    else:
-        words = eng.conv_stack(
-            pooled, word_row_seq, weights.word,
-            engine.word_precision(precision, weights.word))
-    logits, _ = eng.head(
-        words, word_row_seq, weights, _lib.HEAD_LOGITS, want_scores=False)
-    index = torch.from_numpy(
-        (word_starts[:, None] + np.arange(wmax)[None]).astype(np.int64)
-    ).to(device)
-    return logits[index][:, None, :]
+        frame_rows, d_seg_start, d_seg_rows, views['word_seq'], views['word_lo'],
+        views['word_hi'], method)
+    word_row_seq = eng.row_index(
+        views['word_row_start'], views['n_words'], batch, total_words)
+    words = decode(
+        pooled, word_row_seq, views['word_row_start'], np.full(batch, wmax), lengths)
+    return words, word_row_seq, word_starts

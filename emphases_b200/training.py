@@ -84,7 +84,7 @@ class _ConvModelFunction(torch.autograd.Function):
             raise NotImplementedError(
                 f'the backward kernels are built for up to {engine.KERNEL_CHANNELS} '
                 f'channels (CHANNELS={emphases.CHANNELS})')
-        batch, channels, frames = features.shape
+        batch, _, frames = features.shape
         wmax = word_bounds.shape[2]
         with torch.cuda.device(device), _lib.same_stream():
             input_location = model.location == 'input'
@@ -98,19 +98,8 @@ class _ConvModelFunction(torch.autograd.Function):
                 rows, row_seq, row_start, n_rows, _, total = segments._gather(
                     eng, features, lo, count, max_length)
             else:
-                starts, total = engine.packed_starts([frames] * batch)
-                meta = torch.from_numpy(np.concatenate([
-                    starts.astype(np.int32), np.full(batch, frames, dtype=np.int32)])
-                ).to(device)
-                row_start, n_rows = meta[:batch], meta[batch:]
-                row_seq = eng.row_index(row_start, n_rows, batch, total)
-                rows = torch.empty(
-                    (total, channels), dtype=torch.float32, device=device)
-                features32 = features.detach().to(torch.float32).contiguous()
-                _lib.call(
-                    'emph_pack_rows', _lib.ptr(features32), batch, channels, frames,
-                    _lib.ptr(row_start), _lib.ptr(n_rows), _lib.ptr(row_seq), total,
-                    _lib.ptr(rows), _lib.stream_ptr())
+                rows, row_seq, row_start, n_rows, starts, total = \
+                    model_module.pack_batch(eng, features)
             frame_layers, word_layers = _layer_list(model)
 
             def layer_forward(x, seq, weight, bias, act):
@@ -141,9 +130,7 @@ class _ConvModelFunction(torch.autograd.Function):
                 logits, _ = eng.head(
                     frame_acts[-1], row_seq, weights, _lib.HEAD_LOGITS,
                     want_scores=False)
-                index = torch.from_numpy(
-                    (starts[:, None] + np.arange(frames)[None]).astype(np.int64)
-                ).to(device)
+                index = model_module.slot_index(starts, frames, device)
                 ctx.model = model
                 ctx.saved = dict(
                     frame_acts=frame_acts, frame_keys=frame_keys,
@@ -170,9 +157,7 @@ class _ConvModelFunction(torch.autograd.Function):
             logits, _ = eng.head(
                 word_acts[-1], word_row_seq, weights, _lib.HEAD_LOGITS,
                 want_scores=False)
-            index = torch.from_numpy(
-                (word_starts[:, None] + np.arange(wmax)[None]).astype(np.int64)
-            ).to(device)
+            index = model_module.slot_index(word_starts, wmax, device)
         ctx.model = model
         ctx.saved = dict(
             frame_acts=frame_acts, word_acts=word_acts, frame_keys=frame_keys,
@@ -467,17 +452,15 @@ class _NativeConvFunction(torch.autograd.Function):
 
 def forward_with_grad(model, features, frame_lengths, word_bounds, word_lengths):
     """Model.forward in training mode (gradients flow to model.parameters())"""
-    if model.location in ('intermediate', 'loss'):
+    method = emphases.DOWNSAMPLE_METHOD
+    if model.location in ('intermediate', 'loss') and method in ('max', 'center'):
         # raise where the reference's downsample raises; it slices the padded
         # (B, C, T) tensor, so a word may reach any of the T columns
-        method = emphases.DOWNSAMPLE_METHOD
-        if method in ('max', 'center'):
-            bounds = word_bounds.detach().to('cpu', torch.int64).numpy()
-            lengths = word_lengths.detach().to('cpu', torch.int64).numpy()
-            valid = np.arange(bounds.shape[2])[None] < lengths[:, None]
-            engine.validate_bounds(
-                np.stack([bounds[:, 0][valid], bounds[:, 1][valid]], axis=1),
-                features.shape[2], method)
+        from . import model as model_module
+        model_module.check_word_bounds(
+            word_bounds.detach().to('cpu', torch.int64).numpy(),
+            word_lengths.detach().to('cpu', torch.int64).numpy(),
+            features.shape[2], method)
     if native_step_supported(model, features):
         return _NativeConvFunction.apply(
             model, features, frame_lengths, word_bounds, word_lengths,

@@ -430,81 +430,25 @@ def run_stack(
     return h
 
 
-def run_forward(
-    model, eng, weights, features, frame_lengths, word_bounds, word_lengths
-):
-    """Model.forward for the transformer variant (padded (B, C, T) batch)"""
-    from . import model as model_module
-    method = emphases.DOWNSAMPLE_METHOD
-    device = features.device
-    if model.location == 'input':
-        # every word segment is its own attention sequence
-        # (emphases/model/core.py:41-87 with frame_encoder = Transformer)
-        from . import segments
+def encoders(eng, weights):
+    """(encode, decode) of the Transformer architecture for model.run_forward:
+    input_layer and the frame stack, and the word stack.  A sequence of
+    n_queries[u] rows attends over its first n_keys[u] rows."""
 
-        def encode(rows, seg_row_seq, seg_start, max_length, counts):
-            embedded = eng.conv_stack(
-                rows, seg_row_seq, weights.input_layer,
-                engine.linear_precision(weights.input_layer))
-            return run_stack(
-                eng, weights.frame, embedded, seg_start,
-                np.full(len(counts), max_length), counts, seg_row_seq, device)
+    def encode(rows, row_seq, row_start, n_queries, n_keys):
+        # input_layer is a Conv1d over ALL T columns, padding included
+        embedded = eng.conv_stack(
+            rows, row_seq, weights.input_layer,
+            engine.linear_precision(weights.input_layer))
+        if torch.is_tensor(n_keys):          # frame_lengths, maybe on the device
+            n_keys = n_keys.detach().to('cpu', torch.int64).numpy()
+        return run_stack(
+            eng, weights.frame, embedded, row_start, n_queries, n_keys, row_seq,
+            eng.device)
 
-        def decode(pooled, word_row_seq, word_start, wmax, lengths):
-            return run_stack(
-                eng, weights.word, pooled, word_start,
-                np.full(len(lengths), wmax), lengths, word_row_seq, device, tag='word_')
+    def decode(pooled, word_row_seq, word_start, n_queries, n_keys):
+        return run_stack(
+            eng, weights.word, pooled, word_start, n_queries, n_keys,
+            word_row_seq, eng.device, tag='word_')
 
-        return segments.run_forward_input(
-            model, eng, weights, features, word_bounds, word_lengths, method,
-            _lib.PREC_FP32, encode, decode)
-    batch, channels, frames = features.shape
-    frame_keys = frame_lengths.detach().to('cpu', torch.int64).numpy()
-    starts, total = engine.packed_starts([frames] * batch)
-    rows_meta = torch.from_numpy(np.concatenate([
-        starts.astype(np.int32), np.full(batch, frames, dtype=np.int32)])
-    ).to(device)
-    row_start, n_rows = rows_meta[:batch], rows_meta[batch:]
-    row_seq = eng.row_index(row_start, n_rows, batch, total)
-    rows = torch.empty((total, channels), dtype=torch.float32, device=device)
-    features = features.detach().to(torch.float32).contiguous()
-    _lib.call(
-        'emph_pack_rows', _lib.ptr(features), batch, channels, frames,
-        _lib.ptr(row_start), _lib.ptr(n_rows), _lib.ptr(row_seq), total,
-        _lib.ptr(rows), _lib.stream_ptr())
-    # input_layer is a Conv1d over ALL T columns, padding included
-    embedded = eng.conv_stack(
-        rows, row_seq, weights.input_layer,
-        engine.linear_precision(weights.input_layer))
-    frame_rows = run_stack(
-        eng, weights.frame, embedded, row_start, np.full(batch, frames),
-        frame_keys, row_seq, device)
-
-    if model.location == 'inference' and model.training:
-        logits, _ = eng.head(
-            frame_rows, row_seq, weights, _lib.HEAD_LOGITS, want_scores=False)
-        index = torch.from_numpy(
-            (starts[:, None] + np.arange(frames)[None]).astype(np.int64)).to(device)
-        return logits[index][:, None, :]
-
-    views, word_starts, total_words, bounds, lengths = model_module.word_rows(
-        word_bounds, word_lengths, device)
-    wmax = word_bounds.shape[2]
-    valid = np.arange(wmax)[None] < lengths[:, None]
-    engine.validate_bounds(
-        np.stack([bounds[:, 0][valid], bounds[:, 1][valid]], axis=1),
-        np.full(int(valid.sum()), frames), method)
-    pooled = eng.pool(
-        frame_rows, row_start, n_rows, views['word_seq'], views['word_lo'],
-        views['word_hi'], method)
-    word_row_seq = eng.row_index(
-        views['word_row_start'], views['n_words'], batch, total_words)
-    if model.location == 'intermediate':
-        pooled = run_stack(
-            eng, weights.word, pooled, views['word_row_start'],
-            np.full(batch, wmax), lengths, word_row_seq, device, tag='word_')
-    logits, _ = eng.head(
-        pooled, word_row_seq, weights, _lib.HEAD_LOGITS, want_scores=False)
-    index = torch.from_numpy(
-        (word_starts[:, None] + np.arange(wmax)[None]).astype(np.int64)).to(device)
-    return logits[index][:, None, :]
+    return encode, decode

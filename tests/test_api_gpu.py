@@ -389,6 +389,47 @@ def test_transformer_variant(emphases, golden):
                 rtol=0, atol=3e-5)
 
 
+@pytest.mark.parametrize('location', ['loss', 'inference'])
+def test_transformer_variant_without_word_decoder(emphases, golden, location):
+    """Transformer variant at the locations that have no word decoder, vs the
+    oracle in fp64 on the golden weights (B=1 and the padded B=2 batch), and
+    at 'inference' the training-mode frame logits over the valid frames"""
+    data = golden('transformer')
+    emphases.configure(ARCHITECTURE='transformer', DOWNSAMPLE_LOCATION=location)
+    model = emphases.Model()
+    own = model.state_dict()
+    missing = model.load_state_dict(
+        {k: v for k, v in state_from_golden(data).items() if k in own},
+        strict=False)
+    assert all('position.encoding' in key for key in missing.missing_keys)
+    model = model.cuda().eval()
+    # the golden state has no position.encoding; the model's buffer supplies it
+    reference = {k: v.detach().cpu().double() for k, v in model.state_dict().items()}
+    config = {'ARCHITECTURE': 'transformer', 'DOWNSAMPLE_LOCATION': location}
+    features = torch.from_numpy(data['b1.features'])
+    bounds = torch.from_numpy(data['b1.bounds'])
+    b1 = [features, torch.tensor([features.shape[-1]]), bounds,
+          torch.tensor([bounds.shape[-1]])]
+    b2 = [torch.from_numpy(data[f'b2.{name}']) for name in (
+        'features', 'frame_lengths', 'bounds', 'word_lengths')]
+    cases = [(b1, False), (b2, False)] + [(b2, True)] * (location == 'inference')
+    for batch, training in cases:
+        model.train(training)
+        with torch.no_grad():
+            logits = model(batch[0].cuda(), *batch[1:]).cpu().numpy()
+        expected = oracle.model_forward(
+            reference, batch[0].double(), *batch[1:], config=config,
+            training=training).numpy()
+        assert logits.shape == expected.shape
+        # The 'sum'-pooled word logits reach |52| on this batch; fp32
+        # summation order alone moves them by 5.5e-5 from fp64 (1e-6
+        # relative, B200).  Hence the rtol of test_model_forward_sweep.
+        valid = batch[1] if training else batch[3]
+        for i, count in enumerate(valid.tolist()):
+            np.testing.assert_allclose(
+                logits[i, :, :count], expected[i, :, :count], rtol=1e-5, atol=3e-5)
+
+
 def test_transformer_variant_input_location(emphases, golden):
     """Transformer variant at DOWNSAMPLE_LOCATION='input' vs the reference
     (B=1 and a padded B=2 batch): attention runs inside each word segment"""
