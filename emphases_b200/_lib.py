@@ -18,10 +18,20 @@ ACT_NONE, ACT_RELU, ACT_GELU, ACT_LEAKY_RELU, ACT_SILU = 0, 1, 2, 3, 4
 POOL = {'average': 0, 'max': 1, 'sum': 2, 'center': 3}
 HEAD_LOGITS, HEAD_SIGMOID, HEAD_CLAMP = 0, 1, 2
 PREC_FP32, PREC_BF16_TC, PREC_BF16X3_TC, PREC_BF16X6_TC = 0, 1, 2, 3
+# dropout site kinds (EMPH_DROPOUT_*)
+(DROPOUT_POSITIONAL, DROPOUT_ATTENTION, DROPOUT_RESIDUAL1, DROPOUT_FEEDFORWARD,
+ DROPOUT_RESIDUAL2) = range(5)
+
+
+def dropout_site(stack, layer, kind, head=0):
+    """EMPH_DROPOUT_SITE: stack 0 = frame encoder, 1 = word decoder"""
+    return (stack << 24) | (layer << 16) | (kind << 8) | head
 
 _P = ctypes.c_void_p
 _I = ctypes.c_int32
 _F = ctypes.c_float
+_U32 = ctypes.c_uint32
+_U64 = ctypes.c_uint64
 
 # name -> argtypes; every function returns int.  Keep in sync with the header
 # (tests/test_abi.py checks that every declared symbol is exported).
@@ -69,6 +79,20 @@ SIGNATURES = {
     'emph_output_head_backward': [_P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P],
     'emph_masked_loss': [_P, _P, _P, _I, _I, _P, _P, _P],
     'emph_upsample_words': [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P],
+    'emph_dropout_keep': [_U64, _U32, _U64, ctypes.c_int64, _F, _P, _P],
+    'emph_dropout_rows': [_P, _I, _I, _U64, _U32, _F, _P, _P],
+    'emph_linear_rows': [_P, _I, _I, _P, _P, _I, _I, _P, _P, _P],
+    'emph_linear_rows_backward': [_P, _I, _I, _P, _I, _P, _P, _P, _P],
+    'emph_attention_rows_train': [
+        _P, _P, _P, _I, _I, _P, _P, _P, _P, _I, _P, _P, _I, _F, _U64, _U32, _F, _P, _P, _P],
+    'emph_attention_rows_backward': [
+        _P, _P, _P, _P, _P, _P, _I, _I, _P, _P, _P, _I, _P, _P, _I, _P, _P, _I, _F, _U64, _U32,
+        _F, _P, _P, _P, _P],
+    'emph_add_layernorm_train': [
+        _P, _P, _P, _P, _F, _P, _I, _I, _U64, _U32, _F, _P, _P, _P, _P],
+    'emph_layernorm_backward_blocks': [_I],
+    'emph_add_layernorm_backward': [
+        _P, _P, _P, _P, _P, _I, _I, _U64, _U32, _F, _P, _P, _P, _P, _P, _P],
     'emph_word_metric_sums': [
         _P, _P, _P, _P, _I, _I, _I, ctypes.c_double, ctypes.c_double, _P, _P],
 }

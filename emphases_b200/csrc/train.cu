@@ -480,7 +480,7 @@ int emph_activation_forward(
 int emph_conv_weight_grad(
     const float* x, const float* dpre, int32_t total_rows, int32_t channels,
     int32_t kernel_size, float* dw, float* db, void* stream) {
-    if (!(channels == 80 && kernel_size == 3)) {
+    if (!(channels == 80 && (kernel_size == 3 || kernel_size == 1))) {
         emph::set_error("emph_conv_weight_grad: channels=%d kernel_size=%d not compiled in",
                         channels, kernel_size);
         return EMPH_ENOSYS;
@@ -494,7 +494,10 @@ int emph_conv_weight_grad(
     if (total_rows == 0) return EMPH_OK;
     int grid = (total_rows + 63) / 64;
     if (grid > emph::sm_count() * 2) grid = emph::sm_count() * 2;
-    emph::conv_weight_grad_kernel<80, 3, false><<<grid, 256, 0, st>>>(x, dpre, total_rows, dw, db);
+    if (kernel_size == 3)
+        emph::conv_weight_grad_kernel<80, 3, false><<<grid, 256, 0, st>>>(x, dpre, total_rows, dw, db);
+    else        // the Linear maps of the Transformer variant
+        emph::conv_weight_grad_kernel<80, 1, false><<<grid, 256, 0, st>>>(x, dpre, total_rows, dw, db);
     EMPH_CHECK_LAUNCH("emph_conv_weight_grad");
     return EMPH_OK;
 }

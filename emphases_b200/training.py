@@ -1,6 +1,7 @@
-"""Training step of the conv model on device: forward with saved
-activations, hand-written backward kernels (csrc/train.cu), masked loss, and
-a flat-bucket gradient all-reduce for data parallelism.
+"""Training step on device: forward with saved activations, hand-written
+backward kernels (csrc/train.cu for the conv model, csrc/attention.cu and
+csrc/transformer_train.cu for the Transformer variant), masked loss, and a
+flat-bucket gradient all-reduce for data parallelism.
 
 The reference trains on one device (emphases/train/core.py:86-142) with
 torch autograd; it has no data-parallel code.  Here `Model.forward` in
@@ -67,185 +68,279 @@ def _zero_bias(channels, device):
     return _zero_biases[key]
 
 
-class _ConvModelFunction(torch.autograd.Function):
+def _layer_forward(eng, x, seq, weight, bias, act, device):
+    """One conv layer of the training forward: (output, what
+    emph_activation_backward needs): GELU / SiLU keep the pre-activation, the
+    others their output"""
+    if act in (_lib.ACT_GELU, _lib.ACT_SILU):
+        pre = eng.conv_stack(
+            x, seq, _stack(weight, bias, _lib.ACT_NONE, device), _lib.PREC_FP32)
+        y = torch.empty_like(pre)
+        _lib.call(
+            'emph_activation_forward', _lib.ptr(pre), _lib.ptr(seq),
+            pre.shape[0], pre.shape[1], act, _lib.ptr(y), _lib.stream_ptr())
+        return y, pre
+    y = eng.conv_stack(x, seq, _stack(weight, bias, act, device), _lib.PREC_FP32)
+    return y, y
 
-    @staticmethod
-    def forward(ctx, model, features, word_bounds, word_lengths, *parameters):
-        from . import model as model_module
-        device = features.device
-        eng = emphases.get_engine(device)
-        method = emphases.DOWNSAMPLE_METHOD
-        if method not in _lib.POOL:
-            raise ValueError(f'Interpolation method {method} is not defined')
-        if model.architecture != 'convolution':
-            raise NotImplementedError(
-                'the training step is built for the convolution architecture')
-        if emphases.CHANNELS > engine.KERNEL_CHANNELS:
-            raise NotImplementedError(
-                f'the backward kernels are built for up to {engine.KERNEL_CHANNELS} '
-                f'channels (CHANNELS={emphases.CHANNELS})')
-        batch, _, frames = features.shape
-        wmax = word_bounds.shape[2]
-        with torch.cuda.device(device), _lib.same_stream():
-            input_location = model.location == 'input'
-            if input_location:
-                # every word segment is a packed sequence of max_length rows
-                # (emphases/model/core.py:41-87); the features carry no
-                # gradient, so the gather needs no adjoint
-                from . import segments
-                _, seg_lengths, max_length, lo, count = segments._segment_plan(
-                    word_bounds, word_lengths, frames)
-                rows, row_seq, row_start, n_rows, _, total = segments._gather(
-                    eng, features, lo, count, max_length)
-            else:
-                rows, row_seq, row_start, n_rows, starts, total = \
-                    model_module.pack_batch(eng, features)
-            frame_layers, word_layers = _layer_list(model)
 
-            def layer_forward(x, seq, weight, bias, act):
-                """(output, what emph_activation_backward needs): GELU / SiLU
-                keep the pre-activation, the others their output"""
-                if act in (_lib.ACT_GELU, _lib.ACT_SILU):
-                    pre = eng.conv_stack(
-                        x, seq, _stack(weight, bias, _lib.ACT_NONE, device),
-                        _lib.PREC_FP32)
-                    y = torch.empty_like(pre)
-                    _lib.call(
-                        'emph_activation_forward', _lib.ptr(pre), _lib.ptr(seq),
-                        pre.shape[0], pre.shape[1], act, _lib.ptr(y),
-                        _lib.stream_ptr())
-                    return y, pre
-                y = eng.conv_stack(
-                    x, seq, _stack(weight, bias, act, device), _lib.PREC_FP32)
-                return y, y
+def _conv_backward(eng, layers, acts, keys, row_seq, dy, grads):
+    """Adjoint of conv layers run by _layer_forward: weight and bias gradients
+    into `grads`, returns the gradient of the first layer's input"""
+    device = dy.device
+    channels = dy.shape[1]
+    for position in range(len(layers) - 1, -1, -1):
+        weight, bias, act = layers[position]
+        x_in, y_out = acts[position], keys[position]
+        dpre = torch.empty_like(dy)
+        _lib.call(
+            'emph_activation_backward', _lib.ptr(dy), _lib.ptr(y_out),
+            _lib.ptr(row_seq), dy.shape[0], channels, act,
+            _lib.ptr(dpre), _lib.stream_ptr())
+        kernel = weight.shape[2]
+        dw = torch.empty(
+            (kernel, channels, channels), dtype=torch.float32,
+            device=device)
+        db = torch.empty(channels, dtype=torch.float32, device=device)
+        _lib.call(
+            'emph_conv_weight_grad', _lib.ptr(x_in), _lib.ptr(dpre),
+            dy.shape[0], channels, kernel, _lib.ptr(dw), _lib.ptr(db),
+            _lib.stream_ptr())
+        grads[weight] = dw.permute(2, 1, 0).contiguous()
+        grads[bias] = db
+        dy = eng.conv_stack(
+            dpre, row_seq,
+            _stack(weight, bias, act, device, backward=True),
+            _lib.PREC_FP32)
+    return dy
 
-            frame_acts, frame_keys = [rows], []
-            for weight, bias, act in frame_layers:
-                y, key = layer_forward(frame_acts[-1], row_seq, weight, bias, act)
-                frame_acts.append(y)
-                frame_keys.append(key)
-            weights = model.packed_weights()
-            if model.location == 'inference':
-                # frame-resolution logits (model/core.py:119-122)
-                logits, _ = eng.head(
-                    frame_acts[-1], row_seq, weights, _lib.HEAD_LOGITS,
-                    want_scores=False)
-                index = model_module.slot_index(starts, frames, device)
-                ctx.model = model
-                ctx.saved = dict(
-                    frame_acts=frame_acts, frame_keys=frame_keys,
-                    row_seq=row_seq, index=index,
-                    total=total, head_weight=weights.head_weight,
-                    head_kernel=weights.head_kernel, frame_level=True)
-                return logits[index][:, None, :]
-            if input_location:
-                views, word_starts, total_words = segments.input_word_rows(
-                    batch, wmax, seg_lengths, count, max_length, method, device)
-            else:
-                views, word_starts, total_words, bounds, lengths = \
-                    model_module.word_rows(word_bounds, word_lengths, device)
-            pooled = eng.pool(
-                frame_acts[-1], row_start, n_rows, views['word_seq'],
-                views['word_lo'], views['word_hi'], method)
-            word_row_seq = eng.row_index(
-                views['word_row_start'], views['n_words'], batch, total_words)
-            word_acts, word_keys = [pooled], []
-            for weight, bias, act in word_layers:
-                y, key = layer_forward(word_acts[-1], word_row_seq, weight, bias, act)
-                word_acts.append(y)
-                word_keys.append(key)
+
+def _conv_encoders(eng, model, device):
+    """(encode, decode, encode_backward, decode_backward) of the conv model
+    for _model_forward / _model_backward: the frame layers (input layer
+    included) and the word layers.  The conv layers read every packed row,
+    so the sequence counts go unread."""
+    frame_layers, word_layers = _layer_list(model)
+
+    def run(layers):
+        def forward(x, row_seq, row_start, n_queries, n_keys):
+            acts, keys = [x], []
+            for weight, bias, act in layers:
+                y, key = _layer_forward(eng, acts[-1], row_seq, weight, bias, act, device)
+                acts.append(y)
+                keys.append(key)
+            return acts[-1], (acts, keys, row_seq)
+
+        def backward(saved, dy, grads):
+            acts, keys, row_seq = saved
+            return _conv_backward(eng, layers, acts, keys, row_seq, dy, grads)
+        return forward, backward
+
+    encode, encode_backward = run(frame_layers)
+    decode, decode_backward = run(word_layers)
+    return encode, decode, encode_backward, decode_backward
+
+
+def _transformer_encoders(eng, model, device, seed):
+    """The same four functions for the Transformer variant: the input layer and
+    the frame encoder, and the word decoder (transformer.stack_forward_train /
+    stack_backward), dropout drawn from `seed`"""
+    from . import transformer
+    tables = model.packed_weights()
+    input_layer = [(model.input_layer.weight, model.input_layer.bias, _lib.ACT_NONE)]
+
+    def encode(rows, row_seq, row_start, n_queries, n_keys):
+        embedded, key = _layer_forward(eng, rows, row_seq, *input_layer[0], device)
+        out, saved = transformer.stack_forward_train(
+            model.frame_encoder, tables.frame.table, embedded, row_start, n_queries,
+            n_keys, row_seq, seed, 0)
+        return out, ([rows, embedded], [key], row_seq, saved)
+
+    def encode_backward(saved, dy, grads):
+        acts, keys, row_seq, stack = saved
+        d_embedded, stack_grads = transformer.stack_backward(stack, dy)
+        grads.update(stack_grads)
+        return _conv_backward(eng, input_layer, acts, keys, row_seq, d_embedded, grads)
+
+    def decode(pooled, word_row_seq, word_start, n_queries, n_keys):
+        if not hasattr(model, 'word_decoder'):
+            return pooled, None
+        return transformer.stack_forward_train(
+            model.word_decoder, tables.word.table, pooled, word_start, n_queries,
+            n_keys, word_row_seq, seed, 1)
+
+    def decode_backward(saved, dy, grads):
+        if saved is None:
+            return dy
+        d_pooled, stack_grads = transformer.stack_backward(saved, dy)
+        grads.update(stack_grads)
+        return d_pooled
+
+    return encode, decode, encode_backward, decode_backward
+
+
+def _model_forward(ctx, model, features, frame_lengths, word_bounds, word_lengths, encoders):
+    """Training forward on packed rows for both architectures, with the encoder
+    functions of _conv_encoders / _transformer_encoders; keeps in ctx.saved
+    what _model_backward reads"""
+    from . import model as model_module
+    device = features.device
+    eng = emphases.get_engine(device)
+    method = emphases.DOWNSAMPLE_METHOD
+    if method not in _lib.POOL:
+        raise ValueError(f'Interpolation method {method} is not defined')
+    if emphases.CHANNELS > engine.KERNEL_CHANNELS:
+        raise NotImplementedError(
+            f'the backward kernels are built for up to {engine.KERNEL_CHANNELS} '
+            f'channels (CHANNELS={emphases.CHANNELS})')
+    batch, _, frames = features.shape
+    wmax = word_bounds.shape[2]
+    with torch.cuda.device(device), _lib.same_stream():
+        encode, decode, _, _ = encoders(eng, model, device)
+        input_location = model.location == 'input'
+        if input_location:
+            # every word segment is a packed sequence of max_length rows
+            # (emphases/model/core.py:41-87) that attends over its own
+            # frames; the features carry no gradient, so the gather needs
+            # no adjoint
+            from . import segments
+            _, word_counts, max_length, lo, count = segments._segment_plan(
+                word_bounds, word_lengths, frames)
+            rows, row_seq, row_start, n_rows, _, total = segments._gather(
+                eng, features, lo, count, max_length)
+            n_queries, n_keys = np.full(lo.size, max_length), count.reshape(-1)
+        else:
+            rows, row_seq, row_start, n_rows, starts, total = \
+                model_module.pack_batch(eng, features)
+            n_queries = np.full(batch, frames)
+            n_keys = None if frame_lengths is None else \
+                frame_lengths.detach().to('cpu', torch.int64).numpy()
+        frame_rows, frame_saved = encode(rows, row_seq, row_start, n_queries, n_keys)
+        weights = model.packed_weights()
+        if model.location == 'inference':
+            # frame-resolution logits (model/core.py:119-122)
             logits, _ = eng.head(
-                word_acts[-1], word_row_seq, weights, _lib.HEAD_LOGITS,
+                frame_rows, row_seq, weights, _lib.HEAD_LOGITS,
                 want_scores=False)
-            index = model_module.slot_index(word_starts, wmax, device)
-        ctx.model = model
-        ctx.saved = dict(
-            frame_acts=frame_acts, word_acts=word_acts, frame_keys=frame_keys,
-            word_keys=word_keys, row_seq=row_seq,
-            word_row_seq=word_row_seq, row_start=row_start, n_rows=n_rows,
-            views=views, index=index, total=total, total_words=total_words,
-            method=method, head_weight=weights.head_weight,
-            head_kernel=weights.head_kernel, frame_level=False)
-        return logits[index][:, None, :]
+            index = model_module.slot_index(starts, frames, device)
+            ctx.model = model
+            ctx.saved = dict(
+                frame_saved=frame_saved, frame_rows=frame_rows,
+                row_seq=row_seq, index=index,
+                total=total, head_weight=weights.head_weight,
+                head_kernel=weights.head_kernel, frame_level=True)
+            return logits[index][:, None, :]
+        if input_location:
+            views, word_starts, total_words = segments.input_word_rows(
+                batch, wmax, word_counts, count, max_length, method, device)
+        else:
+            views, word_starts, total_words, bounds, word_counts = \
+                model_module.word_rows(word_bounds, word_lengths, device)
+        pooled = eng.pool(
+            frame_rows, row_start, n_rows, views['word_seq'],
+            views['word_lo'], views['word_hi'], method)
+        word_row_seq = eng.row_index(
+            views['word_row_start'], views['n_words'], batch, total_words)
+        word_rows, word_saved = decode(
+            pooled, word_row_seq, views['word_row_start'], np.full(batch, wmax),
+            word_counts)
+        logits, _ = eng.head(
+            word_rows, word_row_seq, weights, _lib.HEAD_LOGITS,
+            want_scores=False)
+        index = model_module.slot_index(word_starts, wmax, device)
+    ctx.model = model
+    ctx.saved = dict(
+        frame_saved=frame_saved, word_saved=word_saved, frame_rows=frame_rows,
+        word_rows=word_rows, row_seq=row_seq,
+        word_row_seq=word_row_seq, row_start=row_start, n_rows=n_rows,
+        views=views, index=index, total=total, total_words=total_words,
+        method=method, head_weight=weights.head_weight,
+        head_kernel=weights.head_kernel, frame_level=False)
+    return logits[index][:, None, :]
 
-    @staticmethod
-    def backward(ctx, grad_logits):
-        model, s = ctx.model, ctx.saved
-        device = grad_logits.device
-        eng = emphases.get_engine(device)
-        channels = s['frame_acts'][0].shape[1]
-        frame_level = s['frame_level']
-        with torch.cuda.device(device), _lib.same_stream():
-            rows = s['total'] if frame_level else s['total_words']
-            head_seq = s['row_seq'] if frame_level else s['word_row_seq']
-            dz = torch.zeros(rows, dtype=torch.float32, device=device)
-            dz[s['index'].reshape(-1)] = grad_logits.reshape(-1).to(torch.float32)
-            frame_layers, word_layers = _layer_list(model)
-            grads = {}
 
-            # output projection
-            x = s['frame_acts'][-1] if frame_level else s['word_acts'][-1]
-            dx = torch.empty_like(x)
-            dw = torch.empty_like(s['head_weight'])
-            db = torch.empty(1, dtype=torch.float32, device=device)
-            _lib.call(
-                'emph_output_head_backward', _lib.ptr(x), _lib.ptr(dz),
-                _lib.ptr(head_seq), rows, channels,
-                s['head_kernel'], _lib.ptr(s['head_weight']), _lib.ptr(dx),
-                _lib.ptr(dw), _lib.ptr(db), _lib.stream_ptr())
-            grads[model.output_layer.weight] = dw.t()[None].contiguous()
-            grads[model.output_layer.bias] = db
+def _model_backward(ctx, grad_logits, encoders):
+    """Gradients of every parameter, in model.parameters() order"""
+    model, s = ctx.model, ctx.saved
+    device = grad_logits.device
+    eng = emphases.get_engine(device)
+    channels = s['frame_rows'].shape[1]
+    frame_level = s['frame_level']
+    with torch.cuda.device(device), _lib.same_stream():
+        _, _, encode_backward, decode_backward = encoders(eng, model, device)
+        rows = s['total'] if frame_level else s['total_words']
+        head_seq = s['row_seq'] if frame_level else s['word_row_seq']
+        dz = torch.zeros(rows, dtype=torch.float32, device=device)
+        dz[s['index'].reshape(-1)] = grad_logits.reshape(-1).to(torch.float32)
+        grads = {}
 
-            def conv_backward(layers, acts, keys, row_seq, dy):
-                for position in range(len(layers) - 1, -1, -1):
-                    weight, bias, act = layers[position]
-                    x_in, y_out = acts[position], keys[position]
-                    dpre = torch.empty_like(dy)
-                    _lib.call(
-                        'emph_activation_backward', _lib.ptr(dy), _lib.ptr(y_out),
-                        _lib.ptr(row_seq), dy.shape[0], channels, act,
-                        _lib.ptr(dpre), _lib.stream_ptr())
-                    kernel = weight.shape[2]
-                    dw = torch.empty(
-                        (kernel, channels, channels), dtype=torch.float32,
-                        device=device)
-                    db = torch.empty(channels, dtype=torch.float32, device=device)
-                    _lib.call(
-                        'emph_conv_weight_grad', _lib.ptr(x_in), _lib.ptr(dpre),
-                        dy.shape[0], channels, kernel, _lib.ptr(dw), _lib.ptr(db),
-                        _lib.stream_ptr())
-                    grads[weight] = dw.permute(2, 1, 0).contiguous()
-                    grads[bias] = db
-                    dy = eng.conv_stack(
-                        dpre, row_seq,
-                        _stack(weight, bias, act, device, backward=True),
-                        _lib.PREC_FP32)
-                return dy
+        # output projection
+        x = s['frame_rows'] if frame_level else s['word_rows']
+        dx = torch.empty_like(x)
+        dw = torch.empty_like(s['head_weight'])
+        db = torch.empty(1, dtype=torch.float32, device=device)
+        _lib.call(
+            'emph_output_head_backward', _lib.ptr(x), _lib.ptr(dz),
+            _lib.ptr(head_seq), rows, channels,
+            s['head_kernel'], _lib.ptr(s['head_weight']), _lib.ptr(dx),
+            _lib.ptr(dw), _lib.ptr(db), _lib.stream_ptr())
+        grads[model.output_layer.weight] = dw.t()[None].contiguous()
+        grads[model.output_layer.bias] = db
 
-            if frame_level:
-                conv_backward(
-                    frame_layers, s['frame_acts'], s['frame_keys'], s['row_seq'], dx)
-                ordered = [
-                    grads[p].to(p.dtype) if p in grads else None
-                    for p in model.parameters()]
-                return (None, None, None, None, *ordered)
-            d_pooled = conv_backward(
-                word_layers, s['word_acts'], s['word_keys'], s['word_row_seq'], dx)
-            d_frames = torch.empty_like(s['frame_acts'][-1])
+        if frame_level:
+            encode_backward(s['frame_saved'], dx, grads)
+        else:
+            d_pooled = decode_backward(s['word_saved'], dx, grads)
+            d_frames = torch.empty_like(s['frame_rows'])
             views = s['views']
             _lib.call(
                 'emph_pool_words_backward', _lib.ptr(d_pooled),
-                _lib.ptr(s['frame_acts'][-1]), channels, _lib.ptr(s['row_start']),
+                _lib.ptr(s['frame_rows']), channels, _lib.ptr(s['row_start']),
                 _lib.ptr(s['n_rows']), _lib.ptr(views['word_seq']),
                 _lib.ptr(views['word_lo']), _lib.ptr(views['word_hi']),
                 s['total_words'], _lib.POOL[s['method']], s['total'],
                 _lib.ptr(d_frames), _lib.stream_ptr())
-            conv_backward(
-                frame_layers, s['frame_acts'], s['frame_keys'], s['row_seq'], d_frames)
-        ordered = [
-            grads[p].to(p.dtype) if p in grads else None
-            for p in model.parameters()]
-        return (None, None, None, None, *ordered)
+            encode_backward(s['frame_saved'], d_frames, grads)
+    return [
+        grads[p].to(p.dtype) if p in grads else None
+        for p in model.parameters()]
+
+
+class _ConvModelFunction(torch.autograd.Function):
+
+    @staticmethod
+    def forward(ctx, model, features, word_bounds, word_lengths, *parameters):
+        if model.architecture != 'convolution':
+            raise NotImplementedError(
+                'the training step is built for the convolution architecture')
+        return _model_forward(
+            ctx, model, features, None, word_bounds, word_lengths, _conv_encoders)
+
+    @staticmethod
+    def backward(ctx, grad_logits):
+        return (None, None, None, None, *_model_backward(ctx, grad_logits, _conv_encoders))
+
+
+class _TransformerModelFunction(torch.autograd.Function):
+    """Training forward and backward of the Transformer variant, with the
+    reference's dropout: one seed per forward, drawn from torch's default CPU
+    generator (no device sync; torch.manual_seed makes a step reproducible),
+    from which the backward regenerates every mask"""
+
+    @staticmethod
+    def forward(ctx, model, features, frame_lengths, word_bounds, word_lengths, *parameters):
+        seed = int(torch.randint(0, 2 ** 62, ()))
+        ctx.seed = seed
+        return _model_forward(
+            ctx, model, features, frame_lengths, word_bounds, word_lengths,
+            lambda eng, model, device: _transformer_encoders(eng, model, device, seed))
+
+    @staticmethod
+    def backward(ctx, grad_logits):
+        seed = ctx.seed
+        return (None, None, None, None, None, *_model_backward(
+            ctx, grad_logits,
+            lambda eng, model, device: _transformer_encoders(eng, model, device, seed)))
 
 
 ###############################################################################
@@ -461,6 +556,10 @@ def forward_with_grad(model, features, frame_lengths, word_bounds, word_lengths)
             word_bounds.detach().to('cpu', torch.int64).numpy(),
             word_lengths.detach().to('cpu', torch.int64).numpy(),
             features.shape[2], method)
+    if model.architecture == 'transformer':
+        return _TransformerModelFunction.apply(
+            model, features, frame_lengths, word_bounds, word_lengths,
+            *model.parameters())
     if native_step_supported(model, features):
         return _NativeConvFunction.apply(
             model, features, frame_lengths, word_bounds, word_lengths,

@@ -452,3 +452,250 @@ def encoders(eng, weights):
             word_row_seq, eng.device, tag='word_')
 
     return encode, decode
+
+
+###############################################################################
+# Training: forward with saved activations, and its backward
+###############################################################################
+
+TRAIN_CHANNELS = 80              # the training kernels are built for 40-dim heads
+KEY_BLOCK = 64                   # kBwdRows of csrc/attention.cu
+
+
+def _f32(tensor):
+    return tensor.detach().to(torch.float32).contiguous()
+
+
+def dropout_rates(module):
+    """p of the five dropout sites of one TransformerEncoderLayer container,
+    read from its modules (a model set to p = 0 trains without dropout)"""
+    return [
+        [layer.self_attn.dropout, layer.dropout1.p, layer.dropout.p, layer.dropout2.p]
+        for layer in module.model.layers]
+
+
+def stack_forward_train(
+    module, table, x, row_start, n_queries, n_keys, row_seq, seed, stack
+):
+    """Training forward of one Transformer container (`frame_encoder` or
+    `word_decoder`, stack 0 / 1 of the dropout sites) on packed rows x: the
+    positional encoding, then per layer post-norm self-attention and
+    feed-forward with the reference's five dropout sites.  Sequence u has
+    n_queries[u] rows (host), of which the first n_keys[u] are keys.
+    Returns (rows, saved): saved keeps per layer only what stack_backward
+    reads (layer input, q / k / v, attention output and log-sum-exp, the
+    LayerNorm sums and statistics, the feed-forward activation); the dropout
+    masks are regenerated from `seed`."""
+    total_rows, channels = x.shape
+    if channels != TRAIN_CHANNELS:
+        raise NotImplementedError(
+            f'the Transformer training kernels are built for {TRAIN_CHANNELS} channels')
+    if int(np.max(n_queries, initial=0)) > table.shape[0]:
+        raise RuntimeError(
+            f'The size of tensor a ({int(np.max(n_queries))}) must match the '
+            f'size of tensor b ({table.shape[0]}) at non-singleton '
+            'dimension 0 (positional encoding table, transformer.py:52)')
+    device = x.device
+    n_seq = len(n_queries)
+    blocks = [query_blocks(n_queries), query_blocks(n_keys, KEY_BLOCK),
+              query_blocks(n_queries, KEY_BLOCK)]
+    parts = [np.asarray(n_queries, dtype=np.int32), np.asarray(n_keys, dtype=np.int32)]
+    for sequence, first in blocks:
+        parts += [sequence, first]
+    meta = torch.from_numpy(np.concatenate(parts)).to(device)
+    cursor, views = 0, []
+    for part in parts:
+        views.append(meta[cursor:cursor + len(part)])
+        cursor += len(part)
+    geometry = dict(
+        row_start=row_start, row_seq=row_seq, n_queries=views[0], n_keys=views[1],
+        forward_blocks=(views[2], views[3], len(blocks[0][0])),
+        key_blocks=(views[4], views[5], len(blocks[1][0])),
+        query_blocks=(views[6], views[7], len(blocks[2][0])),
+        scale=1.0 / math.sqrt(channels // HEADS), seq=n_seq)
+    rates = dropout_rates(module)
+    p_position = float(module.position.dropout.p)
+    stream = _lib.stream_ptr()
+
+    def site(layer, kind):
+        return _lib.dropout_site(stack, layer, kind)
+
+    def empty(*shape):
+        return torch.empty(shape, dtype=torch.float32, device=device)
+
+    h = empty(total_rows, channels)
+    _lib.call(
+        'emph_add_positional', _lib.ptr(x), _lib.ptr(row_start), _lib.ptr(row_seq),
+        total_rows, channels, _lib.ptr(table), table.shape[0], _lib.ptr(h), stream)
+    _lib.call(
+        'emph_dropout_rows', _lib.ptr(h), total_rows, channels, seed,
+        site(0, _lib.DROPOUT_POSITIONAL), p_position, _lib.ptr(h), stream)
+    saved = []
+    for index, layer in enumerate(module.model.layers):
+        p_attention, p_1, p_feedforward, p_2 = rates[index]
+        qkv = empty(3, total_rows, channels)
+        _lib.call(
+            'emph_linear_rows', _lib.ptr(h), total_rows, channels,
+            _lib.ptr(_f32(layer.self_attn.in_proj_weight)),
+            _lib.ptr(_f32(layer.self_attn.in_proj_bias)), 3, _lib.ACT_NONE,
+            _lib.ptr(row_seq), _lib.ptr(qkv), stream)
+        context = empty(total_rows, channels)
+        lse = empty(total_rows, HEADS)
+        block_seq, block_q0, n_blocks = geometry['forward_blocks']
+        _lib.call(
+            'emph_attention_rows_train', _lib.ptr(qkv[0]), _lib.ptr(qkv[1]),
+            _lib.ptr(qkv[2]), channels, HEADS, _lib.ptr(row_start),
+            _lib.ptr(geometry['n_queries']), _lib.ptr(geometry['n_keys']),
+            _lib.ptr(row_seq), total_rows, _lib.ptr(block_seq), _lib.ptr(block_q0),
+            n_blocks, geometry['scale'], seed, site(index, _lib.DROPOUT_ATTENTION),
+            p_attention, _lib.ptr(context), _lib.ptr(lse), stream)
+        attended = empty(total_rows, channels)
+        _lib.call(
+            'emph_linear_rows', _lib.ptr(context), total_rows, channels,
+            _lib.ptr(_f32(layer.self_attn.out_proj.weight)),
+            _lib.ptr(_f32(layer.self_attn.out_proj.bias)), 1, _lib.ACT_NONE,
+            _lib.ptr(row_seq), _lib.ptr(attended), stream)
+        normed, sums1, stats1 = empty(total_rows, channels), empty(total_rows, channels), \
+            empty(total_rows, 2)
+        _lib.call(
+            'emph_add_layernorm_train', _lib.ptr(h), _lib.ptr(attended),
+            _lib.ptr(_f32(layer.norm1.weight)), _lib.ptr(_f32(layer.norm1.bias)),
+            layer.norm1.eps, _lib.ptr(row_seq), total_rows, channels, seed,
+            site(index, _lib.DROPOUT_RESIDUAL1), p_1, _lib.ptr(normed), _lib.ptr(sums1),
+            _lib.ptr(stats1), stream)
+        hidden = empty(total_rows, channels)
+        _lib.call(
+            'emph_linear_rows', _lib.ptr(normed), total_rows, channels,
+            _lib.ptr(_f32(layer.linear1.weight)), _lib.ptr(_f32(layer.linear1.bias)), 1,
+            _lib.ACT_RELU, _lib.ptr(row_seq), _lib.ptr(hidden), stream)
+        dropped = empty(total_rows, channels)
+        _lib.call(
+            'emph_dropout_rows', _lib.ptr(hidden), total_rows, channels, seed,
+            site(index, _lib.DROPOUT_FEEDFORWARD), p_feedforward, _lib.ptr(dropped), stream)
+        forward = empty(total_rows, channels)
+        _lib.call(
+            'emph_linear_rows', _lib.ptr(dropped), total_rows, channels,
+            _lib.ptr(_f32(layer.linear2.weight)), _lib.ptr(_f32(layer.linear2.bias)), 1,
+            _lib.ACT_NONE, _lib.ptr(row_seq), _lib.ptr(forward), stream)
+        out, sums2, stats2 = empty(total_rows, channels), empty(total_rows, channels), \
+            empty(total_rows, 2)
+        _lib.call(
+            'emph_add_layernorm_train', _lib.ptr(normed), _lib.ptr(forward),
+            _lib.ptr(_f32(layer.norm2.weight)), _lib.ptr(_f32(layer.norm2.bias)),
+            layer.norm2.eps, _lib.ptr(row_seq), total_rows, channels, seed,
+            site(index, _lib.DROPOUT_RESIDUAL2), p_2, _lib.ptr(out), _lib.ptr(sums2),
+            _lib.ptr(stats2), stream)
+        saved.append(dict(
+            x=h, qkv=qkv, context=context, lse=lse, normed=normed, sums1=sums1,
+            stats1=stats1, hidden=hidden, sums2=sums2, stats2=stats2))
+        h = out
+    return h, dict(
+        module=module, layers=saved, geometry=geometry, seed=seed, stack=stack,
+        rates=rates, p_position=p_position)
+
+
+def stack_backward(saved, d_rows):
+    """Adjoint of stack_forward_train: (gradient of its input rows, {parameter:
+    gradient}) from the gradient of its output rows"""
+    module, g = saved['module'], saved['geometry']
+    seed, stack = saved['seed'], saved['stack']
+    total_rows, channels = d_rows.shape
+    device = d_rows.device
+    row_seq = g['row_seq']
+    stream = _lib.stream_ptr()
+    grads = {}
+
+    def site(layer, kind):
+        return _lib.dropout_site(stack, layer, kind)
+
+    def empty(*shape):
+        return torch.empty(shape, dtype=torch.float32, device=device)
+
+    partials = empty(_lib.load().emph_layernorm_backward_blocks(total_rows), 2 * channels)
+
+    def weight_grad(x, dy, dw, db):
+        """dw [in][out] (the Linear gradient transposed), db [out]"""
+        _lib.call(
+            'emph_conv_weight_grad', _lib.ptr(x), _lib.ptr(dy), total_rows, channels, 1,
+            _lib.ptr(dw), _lib.ptr(db), stream)
+
+    def norm_backward(dy, sums, stats, norm, kind, p, index):
+        dx, d_branch = empty(total_rows, channels), empty(total_rows, channels)
+        dgamma, dbeta = empty(channels), empty(channels)
+        _lib.call(
+            'emph_add_layernorm_backward', _lib.ptr(dy), _lib.ptr(sums), _lib.ptr(stats),
+            _lib.ptr(_f32(norm.weight)), _lib.ptr(row_seq), total_rows, channels, seed,
+            site(index, kind), p, _lib.ptr(dx), _lib.ptr(d_branch), _lib.ptr(dgamma),
+            _lib.ptr(dbeta), _lib.ptr(partials), stream)
+        grads[norm.weight], grads[norm.bias] = dgamma, dbeta
+        return dx, d_branch
+
+    def linear_backward(x, dy, linear):
+        """weight / bias gradient of one Linear, and dy W"""
+        dw, db = empty(channels, channels), empty(channels)
+        weight_grad(x, dy, dw, db)
+        grads[linear.weight], grads[linear.bias] = dw.t().contiguous(), db
+        dx = empty(total_rows, channels)
+        _lib.call(
+            'emph_linear_rows_backward', _lib.ptr(dy), total_rows, channels,
+            _lib.ptr(_f32(linear.weight)), 1, None, _lib.ptr(row_seq), _lib.ptr(dx), stream)
+        return dx
+
+    d = d_rows.contiguous()
+    for index in range(len(saved['layers']) - 1, -1, -1):
+        layer, s = module.model.layers[index], saved['layers'][index]
+        p_attention, p_1, p_feedforward, p_2 = saved['rates'][index]
+        # h2 = LayerNorm2(h1 + dropout2(linear2(dropout(relu(linear1(h1))))))
+        d_normed, d_forward = norm_backward(
+            d, s['sums2'], s['stats2'], layer.norm2, _lib.DROPOUT_RESIDUAL2, p_2, index)
+        dropped = empty(total_rows, channels)
+        _lib.call(
+            'emph_dropout_rows', _lib.ptr(s['hidden']), total_rows, channels, seed,
+            site(index, _lib.DROPOUT_FEEDFORWARD), p_feedforward, _lib.ptr(dropped), stream)
+        d_dropped = linear_backward(dropped, d_forward, layer.linear2)
+        _lib.call(
+            'emph_dropout_rows', _lib.ptr(d_dropped), total_rows, channels, seed,
+            site(index, _lib.DROPOUT_FEEDFORWARD), p_feedforward, _lib.ptr(d_dropped), stream)
+        d_pre = empty(total_rows, channels)
+        _lib.call(
+            'emph_activation_backward', _lib.ptr(d_dropped), _lib.ptr(s['hidden']),
+            _lib.ptr(row_seq), total_rows, channels, _lib.ACT_RELU, _lib.ptr(d_pre), stream)
+        dw, db = empty(channels, channels), empty(channels)
+        weight_grad(s['normed'], d_pre, dw, db)
+        grads[layer.linear1.weight], grads[layer.linear1.bias] = dw.t().contiguous(), db
+        d_h1 = empty(total_rows, channels)
+        _lib.call(
+            'emph_linear_rows_backward', _lib.ptr(d_pre), total_rows, channels,
+            _lib.ptr(_f32(layer.linear1.weight)), 1, _lib.ptr(d_normed), _lib.ptr(row_seq),
+            _lib.ptr(d_h1), stream)
+        # h1 = LayerNorm1(h + dropout1(out_proj(attention(h))))
+        d_h, d_attended = norm_backward(
+            d_h1, s['sums1'], s['stats1'], layer.norm1, _lib.DROPOUT_RESIDUAL1, p_1, index)
+        d_context = linear_backward(s['context'], d_attended, layer.self_attn.out_proj)
+        qkv, d_qkv = s['qkv'], empty(3, total_rows, channels)
+        key_seq, key_k0, n_key_blocks = g['key_blocks']
+        query_seq, query_q0, n_query_blocks = g['query_blocks']
+        _lib.call(
+            'emph_attention_rows_backward', _lib.ptr(qkv[0]), _lib.ptr(qkv[1]),
+            _lib.ptr(qkv[2]), _lib.ptr(s['context']), _lib.ptr(d_context), _lib.ptr(s['lse']),
+            channels, HEADS, _lib.ptr(g['row_start']), _lib.ptr(g['n_queries']),
+            _lib.ptr(g['n_keys']), total_rows, _lib.ptr(key_seq), _lib.ptr(key_k0),
+            n_key_blocks, _lib.ptr(query_seq), _lib.ptr(query_q0), n_query_blocks,
+            g['scale'], seed, site(index, _lib.DROPOUT_ATTENTION), p_attention,
+            _lib.ptr(d_qkv[0]), _lib.ptr(d_qkv[1]), _lib.ptr(d_qkv[2]), stream)
+        dw, db = empty(3, channels, channels), empty(3 * channels)
+        for part in range(3):
+            weight_grad(s['x'], d_qkv[part], dw[part], db[part * channels:])
+        grads[layer.self_attn.in_proj_weight] = \
+            dw.transpose(1, 2).reshape(3 * channels, channels).contiguous()
+        grads[layer.self_attn.in_proj_bias] = db
+        d = empty(total_rows, channels)
+        _lib.call(
+            'emph_linear_rows_backward', _lib.ptr(d_qkv), total_rows, channels,
+            _lib.ptr(_f32(layer.self_attn.in_proj_weight)), 3, _lib.ptr(d_h),
+            _lib.ptr(row_seq), _lib.ptr(d), stream)
+    # x + PE[:T] under dropout: the positional table is a buffer
+    _lib.call(
+        'emph_dropout_rows', _lib.ptr(d), total_rows, channels, seed,
+        site(0, _lib.DROPOUT_POSITIONAL), saved['p_position'], _lib.ptr(d), stream)
+    return d, grads

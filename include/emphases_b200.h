@@ -501,6 +501,96 @@ int emph_output_head_backward(
 int emph_masked_loss(
     const float* logits, const float* targets, const uint8_t* valid,
     int32_t total_rows, int32_t mode, float* loss, float* dlogits, void* stream);
+
+/*
+ * Training of the Transformer variant (emphases/model/layers/transformer.py:
+ * 13-52 in training mode: dropout after the positional encoding, on the
+ * attention probabilities, on the attention output, inside the feed-forward
+ * block and on its output), fp32, channels 80, 40-dim heads.
+ *
+ * Dropout: Philox4x32-10 keyed by a 64-bit `seed` (one per training forward);
+ * element i of a site keeps its value iff its 32-bit draw >= round(p 2^32),
+ * kept values are scaled by 1 / (1 - p); p = 0 keeps everything, scale 1.
+ * The draw is a function of (seed, site, element index) only, so the
+ * backward regenerates the forward's masks, and emph_dropout_keep writes
+ * keep[i] (1 / 0) for element indices first .. first + count - 1 of any site.
+ *   site  EMPH_DROPOUT_SITE(stack, layer, kind, head): stack 0 frame encoder,
+ *         1 word decoder; the attention kernels add the head themselves
+ *   index row-wise sites: packed_row * channels + channel;
+ *         attention: packed_query_row << 16 | key index within the sequence
+ *
+ *   emph_dropout_rows            y = x * keep / (1 - p), element index = flat
+ *                                index of x (packed rows); its own backward
+ *   emph_linear_rows             y_m = act(x W_m^T + b_m), m < parts: W is the
+ *                                (parts * 80, 80) Linear weight, y is
+ *                                [parts][rows][80]; separator rows zero
+ *   emph_linear_rows_backward    dx = addend + sum_m dy_m W_m (addend may be
+ *                                NULL), dy [parts][rows][80]
+ *   emph_conv_weight_grad        with kernel_size 1: dW^T [in][out] of a Linear
+ *   emph_attention_rows_train    emph_attention_rows with dropout(softmax) V and
+ *                                lse[row * heads + head] = log2-domain
+ *                                log-sum-exp (max + log2 sum) of the scores
+ *                                S * scale * log2(e)
+ *   emph_attention_rows_backward dq, dk, dv from q, k, v, out, d_out, lse (one
+ *                                pass over 64-key blocks, key_block_*, one over
+ *                                64-query blocks, query_block_*: no atomics);
+ *                                rows that are no key get dk = dv = 0, and every
+ *                                row of a sequence without keys NaN (its
+ *                                softmax is NaN)
+ *   emph_add_layernorm_train     emph_add_layernorm with dropout on `residual`;
+ *                                keeps sums = x + dropout(residual) and stats
+ *                                [rows][2] = (mean, rstd)
+ *   emph_add_layernorm_backward  dx = d sums, d_branch = dx * keep / (1 - p),
+ *                                dgamma / dbeta over the non-separator rows via
+ *                                `partials` [emph_layernorm_backward_blocks(rows)]
+ *                                [2 * channels] (per-CTA sums, then one ordered
+ *                                reduction: deterministic)
+ */
+#define EMPH_DROPOUT_SITE(stack, layer, kind, head) \
+    (((uint32_t)(stack) << 24) | ((uint32_t)(layer) << 16) | ((uint32_t)(kind) << 8) | (uint32_t)(head))
+enum {
+    EMPH_DROPOUT_POSITIONAL = 0,   /* position.dropout */
+    EMPH_DROPOUT_ATTENTION = 1,    /* self_attn.dropout, on the probabilities */
+    EMPH_DROPOUT_RESIDUAL1 = 2,    /* dropout1, attention output */
+    EMPH_DROPOUT_FEEDFORWARD = 3,  /* dropout, between linear1 and linear2 */
+    EMPH_DROPOUT_RESIDUAL2 = 4     /* dropout2, feed-forward output */
+};
+int emph_dropout_keep(
+    uint64_t seed, uint32_t site, uint64_t first, int64_t count, float p, uint8_t* keep,
+    void* stream);
+int emph_dropout_rows(
+    const float* x, int32_t total_rows, int32_t channels, uint64_t seed, uint32_t site, float p,
+    float* y, void* stream);
+int emph_linear_rows(
+    const float* x, int32_t total_rows, int32_t channels, const float* weight, const float* bias,
+    int32_t parts, int32_t act, const int32_t* row_seq, float* y, void* stream);
+int emph_linear_rows_backward(
+    const float* dy, int32_t total_rows, int32_t channels, const float* weight, int32_t parts,
+    const float* addend, const int32_t* row_seq, float* dx, void* stream);
+int emph_attention_rows_train(
+    const float* q, const float* k, const float* v, int32_t channels, int32_t heads,
+    const int32_t* row_start, const int32_t* n_queries, const int32_t* n_keys,
+    const int32_t* row_seq, int32_t total_rows,
+    const int32_t* block_seq, const int32_t* block_q0, int32_t n_blocks,
+    float scale, uint64_t seed, uint32_t site, float p, float* out, float* lse, void* stream);
+int emph_attention_rows_backward(
+    const float* q, const float* k, const float* v, const float* out, const float* d_out,
+    const float* lse, int32_t channels, int32_t heads, const int32_t* row_start,
+    const int32_t* n_queries, const int32_t* n_keys, int32_t total_rows,
+    const int32_t* key_block_seq, const int32_t* key_block_k0, int32_t n_key_blocks,
+    const int32_t* query_block_seq, const int32_t* query_block_q0, int32_t n_query_blocks,
+    float scale, uint64_t seed, uint32_t site, float p, float* dq, float* dk, float* dv,
+    void* stream);
+int emph_add_layernorm_train(
+    const float* x, const float* residual, const float* gamma, const float* beta, float eps,
+    const int32_t* row_seq, int32_t total_rows, int32_t channels, uint64_t seed, uint32_t site,
+    float p, float* y, float* sums, float* stats, void* stream);
+int emph_layernorm_backward_blocks(int32_t total_rows);
+int emph_add_layernorm_backward(
+    const float* dy, const float* sums, const float* stats, const float* gamma,
+    const int32_t* row_seq, int32_t total_rows, int32_t channels, uint64_t seed, uint32_t site,
+    float p, float* dx, float* d_branch, float* dgamma, float* dbeta, float* partials,
+    void* stream);
 /*
  * Training-mode forward and backward of the convolution model, ONE call each
  * (emphases/train/core.py:111-142: model(...) and backward() of one step).

@@ -4,14 +4,18 @@ shaped like the reference's collate (B * Tmax <= MAX_TRAINING_FRAMES = 75,000
 frames per GPU, emphases/config/defaults.py:230; utterances U(2, 20) s).
 
     python tools/train_bench.py                                  # 1 GPU
+    python tools/train_bench.py --architecture transformer       # Transformer variant
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N \\
         --master-addr 127.0.0.1 --master-port 29533 tools/train_bench.py
 
 Prints one JSON line: ms per step (CUDA events, max over ranks), frames/s and
 audio-s/s over all ranks (weak scaling: every rank has its own batch), and the
-share of the step spent in the gradient all-reduce.
+share of the step spent in the gradient all-reduce, with the card's name and
+power limit read in the same run.
 """
+import argparse
 import json
+import subprocess
 import os
 import sys
 
@@ -44,7 +48,25 @@ def synthetic_batch(seed, max_frames=75000):
     return (features, torch.tensor(lengths), bounds, torch.tensor(words), targets)
 
 
+def card():
+    """(name, power limit) of the current GPU"""
+    try:
+        index = torch.cuda.current_device()
+        limit = subprocess.run(
+            ['nvidia-smi', f'--id={index}', '--query-gpu=power.limit',
+             '--format=csv,noheader'], capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        limit = 'unknown'
+    return torch.cuda.get_device_name(), limit or 'unknown'
+
+
 def main():
+    parser = argparse.ArgumentParser()
+    parser.add_argument(
+        '--architecture', choices=['convolution', 'transformer'], default='convolution',
+        help='ARCHITECTURE of the trained model (the transformer step trains with the '
+             "reference's dropout, p = 0.1)")
+    args = parser.parse_args()
     rank = int(os.environ.get('RANK', 0))
     local = int(os.environ.get('LOCAL_RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -55,6 +77,7 @@ def main():
         dist.init_process_group('nccl', device_id=device)
     import emphases_b200 as emphases
     emphases.reset_configuration()
+    emphases.configure(ARCHITECTURE=args.architecture)
     torch.manual_seed(0)
     model = emphases.Model().to(device)
     optimizer = torch.optim.Adam(model.parameters(), lr=1e-4)
@@ -103,7 +126,9 @@ def main():
     else:
         frames_total = frames
     if rank == 0:
+        name, power_limit = card()
         print(json.dumps({
+            'architecture': args.architecture, 'gpu': name, 'power_limit': power_limit,
             'metric': 'training step (config 5)', 'n_gpus': world,
             'ms_per_step': ms, 'allreduce_ms': reduce_ms,
             'frames_per_s': frames_total / (ms * 1e-3),
