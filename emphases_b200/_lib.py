@@ -20,7 +20,7 @@ HEAD_LOGITS, HEAD_SIGMOID, HEAD_CLAMP = 0, 1, 2
 PREC_FP32, PREC_BF16_TC, PREC_BF16X3_TC, PREC_BF16X6_TC = 0, 1, 2, 3
 # dropout site kinds (EMPH_DROPOUT_*)
 (DROPOUT_POSITIONAL, DROPOUT_ATTENTION, DROPOUT_RESIDUAL1, DROPOUT_FEEDFORWARD,
- DROPOUT_RESIDUAL2) = range(5)
+ DROPOUT_RESIDUAL2, DROPOUT_CONV) = range(6)
 
 
 def dropout_site(stack, layer, kind, head=0):
@@ -81,6 +81,9 @@ SIGNATURES = {
     'emph_upsample_words': [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P],
     'emph_dropout_keep': [_U64, _U32, _U64, ctypes.c_int64, _F, _P, _P],
     'emph_dropout_rows': [_P, _I, _I, _U64, _U32, _F, _P, _P],
+    'emph_conv_dropout_forward': [_P, _P, _P, _I, _I, _I, _I, _U64, _U32, _F, _P, _P],
+    'emph_activation_dropout_backward': [
+        _P, _P, _P, _P, _I, _I, _I, _I, _U64, _U32, _F, _P, _P],
     'emph_linear_rows': [_P, _I, _I, _P, _P, _I, _I, _P, _P, _P],
     'emph_linear_rows_backward': [_P, _I, _I, _P, _I, _P, _P, _P, _P],
     'emph_attention_rows_train': [
@@ -119,7 +122,8 @@ class TrainModel(ctypes.Structure):
         ('n_frame_layers', _I), ('n_word_layers', _I), ('channels', _I),
         ('kernel_size', _I), ('head_kernel', _I), ('pool_method', _I),
         ('forward_precision', _I), ('precision', _I),
-        ('acts', _P), ('weights', _P), ('biases', _P), ('zero_bias', _P)]
+        ('acts', _P), ('weights', _P), ('biases', _P), ('zero_bias', _P),
+        ('dropout', _P), ('seed', _U64)]
 
 
 ENOSYS = -38        # EMPH_ENOSYS: the configuration is not built / not handled

@@ -12,6 +12,11 @@
 // Element index per site (see EMPH_DROPOUT_SITE in include/emphases_b200.h):
 //   row-wise sites:  packed_row * channels + channel
 //   attention:       packed_query_row << 16 | key index within the sequence
+//   conv blocks:     (n * width + w) * channels + channel (EMPH_DROPOUT_CONV):
+//                    the position in the reference's padded tensor, item or
+//                    segment n = row_seq[r], column w = r - row_start[n], so the
+//                    native step (which skips rows no word reaches) and the
+//                    per-kernel path draw the same mask
 #pragma once
 
 #include <stdint.h>

@@ -9,19 +9,39 @@
 //   dW[tap][ci][co] = sum_r X[r + tap - half][ci] dpre[r][co],  db = sum_r dpre
 //                                             emph_conv_weight_grad
 // plus the backward of word pooling, of the output projection and the masked
-// BCE / MSE loss with its gradient.
+// BCE / MSE loss with its gradient, and the dropout after a layer's activation
+// (emph_conv_dropout_forward / emph_activation_dropout_backward).
 #include <math_constants.h>
 
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "dropout.cuh"
 
 namespace emph {
 
-// dpre = dy * act'(.), separator rows zeroed.  `y` is the layer's OUTPUT for
-// ReLU / LeakyReLU / identity (the sign of the output decides) and the
-// PRE-activation for GELU / SiLU (their derivative is not a function of the
-// output; the training forward keeps it, emph_activation_forward)
+// g * act'(.) at `v`: the layer's OUTPUT for ReLU / LeakyReLU / identity (the
+// sign of the output decides) and the PRE-activation for GELU / SiLU (their
+// derivative is not a function of the output; the training forward keeps it,
+// emph_activation_forward)
+__device__ __forceinline__ float activation_grad(float g, float v, int act) {
+    if (act == EMPH_ACT_RELU) {
+        g = v > 0.f ? g : 0.f;
+    } else if (act == EMPH_ACT_LEAKY_RELU) {
+        g = v > 0.f ? g : 0.01f * g;
+    } else if (act == EMPH_ACT_GELU) {
+        // d/dx [x Phi(x)] = Phi(x) + x phi(x)
+        const float cdf = 0.5f * (1.f + erff(v * 0.70710678118654752f));
+        const float pdf = 0.3989422804014327f * expf(-0.5f * v * v);
+        g *= cdf + v * pdf;
+    } else if (act == EMPH_ACT_SILU) {
+        const float sig = 1.f / (1.f + expf(-v));
+        g *= sig * (1.f + v * (1.f - sig));
+    }
+    return g;
+}
+
+// dpre = dy * act'(.), separator rows zeroed
 __global__ void activation_backward_kernel(
     const float* __restrict__ dy, const float* __restrict__ y,
     const int32_t* __restrict__ row_seq, int total_rows, int channels, int act,
@@ -30,21 +50,7 @@ __global__ void activation_backward_kernel(
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n;
          i += (size_t)gridDim.x * blockDim.x) {
         const int r = (int)(i / channels);
-        float g = dy[i];
-        const float v = y[i];
-        if (act == EMPH_ACT_RELU) {
-            g = v > 0.f ? g : 0.f;
-        } else if (act == EMPH_ACT_LEAKY_RELU) {
-            g = v > 0.f ? g : 0.01f * g;
-        } else if (act == EMPH_ACT_GELU) {
-            // d/dx [x Phi(x)] = Phi(x) + x phi(x)
-            const float cdf = 0.5f * (1.f + erff(v * 0.70710678118654752f));
-            const float pdf = 0.3989422804014327f * expf(-0.5f * v * v);
-            g *= cdf + v * pdf;
-        } else if (act == EMPH_ACT_SILU) {
-            const float sig = 1.f / (1.f + expf(-v));
-            g *= sig * (1.f + v * (1.f - sig));
-        }
+        const float g = activation_grad(dy[i], y[i], act);
         dpre[i] = row_seq[r] >= 0 ? g : 0.f;
     }
 }
@@ -59,6 +65,79 @@ __global__ void activation_forward_kernel(
          i += (size_t)gridDim.x * blockDim.x) {
         const int r = (int)(i / channels);
         y[i] = row_seq[r] >= 0 ? apply_activation(pre[i], act) : 0.f;
+    }
+}
+
+// Dropout after a conv layer's activation (emphases/model/layers/
+// convolution.py:25-30: Conv1d -> activation -> Dropout).  The element index of
+// the mask is the element's position in the reference's padded (N, width, C)
+// tensor, channel fastest:  ((n * width + w) * C + c) with n = row_seq[r] and
+// w = r - row_start[n], so the mask does not depend on how rows are packed.
+// One thread per float4 (four channels of one row: one Philox call, C % 4 == 0).
+
+// y = act(x) * keep / (1 - p), separator rows zeroed.  x may be y (in place).
+__global__ void conv_dropout_forward_kernel(
+    const float4* x, const int32_t* __restrict__ row_seq,
+    const int32_t* __restrict__ row_start, int total_rows, int quads, int width, int act,
+    Dropout drop, float4* y) {
+    const long long n = (long long)total_rows * quads;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+         i += (long long)gridDim.x * blockDim.x) {
+        const int r = (int)(i / quads), q = (int)(i % quads);
+        const int u = row_seq[r];
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (u >= 0) {
+            v = x[i];
+            v.x = apply_activation(v.x, act);
+            v.y = apply_activation(v.y, act);
+            v.z = apply_activation(v.z, act);
+            v.w = apply_activation(v.w, act);
+            if (drop.threshold != 0ull) {
+                const unsigned long long group =
+                    ((unsigned long long)u * width + (r - row_start[u])) * quads + q;
+                const uint4 draws = philox_draws(drop.seed, drop.site, group);
+                v.x *= dropout_factor(drop, draws, 4 * group);
+                v.y *= dropout_factor(drop, draws, 4 * group + 1);
+                v.z *= dropout_factor(drop, draws, 4 * group + 2);
+                v.w *= dropout_factor(drop, draws, 4 * group + 3);
+            }
+        }
+        y[i] = v;
+    }
+}
+
+// dpre = dy * keep / (1 - p) * act'(.), the mask regenerated from the seed;
+// `y` as for activation_grad.  For ReLU / LeakyReLU the kept output is the
+// dropped one: where the mask keeps an element its sign is the activation's,
+// and where it drops one the factor is 0.
+__global__ void activation_dropout_backward_kernel(
+    const float4* __restrict__ dy, const float4* __restrict__ y,
+    const int32_t* __restrict__ row_seq, const int32_t* __restrict__ row_start, int total_rows,
+    int quads, int width, int act, Dropout drop, float4* __restrict__ dpre) {
+    const long long n = (long long)total_rows * quads;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+         i += (long long)gridDim.x * blockDim.x) {
+        const int r = (int)(i / quads), q = (int)(i % quads);
+        const int u = row_seq[r];
+        float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (u >= 0) {
+            g = dy[i];
+            const float4 v = y[i];
+            if (drop.threshold != 0ull) {
+                const unsigned long long group =
+                    ((unsigned long long)u * width + (r - row_start[u])) * quads + q;
+                const uint4 draws = philox_draws(drop.seed, drop.site, group);
+                g.x *= dropout_factor(drop, draws, 4 * group);
+                g.y *= dropout_factor(drop, draws, 4 * group + 1);
+                g.z *= dropout_factor(drop, draws, 4 * group + 2);
+                g.w *= dropout_factor(drop, draws, 4 * group + 3);
+            }
+            g.x = activation_grad(g.x, v.x, act);
+            g.y = activation_grad(g.y, v.y, act);
+            g.z = activation_grad(g.z, v.z, act);
+            g.w = activation_grad(g.w, v.w, act);
+        }
+        dpre[i] = g;
     }
 }
 
@@ -474,6 +553,53 @@ int emph_activation_forward(
     emph::activation_forward_kernel<<<emph::sm_count() * 4, 256, 0, (cudaStream_t)stream>>>(
         pre, row_seq, total_rows, channels, act, y);
     EMPH_CHECK_LAUNCH("emph_activation_forward");
+    return EMPH_OK;
+}
+
+static int conv_dropout_grid(int total_rows, int quads) {
+    long long blocks = ((long long)total_rows * quads + 255) / 256;
+    if (blocks > emph::sm_count() * 8) blocks = emph::sm_count() * 8;
+    return (int)blocks;
+}
+
+int emph_conv_dropout_forward(
+    const float* x, const int32_t* row_seq, const int32_t* row_start, int32_t total_rows,
+    int32_t channels, int32_t width, int32_t act, uint64_t seed, uint32_t site, float p,
+    float* y, void* stream) {
+    EMPH_REQUIRE(act >= EMPH_ACT_NONE && act <= EMPH_ACT_SILU,
+                 "emph_conv_dropout_forward: unknown activation %d", act);
+    EMPH_REQUIRE(total_rows >= 0 && channels > 0 && channels % 4 == 0 && width > 0 &&
+                     p >= 0.f && p <= 1.f,
+                 "emph_conv_dropout_forward: rows %d, channels %d, width %d, p %f",
+                 total_rows, channels, width, p);
+    if (total_rows == 0) return EMPH_OK;
+    const int quads = channels / 4;
+    emph::conv_dropout_forward_kernel<<<conv_dropout_grid(total_rows, quads), 256, 0,
+                                        (cudaStream_t)stream>>>(
+        reinterpret_cast<const float4*>(x), row_seq, row_start, total_rows, quads, width, act,
+        emph::make_dropout(seed, site, p), reinterpret_cast<float4*>(y));
+    EMPH_CHECK_LAUNCH("emph_conv_dropout_forward");
+    return EMPH_OK;
+}
+
+int emph_activation_dropout_backward(
+    const float* dy, const float* y, const int32_t* row_seq, const int32_t* row_start,
+    int32_t total_rows, int32_t channels, int32_t width, int32_t act, uint64_t seed,
+    uint32_t site, float p, float* dpre, void* stream) {
+    EMPH_REQUIRE(act >= EMPH_ACT_NONE && act <= EMPH_ACT_SILU,
+                 "emph_activation_dropout_backward: unknown activation %d", act);
+    EMPH_REQUIRE(total_rows >= 0 && channels > 0 && channels % 4 == 0 && width > 0 &&
+                     p >= 0.f && p <= 1.f,
+                 "emph_activation_dropout_backward: rows %d, channels %d, width %d, p %f",
+                 total_rows, channels, width, p);
+    if (total_rows == 0) return EMPH_OK;
+    const int quads = channels / 4;
+    emph::activation_dropout_backward_kernel<<<conv_dropout_grid(total_rows, quads), 256, 0,
+                                               (cudaStream_t)stream>>>(
+        reinterpret_cast<const float4*>(dy), reinterpret_cast<const float4*>(y), row_seq,
+        row_start, total_rows, quads, width, act, emph::make_dropout(seed, site, p),
+        reinterpret_cast<float4*>(dpre));
+    EMPH_CHECK_LAUNCH("emph_activation_dropout_backward");
     return EMPH_OK;
 }
 

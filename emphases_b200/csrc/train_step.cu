@@ -12,6 +12,15 @@
 // kernel, or the split-bf16 tensor-core kernel (bf16x3 / bf16x6, fp32-grade)
 // for the forward and the input-gradient passes.  Weight gradients run on the
 // split-bf16 mma.sync kernel in every mode (16-bit operands, fp32 accumulate).
+//
+// Dropout (the reference's Conv1d -> activation -> Dropout blocks): a layer
+// with p > 0 runs emph_conv_dropout_forward after its convolution, in place on
+// the activated output (ReLU / LeakyReLU / identity) or in place of
+// emph_activation_forward (GELU / SiLU, whose pre-activation stays kept).  Its
+// output buffer then holds the dropped values that pooling and the next layer
+// read, and the backward uses emph_activation_dropout_backward, which
+// regenerates the mask from the seed: nothing else is stored, and the
+// backward launches no extra kernel.
 #include <vector>
 
 #include "common.cuh"
@@ -87,6 +96,19 @@ struct TrainLayout {
 };
 
 static bool keeps_pre(int act) { return act == EMPH_ACT_GELU || act == EMPH_ACT_SILU; }
+
+// p of the dropout after layer `index` (0: none; the input layer has none)
+static float dropout_p(const emph_train_model& m, int index) {
+    return m.dropout && index > 0 ? m.dropout[index] : 0.f;
+}
+
+// dropout site of layer `index`: frame encoder block index - 1, word decoder
+// block index - n_frame_layers
+static uint32_t dropout_site(const emph_train_model& m, int index) {
+    const bool word = index >= m.n_frame_layers;
+    return EMPH_DROPOUT_SITE(word ? 1 : 0, word ? index - m.n_frame_layers : index - 1,
+                             EMPH_DROPOUT_CONV, 0);
+}
 
 // Rows kept per item.  The reference convolves all `frames` padded columns of
 // every item (emphases/model/layers/convolution.py:36-37 ignores the lengths),
@@ -177,6 +199,9 @@ static int check_model(const emph_train_model& m) {
         EMPH_REQUIRE(precision == EMPH_PREC_FP32 || precision == EMPH_PREC_BF16X3_TC ||
                          precision == EMPH_PREC_BF16X6_TC,
                      "emph_train_*: precision %d (fp32, bf16x3 or bf16x6)", precision);
+    for (int i = 1; m.dropout && i < m.n_frame_layers + m.n_word_layers; ++i)
+        EMPH_REQUIRE(m.dropout[i] >= 0.f && m.dropout[i] < 1.f,
+                     "emph_train_*: dropout p %f after layer %d", m.dropout[i], i);
     return EMPH_OK;
 }
 
@@ -279,33 +304,46 @@ extern "C" int emph_train_forward(
 
     // ---- layers, every output kept ----
     if ((s = pack_direction(m, l, base, false, stream))) return s;
+    // `starts` / `width`: the sequences' first rows and the reference's padded
+    // width, which place a row in the dropout masks
     auto run_stack = [&](int first, int count, const float* input, const int32_t* seq, int rows,
+                         const int32_t* starts, int width,
                          const std::vector<size_t>& out, const std::vector<size_t>& pre) -> int {
         const float* x = input;
         for (int i = 0; i < count; ++i) {
             const int act = m.acts[first + i];
+            const float p = dropout_p(m, first + i);
             int status;
             if (keeps_pre(act)) {
                 status = conv_layer(m, l, base, x, seq, rows, first + i, m.biases[first + i],
                                     EMPH_ACT_NONE, false, floats(pre[i]), stream);
-                if (status == EMPH_OK)
+                if (status == EMPH_OK && p > 0.f)
+                    status = emph_conv_dropout_forward(
+                        floats(pre[i]), seq, starts, rows, kTrainChannels, width, act, m.seed,
+                        dropout_site(m, first + i), p, floats(out[i]), stream);
+                else if (status == EMPH_OK)
                     status = emph_activation_forward(floats(pre[i]), seq, rows, kTrainChannels, act,
                                                      floats(out[i]), stream);
             } else {
                 status = conv_layer(m, l, base, x, seq, rows, first + i, m.biases[first + i],
                                     act, false, floats(out[i]), stream);
+                if (status == EMPH_OK && p > 0.f)
+                    status = emph_conv_dropout_forward(
+                        floats(out[i]), seq, starts, rows, kTrainChannels, width, EMPH_ACT_NONE,
+                        m.seed, dropout_site(m, first + i), p, floats(out[i]), stream);
             }
             if (status != EMPH_OK) return status;
             x = floats(out[i]);
         }
         return EMPH_OK;
     };
-    if ((s = run_stack(0, l.n_frame, floats(l.rows), ints(l.row_seq), l.total, l.frame_out, l.frame_pre))) return s;
+    if ((s = run_stack(0, l.n_frame, floats(l.rows), ints(l.row_seq), l.total, ints(l.row_start),
+                       frames, l.frame_out, l.frame_pre))) return s;
     if ((s = emph_pool_words(floats(l.frame_out.back()), kTrainChannels, ints(l.row_start), ints(l.n_rows),
                              ints(l.word_seq), ints(l.word_lo), ints(l.word_hi), l.total_words,
                              m.pool_method, floats(l.pooled), stream))) return s;
     if ((s = run_stack(l.n_frame, l.n_word, floats(l.pooled), ints(l.word_row_seq), l.total_words,
-                       l.word_out, l.word_pre))) return s;
+                       ints(l.word_row_start), wmax, l.word_out, l.word_pre))) return s;
     const float* head_in = l.n_word ? floats(l.word_out.back()) : floats(l.pooled);
     // output layer: Conv1d (1, C, k) weight -> [k][C], bias from device memory
     float* head_w = floats(l.head_w);
@@ -364,12 +402,18 @@ extern "C" int emph_train_backward(
     // conv stacks, last layer first; dy in `dx`, result back in `dx`
     if ((s = pack_direction(m, l, base, true, stream))) return s;
     auto stack_backward = [&](int first, int count, const float* input, const int32_t* seq, int rows,
+                              const int32_t* starts, int width,
                               const std::vector<size_t>& out, const std::vector<size_t>& pre) -> int {
         for (int i = count - 1; i >= 0; --i) {
             const int act = m.acts[first + i];
-            const float* x_in = i ? floats(out[i - 1]) : input;
-            int status = emph_activation_backward(dx, floats(pre[i]), seq, rows, kTrainChannels, act,
-                                                  other, stream);                  // dpre
+            const float p = dropout_p(m, first + i);
+            const float* x_in = i ? floats(out[i - 1]) : input;       // dropped, as the forward read it
+            int status = p > 0.f
+                ? emph_activation_dropout_backward(dx, floats(pre[i]), seq, starts, rows,
+                                                   kTrainChannels, width, act, m.seed,
+                                                   dropout_site(m, first + i), p, other, stream)
+                : emph_activation_backward(dx, floats(pre[i]), seq, rows, kTrainChannels, act,
+                                           other, stream);                          // dpre
             if (status != EMPH_OK) return status;
             // straight into the parameters' gradients, (out, in, k) and (out)
             status = conv1d_weight_grad(x_in, other, rows, kTrainChannels, kTrainKernel,
@@ -386,12 +430,14 @@ extern "C" int emph_train_backward(
     };
     if (l.n_word) {
         if ((s = stack_backward(l.n_frame, l.n_word, floats(l.pooled), ints(l.word_row_seq),
-                                l.total_words, l.word_out, l.word_pre))) return s;
+                                l.total_words, ints(l.word_row_start), wmax, l.word_out,
+                                l.word_pre))) return s;
     }
     // pooling adjoint: d pooled (in dx) -> d frames (in other), then swap roles
     if ((s = emph_pool_words_backward(dx, floats(l.frame_out.back()), kTrainChannels, ints(l.row_start),
                                       ints(l.n_rows), ints(l.word_seq), ints(l.word_lo), ints(l.word_hi),
                                       l.total_words, m.pool_method, l.total, other, stream))) return s;
     std::swap(dx, other);
-    return stack_backward(0, l.n_frame, floats(l.rows), ints(l.row_seq), l.total, l.frame_out, l.frame_pre);
+    return stack_backward(0, l.n_frame, floats(l.rows), ints(l.row_seq), l.total, ints(l.row_start),
+                          frames, l.frame_out, l.frame_pre);
 }

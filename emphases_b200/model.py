@@ -119,18 +119,19 @@ class Model(torch.nn.Module):
                 '(there is no CPU fallback)')
         if self.input_layer.in_channels != emphases.NUM_MELS:
             emphases.require_mel_features_only()
-        if self.training and self.dropout is not None:
-            # the reference applies torch.nn.Dropout after every activation in
-            # training mode (emphases/model/layers/convolution.py:29-30)
-            raise NotImplementedError(
-                'dropout is not implemented in the training-mode forward: set '
-                'DROPOUT=None or call model.eval()')
         if torch.is_grad_enabled() and any(
             p.requires_grad for p in self.parameters()
         ) and self.training:
             from . import training
             return training.forward_with_grad(
                 self, features, frame_lengths, word_bounds, word_lengths)
+        if self.training and self.dropout is not None:
+            # the reference applies torch.nn.Dropout after every activation in
+            # training mode (emphases/model/layers/convolution.py:29-30); the
+            # training step (autograd on) applies it, the inference kernels do not
+            raise NotImplementedError(
+                'dropout is not implemented in a training-mode forward without '
+                'autograd: enable gradients, set DROPOUT=None or call model.eval()')
         with torch.cuda.device(features.device):
             return run_forward(
                 self, features, frame_lengths, word_bounds, word_lengths)

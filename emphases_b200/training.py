@@ -37,6 +37,29 @@ def _layer_list(model):
     return frame, word
 
 
+def _dropout_rates(model):
+    """p of the Dropout after each layer of _layer_list, read from the modules
+    (a model whose modules are set to p = 0 trains without dropout); the input
+    layer has none (emphases/model/layers/convolution.py:25-30)"""
+    if model.dropout is None:
+        frame, word = _layer_list(model)
+        return [0.] * len(frame), [0.] * len(word)
+    frame = [0.] + [float(model.frame_encoder[3 * i + 2].p) for i in range(model.layers)]
+    word = []
+    if hasattr(model, 'word_decoder'):
+        word = [float(model.word_decoder[3 * i + 2].p) for i in range(model.layers)]
+    return frame, word
+
+
+def _draw_seed(model):
+    """One dropout seed per training forward from torch's default CPU
+    generator (no device sync; torch.manual_seed makes a step reproducible);
+    None, and no draw, for a model without dropout modules"""
+    if model.architecture == 'convolution' and model.dropout is None:
+        return None
+    return int(torch.randint(0, 2 ** 62, ()))
+
+
 def _stack(weight, bias, act, device, backward=False):
     """One-layer ConvStack; backward=True packs the adjoint (taps flipped,
     channel matrix transposed) with zero bias and no activation"""
@@ -68,35 +91,59 @@ def _zero_bias(channels, device):
     return _zero_biases[key]
 
 
-def _layer_forward(eng, x, seq, weight, bias, act, device):
-    """One conv layer of the training forward: (output, what
+def _conv_dropout(x, seq, act, drop, y):
+    """y = act(x) * keep / (1 - p) (emph_conv_dropout_forward); `drop` is
+    (seed, site, p, device row_start, width)"""
+    seed, site, p, row_start, width = drop
+    _lib.call(
+        'emph_conv_dropout_forward', _lib.ptr(x), _lib.ptr(seq), _lib.ptr(row_start),
+        x.shape[0], x.shape[1], width, act, seed, site, p, _lib.ptr(y), _lib.stream_ptr())
+
+
+def _layer_forward(eng, x, seq, weight, bias, act, device, drop=None):
+    """One conv layer of the training forward, with the dropout `drop` of
+    _conv_dropout after it (None: none): (output, what
     emph_activation_backward needs): GELU / SiLU keep the pre-activation, the
-    others their output"""
+    others their (dropped) output"""
     if act in (_lib.ACT_GELU, _lib.ACT_SILU):
         pre = eng.conv_stack(
             x, seq, _stack(weight, bias, _lib.ACT_NONE, device), _lib.PREC_FP32)
         y = torch.empty_like(pre)
-        _lib.call(
-            'emph_activation_forward', _lib.ptr(pre), _lib.ptr(seq),
-            pre.shape[0], pre.shape[1], act, _lib.ptr(y), _lib.stream_ptr())
+        if drop is not None:
+            _conv_dropout(pre, seq, act, drop, y)
+        else:
+            _lib.call(
+                'emph_activation_forward', _lib.ptr(pre), _lib.ptr(seq),
+                pre.shape[0], pre.shape[1], act, _lib.ptr(y), _lib.stream_ptr())
         return y, pre
     y = eng.conv_stack(x, seq, _stack(weight, bias, act, device), _lib.PREC_FP32)
+    if drop is not None:
+        _conv_dropout(y, seq, _lib.ACT_NONE, drop, y)
     return y, y
 
 
-def _conv_backward(eng, layers, acts, keys, row_seq, dy, grads):
-    """Adjoint of conv layers run by _layer_forward: weight and bias gradients
-    into `grads`, returns the gradient of the first layer's input"""
+def _conv_backward(eng, layers, acts, keys, row_seq, dy, grads, drops=None):
+    """Adjoint of conv layers run by _layer_forward (`drops`: their dropout,
+    the masks regenerated): weight and bias gradients into `grads`, returns
+    the gradient of the first layer's input"""
     device = dy.device
     channels = dy.shape[1]
     for position in range(len(layers) - 1, -1, -1):
         weight, bias, act = layers[position]
         x_in, y_out = acts[position], keys[position]
         dpre = torch.empty_like(dy)
-        _lib.call(
-            'emph_activation_backward', _lib.ptr(dy), _lib.ptr(y_out),
-            _lib.ptr(row_seq), dy.shape[0], channels, act,
-            _lib.ptr(dpre), _lib.stream_ptr())
+        drop = drops[position] if drops else None
+        if drop is not None:
+            seed, site, p, row_start, width = drop
+            _lib.call(
+                'emph_activation_dropout_backward', _lib.ptr(dy), _lib.ptr(y_out),
+                _lib.ptr(row_seq), _lib.ptr(row_start), dy.shape[0], channels, width, act,
+                seed, site, p, _lib.ptr(dpre), _lib.stream_ptr())
+        else:
+            _lib.call(
+                'emph_activation_backward', _lib.ptr(dy), _lib.ptr(y_out),
+                _lib.ptr(row_seq), dy.shape[0], channels, act,
+                _lib.ptr(dpre), _lib.stream_ptr())
         kernel = weight.shape[2]
         dw = torch.empty(
             (kernel, channels, channels), dtype=torch.float32,
@@ -115,29 +162,42 @@ def _conv_backward(eng, layers, acts, keys, row_seq, dy, grads):
     return dy
 
 
-def _conv_encoders(eng, model, device):
+def _conv_encoders(eng, model, device, seed=None):
     """(encode, decode, encode_backward, decode_backward) of the conv model
     for _model_forward / _model_backward: the frame layers (input layer
-    included) and the word layers.  The conv layers read every packed row,
-    so the sequence counts go unread."""
+    included) and the word layers, with dropout drawn from `seed`.  The conv
+    layers read every packed row, so the key counts go unread; every sequence
+    has n_queries[0] rows, the padded width that places a row in the dropout
+    masks (T, max_length at 'input', or Wmax)."""
     frame_layers, word_layers = _layer_list(model)
+    frame_rates, word_rates = _dropout_rates(model)
 
-    def run(layers):
+    def run(layers, rates, stack):
+        # frame stack: layer 0 is the input layer, block i - 1 of frame_encoder
+        first_block = -1 if stack == 0 else 0
+
         def forward(x, row_seq, row_start, n_queries, n_keys):
-            acts, keys = [x], []
-            for weight, bias, act in layers:
-                y, key = _layer_forward(eng, acts[-1], row_seq, weight, bias, act, device)
+            width = max(int(n_queries[0]), 1) if len(n_queries) else 1
+            acts, keys, drops = [x], [], []
+            for i, ((weight, bias, act), p) in enumerate(zip(layers, rates)):
+                drop = None
+                if p > 0:
+                    site = _lib.dropout_site(stack, first_block + i, _lib.DROPOUT_CONV)
+                    drop = (seed, site, p, row_start, width)
+                y, key = _layer_forward(
+                    eng, acts[-1], row_seq, weight, bias, act, device, drop)
                 acts.append(y)
                 keys.append(key)
-            return acts[-1], (acts, keys, row_seq)
+                drops.append(drop)
+            return acts[-1], (acts, keys, row_seq, drops)
 
         def backward(saved, dy, grads):
-            acts, keys, row_seq = saved
-            return _conv_backward(eng, layers, acts, keys, row_seq, dy, grads)
+            acts, keys, row_seq, drops = saved
+            return _conv_backward(eng, layers, acts, keys, row_seq, dy, grads, drops)
         return forward, backward
 
-    encode, encode_backward = run(frame_layers)
-    decode, decode_backward = run(word_layers)
+    encode, encode_backward = run(frame_layers, frame_rates, 0)
+    decode, decode_backward = run(word_layers, word_rates, 1)
     return encode, decode, encode_backward, decode_backward
 
 
@@ -307,18 +367,26 @@ def _model_backward(ctx, grad_logits, encoders):
 
 
 class _ConvModelFunction(torch.autograd.Function):
+    """Per-kernel training step of the conv model; a model with dropout
+    modules draws one seed per forward (_draw_seed), from which the backward
+    regenerates the masks"""
 
     @staticmethod
     def forward(ctx, model, features, word_bounds, word_lengths, *parameters):
         if model.architecture != 'convolution':
             raise NotImplementedError(
                 'the training step is built for the convolution architecture')
+        seed = ctx.seed = _draw_seed(model)
         return _model_forward(
-            ctx, model, features, None, word_bounds, word_lengths, _conv_encoders)
+            ctx, model, features, None, word_bounds, word_lengths,
+            lambda eng, model, device: _conv_encoders(eng, model, device, seed))
 
     @staticmethod
     def backward(ctx, grad_logits):
-        return (None, None, None, None, *_model_backward(ctx, grad_logits, _conv_encoders))
+        seed = ctx.seed
+        return (None, None, None, None, *_model_backward(
+            ctx, grad_logits,
+            lambda eng, model, device: _conv_encoders(eng, model, device, seed)))
 
 
 class _TransformerModelFunction(torch.autograd.Function):
@@ -329,8 +397,7 @@ class _TransformerModelFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, model, features, frame_lengths, word_bounds, word_lengths, *parameters):
-        seed = int(torch.randint(0, 2 ** 62, ()))
-        ctx.seed = seed
+        seed = ctx.seed = _draw_seed(model)
         return _model_forward(
             ctx, model, features, frame_lengths, word_bounds, word_lengths,
             lambda eng, model, device: _transformer_encoders(eng, model, device, seed))
@@ -384,6 +451,7 @@ class _NativeState:
         self.zero_bias = torch.zeros(engine.KERNEL_CHANNELS, dtype=torch.float32, device=device)
         self.acts = np.ascontiguousarray(
             np.asarray([act for _, _, act in self.layers], dtype=np.int32))
+        self.dropout = np.zeros(len(self.layers), dtype=np.float32)
         count = len(self.layers) + 1
         self.weight_pointers = (ctypes.c_void_p * count)()
         self.bias_pointers = (ctypes.c_void_p * count)()
@@ -474,6 +542,14 @@ class _NativeConvFunction(torch.autograd.Function):
         frame_lengths = torch.from_numpy(np.maximum(
             frame_lengths.detach().to('cpu', torch.int64).numpy(), reach))
         descriptor = state.descriptor
+        ctx.seed = _draw_seed(model)
+        if ctx.seed is None:
+            descriptor.dropout, descriptor.seed = None, 0
+        else:
+            frame_rates, word_rates = _dropout_rates(model)
+            state.dropout[:] = frame_rates + word_rates
+            ctx.dropout = state.dropout.copy()
+            descriptor.dropout, descriptor.seed = state.dropout.ctypes.data, ctx.seed
         descriptor.pool_method = _lib.POOL[emphases.DOWNSAMPLE_METHOD]
         descriptor.forward_precision, descriptor.precision = _TRAIN_PRECISIONS[TRAIN_PRECISION]
         need = state.lib.emph_train_workspace(ctypes.byref(descriptor), batch, frames, wmax)
@@ -526,6 +602,11 @@ class _NativeConvFunction(torch.autograd.Function):
         views = state.views(target)
         for i, view in enumerate(views):
             state.grad_pointers[i] = view.data_ptr()
+        if ctx.seed is not None:
+            # the descriptor is shared: the masks are this forward's
+            state.dropout[:] = ctx.dropout
+            state.descriptor.dropout = state.dropout.ctypes.data
+            state.descriptor.seed = ctx.seed
         with torch.cuda.device(device):
             stream = torch._C._cuda_getCurrentRawStream(device.index)
             status = state.lib.emph_train_backward(

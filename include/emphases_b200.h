@@ -501,6 +501,32 @@ int emph_output_head_backward(
 int emph_masked_loss(
     const float* logits, const float* targets, const uint8_t* valid,
     int32_t total_rows, int32_t mode, float* loss, float* dlogits, void* stream);
+/*
+ * Dropout of the convolution model (emphases/model/layers/convolution.py:
+ * 25-30: Conv1d -> activation -> Dropout(p) in every block of frame_encoder and
+ * word_decoder), with the masks of EMPH_DROPOUT_CONV sites (see the dropout
+ * comment below).  Rows are packed sequences: sequence n = row_seq[r] (-1 on
+ * separator rows) starts at row_start[n] and stands for item (or segment) n of
+ * the reference's padded tensor of `width` columns (T, max_length at the
+ * 'input' location, or Wmax); channels % 4 == 0.
+ *   emph_conv_dropout_forward        y = act(x) * keep / (1 - p), separators
+ *                                    zero; with EMPH_ACT_NONE in place on a conv
+ *                                    output whose activation is applied, with
+ *                                    GELU / SiLU on the kept pre-activation
+ *   emph_activation_dropout_backward dpre = dy * keep / (1 - p) * act'(.), the
+ *                                    mask regenerated; `y` as for
+ *                                    emph_activation_backward, where the output
+ *                                    of ReLU / LeakyReLU / identity layers is
+ *                                    the dropped output
+ */
+int emph_conv_dropout_forward(
+    const float* x, const int32_t* row_seq, const int32_t* row_start, int32_t total_rows,
+    int32_t channels, int32_t width, int32_t act, uint64_t seed, uint32_t site, float p,
+    float* y, void* stream);
+int emph_activation_dropout_backward(
+    const float* dy, const float* y, const int32_t* row_seq, const int32_t* row_start,
+    int32_t total_rows, int32_t channels, int32_t width, int32_t act, uint64_t seed,
+    uint32_t site, float p, float* dpre, void* stream);
 
 /*
  * Training of the Transformer variant (emphases/model/layers/transformer.py:
@@ -515,9 +541,17 @@ int emph_masked_loss(
  * backward regenerates the forward's masks, and emph_dropout_keep writes
  * keep[i] (1 / 0) for element indices first .. first + count - 1 of any site.
  *   site  EMPH_DROPOUT_SITE(stack, layer, kind, head): stack 0 frame encoder,
- *         1 word decoder; the attention kernels add the head themselves
+ *         1 word decoder; the attention kernels add the head themselves.  The
+ *         convolution model's blocks use EMPH_DROPOUT_CONV with `layer` the
+ *         block index in its stack and head 0 (no dropout on input_layer or
+ *         output_layer)
  *   index row-wise sites: packed_row * channels + channel;
- *         attention: packed_query_row << 16 | key index within the sequence
+ *         attention: packed_query_row << 16 | key index within the sequence;
+ *         conv blocks: (n * width + w) * channels + channel, the element's
+ *         position in the reference's padded (N, C, width) tensor taken
+ *         channel fastest (n the item or segment, w its column), so any
+ *         packing of the rows draws the same mask, and emph_dropout_keep over
+ *         0 .. N * width * channels - 1 returns it in (N, width, C) order
  *
  *   emph_dropout_rows            y = x * keep / (1 - p), element index = flat
  *                                index of x (packed rows); its own backward
@@ -553,7 +587,8 @@ enum {
     EMPH_DROPOUT_ATTENTION = 1,    /* self_attn.dropout, on the probabilities */
     EMPH_DROPOUT_RESIDUAL1 = 2,    /* dropout1, attention output */
     EMPH_DROPOUT_FEEDFORWARD = 3,  /* dropout, between linear1 and linear2 */
-    EMPH_DROPOUT_RESIDUAL2 = 4     /* dropout2, feed-forward output */
+    EMPH_DROPOUT_RESIDUAL2 = 4,    /* dropout2, feed-forward output */
+    EMPH_DROPOUT_CONV = 5          /* convolution model: after each block's activation */
 };
 int emph_dropout_keep(
     uint64_t seed, uint32_t site, uint64_t first, int64_t count, float p, uint8_t* keep,
@@ -627,6 +662,14 @@ int emph_add_layernorm_backward(
  *   grads     host array of device pointers, two per layer (weight then bias)
  *             in the order above plus the output projection's: gradients in
  *             the parameters' own layouts, written (accumulate = 0) or added
+ *   dropout   host array, p after layer i's activation (one per frame and
+ *             word layer; the input layer's is ignored), or NULL: layer i of
+ *             the frame stack (i >= 1) draws its mask from site
+ *             EMPH_DROPOUT_SITE(0, i - 1, EMPH_DROPOUT_CONV, 0), word layer j
+ *             from (1, j, EMPH_DROPOUT_CONV, 0), keyed by `seed`.  The forward
+ *             keeps the dropped outputs and the backward regenerates the
+ *             masks, so both calls need the same seed.  p = 0 everywhere (or
+ *             NULL) launches no dropout kernel.
  */
 typedef struct {
     int32_t n_frame_layers, n_word_layers, channels, kernel_size, head_kernel;
@@ -637,6 +680,8 @@ typedef struct {
     const float* const* weights;
     const float* const* biases;
     const float* zero_bias;         /* device [channels] zeros */
+    const float* dropout;           /* host [n_frame_layers + n_word_layers] or NULL */
+    uint64_t seed;                  /* dropout key of this step */
 } emph_train_model;
 
 long long emph_train_workspace(

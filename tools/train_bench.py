@@ -5,6 +5,7 @@ frames per GPU, emphases/config/defaults.py:230; utterances U(2, 20) s).
 
     python tools/train_bench.py                                  # 1 GPU
     python tools/train_bench.py --architecture transformer       # Transformer variant
+    python tools/train_bench.py --dropout 0.1                    # conv model, DROPOUT=0.1
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N \\
         --master-addr 127.0.0.1 --master-port 29533 tools/train_bench.py
 
@@ -66,7 +67,13 @@ def main():
         '--architecture', choices=['convolution', 'transformer'], default='convolution',
         help='ARCHITECTURE of the trained model (the transformer step trains with the '
              "reference's dropout, p = 0.1)")
+    parser.add_argument(
+        '--dropout', type=float, default=None,
+        help='DROPOUT of the convolution model (the reference sweeps 0.05 and 0.1); '
+             'default None: no dropout modules')
     args = parser.parse_args()
+    if args.dropout is not None and args.architecture != 'convolution':
+        parser.error('--dropout sets DROPOUT, which only the convolution model reads')
     rank = int(os.environ.get('RANK', 0))
     local = int(os.environ.get('LOCAL_RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -78,6 +85,8 @@ def main():
     import emphases_b200 as emphases
     emphases.reset_configuration()
     emphases.configure(ARCHITECTURE=args.architecture)
+    if args.dropout is not None:
+        emphases.configure(DROPOUT=args.dropout)
     torch.manual_seed(0)
     model = emphases.Model().to(device)
     optimizer = torch.optim.Adam(model.parameters(), lr=1e-4)
@@ -128,7 +137,8 @@ def main():
     if rank == 0:
         name, power_limit = card()
         print(json.dumps({
-            'architecture': args.architecture, 'gpu': name, 'power_limit': power_limit,
+            'architecture': args.architecture, 'dropout': args.dropout,
+            'gpu': name, 'power_limit': power_limit,
             'metric': 'training step (config 5)', 'n_gpus': world,
             'ms_per_step': ms, 'allreduce_ms': reduce_ms,
             'frames_per_s': frames_total / (ms * 1e-3),
