@@ -220,30 +220,53 @@ conv_weight_grad_kernel(
 // ---------------------------------------------------------------------------
 // Weight gradient on the warp-level tensor path (mma.sync m16n8k16, bf16
 // operands split hi + lo, fp32 accumulate): per tap
-//     dW_tap[in][out] = sum_r X[r + tap - 1][in] * dPre[r][out]
+//     dW_tap[in][out] = sum_r X[r + tap - (KS - 1) / 2][in] * dPre[r][out]
 // is a GEMM with the ROW axis as K.  Both operands sit in shared memory as they
 // sit in HBM, [row][channel], converted to a bf16 hi and a bf16 lo plane while
 // they are staged (x = hi + lo to 16 bits; hi*hi + lo*hi + hi*lo keeps the
 // products to ~1.5e-5), and ldmatrix.trans hands out the K-major fragments.
-// A CTA walks a contiguous range of 64-row tiles with the whole 240 x 80
-// result in registers (8 warps x 19-20 m16n8 tiles) and adds it to the
-// gradient once at the end (split-K over CTAs).  This replaces the FFMA kernel
-// above in the training step: ~15 instead of ~110 us per frame layer.
+// A tile stages X rows r0 - (KS - 1) / 2 .. r0 + R - 1 + (KS - 1) / 2 (the
+// halo of every tap) and dPre rows r0 .. r0 + R - 1.
+//
+// Work split.  The result is KS x C/16 (tap, m-tile) strips of C/8 m16n8
+// tiles each (4 floats per lane per tile).  A CTA keeps PER_WARP strips per
+// warp in registers while it walks a contiguous range of 64-row tiles, and
+// adds them to the gradient once at the end (split-K over CTAs, one float
+// atomic per element and CTA).  When the strips do not fit in one CTA they
+// are spread over gridDim.y (SLICES), each slice staging the same tiles:
+//   C = 80:  2 strips per warp (80 accumulators), ceil(5 KS / 16) slices:
+//            k = 3 one slice (15 strips), k = 5 two, k = 7 three;
+//   C = 128: 1 strip per warp (16 n-tiles: 64 accumulators, plus 64
+//            registers of dPre fragments per k-step), so one tap per slice.
+// Only slice 0 sums the bias.  Every slice gets sm_count / SLICES CTAs, so the
+// grid fills the SMs once; <80, 3> keeps its one-slice launch of one CTA per
+// SM.  Rows are padded to LD bf16 = C + 8 (176 B at 80, 272 B at 128: odd
+// multiples of 16 B, so the 8 row addresses of an ldmatrix hit distinct banks).
+// This replaces the FFMA kernel above in the native training step: ~15 instead
+// of ~110 us per frame layer at 80 channels, kernel size 3.
 // ---------------------------------------------------------------------------
 namespace wgrad {
-constexpr int C = 80;
-constexpr int KS = 3;
 constexpr int R = 64;                       // rows per tile (K of the GEMM)
-constexpr int LD = 88;                      // bf16 per smem row: 176 B, ldmatrix conflict-free
-constexpr int XROWS = R + KS - 1;
-constexpr int MT = C / 16;                  // 5 m-tiles per tap
-constexpr int NT = C / 8;                   // 10 n-tiles
-constexpr int ROWSETS = KS * MT;            // 15 (tap, m-tile) strips, dealt to 8 warps
-constexpr int PER_WARP = 2;
 
+template <int C, int KS>
+struct Shape {
+    static constexpr int LD = C + 8;        // bf16 per smem row
+    static constexpr int XROWS = R + KS - 1;
+    static constexpr int HALF = (KS - 1) / 2;
+    static constexpr int MT = C / 16;       // m-tiles per tap
+    static constexpr int NT = C / 8;        // n-tiles
+    static constexpr int ROWSETS = KS * MT; // (tap, m-tile) strips
+    static constexpr int PER_WARP = C <= 80 ? 2 : 1;
+    static constexpr int SLICE = 8 * PER_WARP;                  // strips per CTA
+    static constexpr int SLICES = (ROWSETS + SLICE - 1) / SLICE;
+    static constexpr int C4 = C / 4;        // float4 columns
+    static constexpr int ROW_GROUPS = 256 / C4;                 // staging threads per column
+};
+
+template <int C, int KS>
 struct Smem {
-    __nv_bfloat16 x[2][XROWS][LD];          // [hi / lo][row][channel]
-    __nv_bfloat16 d[2][R][LD];
+    __nv_bfloat16 x[2][Shape<C, KS>::XROWS][Shape<C, KS>::LD];  // [hi / lo][row][channel]
+    __nv_bfloat16 d[2][R][Shape<C, KS>::LD];
     float bias[C];
 };
 
@@ -269,13 +292,16 @@ __device__ __forceinline__ void split_store(__nv_bfloat16* hi, __nv_bfloat16* lo
         make_uint2(*reinterpret_cast<const uint32_t*>(&l0), *reinterpret_cast<const uint32_t*>(&l1));
 }
 
-template <bool CONV1D>
+template <int C, int KS, bool CONV1D>
 __global__ void __launch_bounds__(256)
 conv_weight_grad_mma_kernel(
     const float* __restrict__ x, const float* __restrict__ dpre, int total_rows, int tiles_per_cta,
     float* __restrict__ dw, float* __restrict__ db) {
+    using S = Shape<C, KS>;
+    constexpr int NT = S::NT, MT = S::MT, PER_WARP = S::PER_WARP, C4 = S::C4;
+    constexpr int GROUPS = S::ROW_GROUPS;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
+    Smem<C, KS>& sm = *reinterpret_cast<Smem<C, KS>*>(smem_raw);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     float acc[PER_WARP][NT][4];
 #pragma unroll
@@ -284,38 +310,45 @@ conv_weight_grad_mma_kernel(
         for (int n = 0; n < NT; ++n)
 #pragma unroll
             for (int j = 0; j < 4; ++j) acc[s][n][j] = 0.f;
-    // bias gradient: thread (c4 = tid % 20) sums its 4 channels over rows tid / 20, + 12, ...
+    // bias gradient: thread (c4 = tid % C4) sums its 4 channels over rows
+    // tid / C4, + GROUPS, ...
     float4 bias_acc = make_float4(0.f, 0.f, 0.f, 0.f);
 
     const int n_tiles = (total_rows + R - 1) / R;
     const int first = blockIdx.x * tiles_per_cta;
     const int last = min(first + tiles_per_cta, n_tiles);
-    // strips of this warp: (tap, m-tile) = strip / MT, strip % MT
+    // strips of this warp: (tap, m-tile) = strip / MT, strip % MT; strips
+    // >= ROWSETS do not exist (<80, 3>: strip 15).  Slice 0 sums the bias.
+    const int slice = S::SLICES == 1 ? 0 : blockIdx.y;
+    const bool bias_slice = slice == 0;
     int strip[PER_WARP];
 #pragma unroll
-    for (int s = 0; s < PER_WARP; ++s) strip[s] = warp + 8 * s;         // 0..15; 15 does not exist
+    for (int s = 0; s < PER_WARP; ++s) strip[s] = slice * S::SLICE + warp + 8 * s;
 
     for (int tile = first; tile < last; ++tile) {
         const int r0 = tile * R;
         __syncthreads();
-        // ---- stage X rows r0 - 1 .. r0 + R and dPre rows r0 .. r0 + R - 1, split hi / lo;
-        // thread = (row % 12, float4 column): a fixed column per thread, so the
-        // bias gradient (column sums of dPre) accumulates in registers ----
-        if (tid < 12 * (C / 4)) {
-            const int c4 = tid % (C / 4);
-            for (int r = tid / (C / 4); r < XROWS; r += 12) {
-                const int g = r0 + r - 1;
+        // ---- stage X rows r0 - HALF .. r0 + R - 1 + HALF and dPre rows
+        // r0 .. r0 + R - 1, split hi / lo; thread = (row % GROUPS, float4
+        // column): a fixed column per thread, so the bias gradient (column
+        // sums of dPre) accumulates in registers ----
+        if (tid < GROUPS * C4) {
+            const int c4 = tid % C4;
+            for (int r = tid / C4; r < S::XROWS; r += GROUPS) {
+                const int g = r0 + r - S::HALF;
                 float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (g >= 0 && g < total_rows)
                     v = *reinterpret_cast<const float4*>(x + (size_t)g * C + 4 * c4);
                 split_store(&sm.x[0][r][4 * c4], &sm.x[1][r][4 * c4], v);
             }
-            for (int r = tid / (C / 4); r < R; r += 12) {
+            for (int r = tid / C4; r < R; r += GROUPS) {
                 const int g = r0 + r;
                 float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (g < total_rows)
                     v = *reinterpret_cast<const float4*>(dpre + (size_t)g * C + 4 * c4);
-                bias_acc.x += v.x; bias_acc.y += v.y; bias_acc.z += v.z; bias_acc.w += v.w;
+                if (bias_slice) {
+                    bias_acc.x += v.x; bias_acc.y += v.y; bias_acc.z += v.z; bias_acc.w += v.w;
+                }
                 split_store(&sm.d[0][r][4 * c4], &sm.d[1][r][4 * c4], v);
             }
         }
@@ -323,7 +356,7 @@ conv_weight_grad_mma_kernel(
         // ---- 4 k-steps of 16 rows ----
 #pragma unroll 1
         for (int k0 = 0; k0 < R; k0 += 16) {
-            // B fragments of all 10 n-tiles, hi and lo: x4.trans covers two n-tiles
+            // B fragments of all NT n-tiles, hi and lo: x4.trans covers two n-tiles
             // (matrices: [k0..7][n0..7], [k0+8..15][n0..7], [k0..7][n0+8..15], [k0+8..15][n0+8..15])
             uint32_t bh[NT][2], bl[NT][2];
 #pragma unroll
@@ -338,7 +371,7 @@ conv_weight_grad_mma_kernel(
             }
 #pragma unroll
             for (int s = 0; s < PER_WARP; ++s) {
-                if (strip[s] >= ROWSETS) continue;                 // warp-uniform
+                if (strip[s] >= S::ROWSETS) continue;              // warp-uniform
                 const int tap = strip[s] / MT, m0 = (strip[s] % MT) * 16;
                 // A fragment = X^T: matrices [k0..7][m0..7], [k0..7][m0+8..15],
                 // [k0+8..15][m0..7], [k0+8..15][m0+8..15]; tap t reads buffer row k + t
@@ -360,7 +393,7 @@ conv_weight_grad_mma_kernel(
     const int g = lane >> 2, t = lane & 3;
 #pragma unroll
     for (int s = 0; s < PER_WARP; ++s) {
-        if (strip[s] >= ROWSETS) continue;
+        if (strip[s] >= S::ROWSETS) continue;
         const int tap = strip[s] / MT, m0 = (strip[s] % MT) * 16;
 #pragma unroll
         for (int n = 0; n < NT; ++n) {
@@ -373,12 +406,13 @@ conv_weight_grad_mma_kernel(
             }
         }
     }
-    // bias: the 12 row-groups' column sums -> shared -> the gradient
+    // bias: the GROUPS row-groups' column sums -> shared -> the gradient
+    if (!bias_slice) return;                                    // CTA-uniform
     __syncthreads();
     for (int i = tid; i < C; i += 256) sm.bias[i] = 0.f;
     __syncthreads();
-    if (tid < 12 * (C / 4)) {
-        const int c4 = tid % (C / 4);
+    if (tid < GROUPS * C4) {
+        const int c4 = tid % C4;
         atomicAdd(&sm.bias[4 * c4 + 0], bias_acc.x);
         atomicAdd(&sm.bias[4 * c4 + 1], bias_acc.y);
         atomicAdd(&sm.bias[4 * c4 + 2], bias_acc.z);
@@ -386,6 +420,33 @@ conv_weight_grad_mma_kernel(
     }
     __syncthreads();
     for (int i = tid; i < C; i += 256) atomicAdd(db + i, sm.bias[i]);
+}
+
+// Adds the gradient of `total_rows` rows to dw / db (zeroed by the caller):
+// contiguous ranges of 64-row tiles, sm_count / SLICES CTAs per slice
+template <int C, int KS, bool CONV1D>
+int launch(const float* x, const float* dpre, int total_rows, float* dw, float* db,
+           cudaStream_t st) {
+    using S = Shape<C, KS>;
+    static bool configured = false;         // one attribute call per instantiation
+    if (!configured) {
+        int s = check_cuda(
+            cudaFuncSetAttribute(conv_weight_grad_mma_kernel<C, KS, CONV1D>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)sizeof(Smem<C, KS>)),
+            "weight gradient smem attribute");
+        if (s != EMPH_OK) return s;
+        configured = true;
+    }
+    const int n_tiles = (total_rows + R - 1) / R;
+    const int per_slice = sm_count() / S::SLICES > 0 ? sm_count() / S::SLICES : 1;
+    const int ctas = n_tiles < per_slice ? n_tiles : per_slice;
+    const int tiles_per_cta = (n_tiles + ctas - 1) / ctas;
+    const int grid = (n_tiles + tiles_per_cta - 1) / tiles_per_cta;
+    conv_weight_grad_mma_kernel<C, KS, CONV1D>
+        <<<dim3(grid, S::SLICES), 256, sizeof(Smem<C, KS>), st>>>(
+            x, dpre, total_rows, tiles_per_cta, dw, db);
+    return EMPH_OK;
 }
 }  // namespace wgrad
 
@@ -606,7 +667,14 @@ int emph_activation_dropout_backward(
 int emph_conv_weight_grad(
     const float* x, const float* dpre, int32_t total_rows, int32_t channels,
     int32_t kernel_size, float* dw, float* db, void* stream) {
-    if (!(channels == 80 && (kernel_size == 3 || kernel_size == 1))) {
+    // 80 channels, kernel size 1 / 3: the FFMA kernel (the per-kernel path's
+    // fp32 step and the Linear maps of the Transformer variant); 80 / 5, 7
+    // and 128 / 1, 3, 5, 7: the split-bf16 mma.sync kernel
+    const bool ffma = channels == 80 && (kernel_size == 1 || kernel_size == 3);
+    const bool mma = (channels == 80 && (kernel_size == 5 || kernel_size == 7)) ||
+                     (channels == 128 && (kernel_size == 1 || kernel_size == 3 ||
+                                          kernel_size == 5 || kernel_size == 7));
+    if (!(ffma || mma)) {
         emph::set_error("emph_conv_weight_grad: channels=%d kernel_size=%d not compiled in",
                         channels, kernel_size);
         return EMPH_ENOSYS;
@@ -618,12 +686,30 @@ int emph_conv_weight_grad(
     s = emph::check_cuda(cudaMemsetAsync(db, 0, sizeof(float) * channels, st), "memset db");
     if (s != EMPH_OK) return s;
     if (total_rows == 0) return EMPH_OK;
-    int grid = (total_rows + 63) / 64;
-    if (grid > emph::sm_count() * 2) grid = emph::sm_count() * 2;
-    if (kernel_size == 3)
-        emph::conv_weight_grad_kernel<80, 3, false><<<grid, 256, 0, st>>>(x, dpre, total_rows, dw, db);
-    else        // the Linear maps of the Transformer variant
-        emph::conv_weight_grad_kernel<80, 1, false><<<grid, 256, 0, st>>>(x, dpre, total_rows, dw, db);
+    if (ffma) {
+        int grid = (total_rows + 63) / 64;
+        if (grid > emph::sm_count() * 2) grid = emph::sm_count() * 2;
+        if (kernel_size == 3)
+            emph::conv_weight_grad_kernel<80, 3, false><<<grid, 256, 0, st>>>(
+                x, dpre, total_rows, dw, db);
+        else        // the Linear maps of the Transformer variant
+            emph::conv_weight_grad_kernel<80, 1, false><<<grid, 256, 0, st>>>(
+                x, dpre, total_rows, dw, db);
+    } else {
+        namespace w = emph::wgrad;
+        if (channels == 80)
+            s = kernel_size == 5 ? w::launch<80, 5, false>(x, dpre, total_rows, dw, db, st)
+                                 : w::launch<80, 7, false>(x, dpre, total_rows, dw, db, st);
+        else if (kernel_size == 1)
+            s = w::launch<128, 1, false>(x, dpre, total_rows, dw, db, st);
+        else if (kernel_size == 3)
+            s = w::launch<128, 3, false>(x, dpre, total_rows, dw, db, st);
+        else if (kernel_size == 5)
+            s = w::launch<128, 5, false>(x, dpre, total_rows, dw, db, st);
+        else
+            s = w::launch<128, 7, false>(x, dpre, total_rows, dw, db, st);
+        if (s != EMPH_OK) return s;
+    }
     EMPH_CHECK_LAUNCH("emph_conv_weight_grad");
     return EMPH_OK;
 }
@@ -653,22 +739,8 @@ int conv1d_weight_grad(
     // and halving their number beats the second CTA's latency hiding (measured:
     // 2.015 / 2.049 / 2.20 / 2.36 ms per training step at 1 / 2 / 3 / 4 CTAs per SM)
     // tensor-core kernel: contiguous ranges of 64-row tiles, one CTA per SM
-    const int n_tiles = (total_rows + wgrad::R - 1) / wgrad::R;
-    const int ctas = n_tiles < sm_count() ? n_tiles : sm_count();
-    const int tiles_per_cta = (n_tiles + ctas - 1) / ctas;
-    const int grid = (n_tiles + tiles_per_cta - 1) / tiles_per_cta;
-    static bool configured = false;
-    if (!configured) {
-        int s = check_cuda(
-            cudaFuncSetAttribute(wgrad::conv_weight_grad_mma_kernel<true>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)sizeof(wgrad::Smem)),
-            "conv1d_weight_grad smem attribute");
-        if (s != EMPH_OK) return s;
-        configured = true;
-    }
-    wgrad::conv_weight_grad_mma_kernel<true><<<grid, 256, sizeof(wgrad::Smem), st>>>(
-        x, dpre, total_rows, tiles_per_cta, grad_weight, grad_bias);
+    const int s = wgrad::launch<80, 3, true>(x, dpre, total_rows, grad_weight, grad_bias, st);
+    if (s != EMPH_OK) return s;
     EMPH_CHECK_LAUNCH("conv1d_weight_grad");
     return EMPH_OK;
 }

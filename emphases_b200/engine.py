@@ -443,6 +443,24 @@ def _pack_conv(weight, device):
     return packed
 
 
+def kernel_width(largest):
+    """Channel count the kernels run a model at whose widest conv has
+    `largest` channels: 80, or 128 for wider models"""
+    return KERNEL_CHANNELS if largest <= KERNEL_CHANNELS else WIDE_CHANNELS
+
+
+def pad(tensor, shape):
+    """Zero-pad a weight/bias to the kernels' channel count.  Padded
+    output channels compute act(0) = 0 for every supported activation and
+    padded input channels multiply zeros, so the embedding is exact."""
+    tensor = tensor.detach().to(torch.float32)
+    if tuple(tensor.shape) == tuple(shape):
+        return tensor
+    padded = torch.zeros(shape, dtype=torch.float32, device=tensor.device)
+    padded[tuple(slice(0, n) for n in tensor.shape)] = tensor
+    return padded
+
+
 def pack_weights(state, device, layers, activation, dropout, has_decoder):
     """Reference state_dict (SURVEY.md A.8) -> packed device buffers
 
@@ -452,22 +470,9 @@ def pack_weights(state, device, layers, activation, dropout, has_decoder):
     """
     step = 3 if dropout is not None else 2
     act = ACTIVATIONS[activation]
-    # channel count the kernels are built for: 80, or 128 for wider models
-    largest = max(
+    width = kernel_width(max(
         max(value.shape[0], value.shape[1]) for key, value in state.items()
-        if key.endswith('.weight') and value.dim() == 3)
-    width = KERNEL_CHANNELS if largest <= KERNEL_CHANNELS else WIDE_CHANNELS
-
-    def pad(tensor, shape):
-        """Zero-pad a weight/bias to the kernels' channel count.  Padded
-        output channels compute act(0) = 0 for every supported activation and
-        padded input channels multiply zeros, so the embedding is exact."""
-        tensor = tensor.detach().to(torch.float32)
-        if tuple(tensor.shape) == tuple(shape):
-            return tensor
-        padded = torch.zeros(shape, dtype=torch.float32, device=tensor.device)
-        padded[tuple(slice(0, n) for n in tensor.shape)] = tensor
-        return padded
+        if key.endswith('.weight') and value.dim() == 3))
 
     def stack(first, prefix):
         convs = list(first)

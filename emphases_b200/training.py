@@ -60,25 +60,39 @@ def _draw_seed(model):
     return int(torch.randint(0, 2 ** 62, ()))
 
 
-def _stack(weight, bias, act, device, backward=False):
-    """One-layer ConvStack; backward=True packs the adjoint (taps flipped,
-    channel matrix transposed) with zero bias and no activation"""
+def _kernel_width(model):
+    """Channel count the conv model trains at, by inference's rule
+    (engine.pack_weights): 80, or 128 when its widest conv is wider.  Its
+    weights and biases are zero-padded to it: a padded channel stays zero
+    through every layer, as act(0) = 0 and dropout keeps a zero a zero."""
+    frame, word = _layer_list(model)
+    largest = max(max(w.shape[0], w.shape[1]) for w, _, _ in frame + word)
+    if largest > engine.WIDE_CHANNELS:
+        raise NotImplementedError(
+            f'the training kernels are built for up to {engine.WIDE_CHANNELS} '
+            f'channels (this model has {largest})')
+    return engine.kernel_width(largest)
+
+
+def _stack(weight, bias, act, device, width, backward=False):
+    """One-layer ConvStack at `width` channels (the weight zero-padded to
+    (width, width, k)); backward=True packs the adjoint (taps flipped, channel
+    matrix transposed) with zero bias and no activation"""
+    kernel = weight.shape[2]
+    padded = engine.pad(weight, (width, width, kernel))
     if backward:
-        source = weight.detach().to(device=device, dtype=torch.float32).contiguous()
-        out_channels, in_channels, kernel = source.shape
-        packed = torch.empty(
-            (kernel, out_channels, in_channels), dtype=torch.float32, device=device)
+        source = padded.to(device).contiguous()
+        packed = torch.empty((kernel, width, width), dtype=torch.float32, device=device)
         _lib.call(
-            'emph_pack_conv_weights_adjoint', _lib.ptr(source), out_channels,
-            in_channels, kernel, _lib.ptr(packed), _lib.stream_ptr())
-        bias = _zero_bias(weight.shape[0], device)
+            'emph_pack_conv_weights_adjoint', _lib.ptr(source), width, width, kernel,
+            _lib.ptr(packed), _lib.stream_ptr())
+        bias = _zero_bias(width, device)
         act = _lib.ACT_NONE
     else:
-        packed = engine._pack_conv(weight, device)      # [k][in][out]
-        bias = bias.detach().to(device, torch.float32)
+        packed = engine._pack_conv(padded, device)      # [k][in][out]
+        bias = engine.pad(bias, (width,)).to(device)
     return engine.ConvStack(
-        packed[None], bias[None],
-        np.asarray([act], dtype=np.int32), weight.shape[2], weight.shape[0])
+        packed[None], bias[None], np.asarray([act], dtype=np.int32), kernel, width)
 
 
 _zero_biases = {}
@@ -101,13 +115,14 @@ def _conv_dropout(x, seq, act, drop, y):
 
 
 def _layer_forward(eng, x, seq, weight, bias, act, device, drop=None):
-    """One conv layer of the training forward, with the dropout `drop` of
-    _conv_dropout after it (None: none): (output, what
-    emph_activation_backward needs): GELU / SiLU keep the pre-activation, the
-    others their (dropped) output"""
+    """One conv layer of the training forward on rows `x` of the kernel
+    width, with the dropout `drop` of _conv_dropout after it (None: none):
+    (output, what emph_activation_backward needs): GELU / SiLU keep the
+    pre-activation, the others their (dropped) output"""
+    width = x.shape[1]
     if act in (_lib.ACT_GELU, _lib.ACT_SILU):
         pre = eng.conv_stack(
-            x, seq, _stack(weight, bias, _lib.ACT_NONE, device), _lib.PREC_FP32)
+            x, seq, _stack(weight, bias, _lib.ACT_NONE, device, width), _lib.PREC_FP32)
         y = torch.empty_like(pre)
         if drop is not None:
             _conv_dropout(pre, seq, act, drop, y)
@@ -116,16 +131,18 @@ def _layer_forward(eng, x, seq, weight, bias, act, device, drop=None):
                 'emph_activation_forward', _lib.ptr(pre), _lib.ptr(seq),
                 pre.shape[0], pre.shape[1], act, _lib.ptr(y), _lib.stream_ptr())
         return y, pre
-    y = eng.conv_stack(x, seq, _stack(weight, bias, act, device), _lib.PREC_FP32)
+    y = eng.conv_stack(x, seq, _stack(weight, bias, act, device, width), _lib.PREC_FP32)
     if drop is not None:
         _conv_dropout(y, seq, _lib.ACT_NONE, drop, y)
     return y, y
 
 
-def _conv_backward(eng, layers, acts, keys, row_seq, dy, grads, drops=None):
+def _conv_backward(eng, layers, acts, keys, row_seq, dy, grads, drops=None,
+                   input_grad=True):
     """Adjoint of conv layers run by _layer_forward (`drops`: their dropout,
-    the masks regenerated): weight and bias gradients into `grads`, returns
-    the gradient of the first layer's input"""
+    the masks regenerated): weight and bias gradients into `grads`, sliced
+    from the kernel width to each parameter's shape; returns the gradient of
+    the first layer's input (None without input_grad)"""
     device = dy.device
     channels = dy.shape[1]
     for position in range(len(layers) - 1, -1, -1):
@@ -153,11 +170,14 @@ def _conv_backward(eng, layers, acts, keys, row_seq, dy, grads, drops=None):
             'emph_conv_weight_grad', _lib.ptr(x_in), _lib.ptr(dpre),
             dy.shape[0], channels, kernel, _lib.ptr(dw), _lib.ptr(db),
             _lib.stream_ptr())
-        grads[weight] = dw.permute(2, 1, 0).contiguous()
-        grads[bias] = db
+        out_channels, in_channels, _ = weight.shape
+        grads[weight] = dw.permute(2, 1, 0)[:out_channels, :in_channels].contiguous()
+        grads[bias] = db[:out_channels]
+        if position == 0 and not input_grad:
+            return None
         dy = eng.conv_stack(
             dpre, row_seq,
-            _stack(weight, bias, act, device, backward=True),
+            _stack(weight, bias, act, device, channels, backward=True),
             _lib.PREC_FP32)
     return dy
 
@@ -168,9 +188,13 @@ def _conv_encoders(eng, model, device, seed=None):
     included) and the word layers, with dropout drawn from `seed`.  The conv
     layers read every packed row, so the key counts go unread; every sequence
     has n_queries[0] rows, the padded width that places a row in the dropout
-    masks (T, max_length at 'input', or Wmax)."""
+    masks (T, max_length at 'input', or Wmax).  Every layer runs at the
+    kernel width (_kernel_width): the 80 input features enter a wider model
+    widened, and the masks are drawn over the padded channels.  The frame
+    stack's input gradient is not computed: the features carry none."""
     frame_layers, word_layers = _layer_list(model)
     frame_rates, word_rates = _dropout_rates(model)
+    kernel_width = _kernel_width(model)
 
     def run(layers, rates, stack):
         # frame stack: layer 0 is the input layer, block i - 1 of frame_encoder
@@ -178,6 +202,8 @@ def _conv_encoders(eng, model, device, seed=None):
 
         def forward(x, row_seq, row_start, n_queries, n_keys):
             width = max(int(n_queries[0]), 1) if len(n_queries) else 1
+            if x.shape[1] < kernel_width:
+                x = eng.widen(x, kernel_width)
             acts, keys, drops = [x], [], []
             for i, ((weight, bias, act), p) in enumerate(zip(layers, rates)):
                 drop = None
@@ -193,7 +219,8 @@ def _conv_encoders(eng, model, device, seed=None):
 
         def backward(saved, dy, grads):
             acts, keys, row_seq, drops = saved
-            return _conv_backward(eng, layers, acts, keys, row_seq, dy, grads, drops)
+            return _conv_backward(
+                eng, layers, acts, keys, row_seq, dy, grads, drops, input_grad=stack != 0)
         return forward, backward
 
     encode, encode_backward = run(frame_layers, frame_rates, 0)
@@ -249,10 +276,12 @@ def _model_forward(ctx, model, features, frame_lengths, word_bounds, word_length
     method = emphases.DOWNSAMPLE_METHOD
     if method not in _lib.POOL:
         raise ValueError(f'Interpolation method {method} is not defined')
-    if emphases.CHANNELS > engine.KERNEL_CHANNELS:
+    if model.architecture == 'convolution':
+        _kernel_width(model)                # raises above 128 channels
+    elif model.input_layer.out_channels != engine.KERNEL_CHANNELS:
         raise NotImplementedError(
-            f'the backward kernels are built for up to {engine.KERNEL_CHANNELS} '
-            f'channels (CHANNELS={emphases.CHANNELS})')
+            f'the Transformer variant trains at {engine.KERNEL_CHANNELS} channels '
+            f'(this model has {model.input_layer.out_channels})')
     batch, _, frames = features.shape
     wmax = word_bounds.shape[2]
     with torch.cuda.device(device), _lib.same_stream():
@@ -344,7 +373,8 @@ def _model_backward(ctx, grad_logits, encoders):
             _lib.ptr(head_seq), rows, channels,
             s['head_kernel'], _lib.ptr(s['head_weight']), _lib.ptr(dx),
             _lib.ptr(dw), _lib.ptr(db), _lib.stream_ptr())
-        grads[model.output_layer.weight] = dw.t()[None].contiguous()
+        grads[model.output_layer.weight] = \
+            dw.t()[None, :model.output_layer.in_channels].contiguous()
         grads[model.output_layer.bias] = db
 
         if frame_level:

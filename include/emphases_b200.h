@@ -473,7 +473,15 @@ int emph_add_layernorm(
  *                             forward keeps by running the conv with
  *                             EMPH_ACT_NONE and emph_activation_forward after it
  *   emph_conv_stack           dx = conv(dpre, W flipped and transposed)
- *   emph_conv_weight_grad     dw [k][in][out], db [out] (zeroed, then summed)
+ *   emph_conv_weight_grad     dw [k][in][out], db [out] (zeroed, then summed);
+ *                             channels 80 at kernel sizes 1 / 3: fp32 FFMA
+ *                             kernel; channels 80 at 5 / 7 and 128 at 1 / 3 /
+ *                             5 / 7: split-bf16 mma.sync kernel (hi*hi +
+ *                             lo*hi + hi*lo, fp32 accumulation, ~1e-6 of
+ *                             |X|^T |dPre|); any other shape: EMPH_ENOSYS,
+ *                             nothing launched.  A model narrower than 80 or
+ *                             between 80 and 128 channels trains zero-padded
+ *                             to the next of these widths.
  * emph_pool_words_backward / emph_output_head_backward are the adjoints of
  * emph_pool_words / emph_output_head (logits).  emph_masked_loss: mean BCE-with-
  * logits (mode 0) or squared error (mode 1) over word rows with valid != 0, and

@@ -6,13 +6,20 @@ frames per GPU, emphases/config/defaults.py:230; utterances U(2, 20) s).
     python tools/train_bench.py                                  # 1 GPU
     python tools/train_bench.py --architecture transformer       # Transformer variant
     python tools/train_bench.py --dropout 0.1                    # conv model, DROPOUT=0.1
+    python tools/train_bench.py --channels 128 --encoder-kernel 7  # a hyper-parameter sweep shape
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N \\
         --master-addr 127.0.0.1 --master-port 29533 tools/train_bench.py
 
 Prints one JSON line: ms per step (CUDA events, max over ranks), frames/s and
 audio-s/s over all ranks (weak scaling: every rank has its own batch), and the
 share of the step spent in the gradient all-reduce, with the card's name and
-power limit read in the same run.
+power limit read in the same run.  A convolution model of another shape than
+the default also gets `weight_grad`: the time per layer of emph_conv_weight_grad
+at its kernel width and each kernel size, from CUDA events over 50 launches on
+the batch's packed frame rows, and its useful rate 2 k C^2 rows / time; beside
+it the native step's <80, 3> weight gradient, timed with torch.profiler on the
+same batch (a LAYERS=0 model at 'loss', whose one weight gradient is the input
+layer's over the native step's kept frame rows).
 """
 import argparse
 import json
@@ -61,6 +68,61 @@ def card():
     return torch.cuda.get_device_name(), limit or 'unknown'
 
 
+def time_weight_grad(emphases, width, kernel, rows, launches=50):
+    """(us per launch, rows) of emph_conv_weight_grad on random (rows, width)
+    operands, CUDA events over `launches` launches after a warm-up"""
+    from emphases_b200 import _lib
+    generator = torch.Generator(device='cuda').manual_seed(kernel)
+    x = torch.randn(rows, width, device='cuda', generator=generator)
+    dpre = torch.randn(rows, width, device='cuda', generator=generator)
+    dw = torch.empty(kernel, width, width, device='cuda')
+    db = torch.empty(width, device='cuda')
+
+    def launch():
+        _lib.call('emph_conv_weight_grad', _lib.ptr(x), _lib.ptr(dpre), rows, width, kernel,
+                  _lib.ptr(dw), _lib.ptr(db), _lib.stream_ptr())
+    for _ in range(5):
+        launch()
+    start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    start.record()
+    for _ in range(launches):
+        launch()
+    end.record()
+    torch.cuda.synchronize()
+    return start.elapsed_time(end) * 1e3 / launches
+
+
+def native_weight_grad(emphases, batch, steps=20):
+    """us per launch of the native step's <80, 3> weight gradient and its rows:
+    a LAYERS=0 model at 'loss' runs it once per step, on the input layer"""
+    from torch.profiler import ProfilerActivity, profile
+    emphases.reset_configuration()
+    emphases.configure(LAYERS=0, DOWNSAMPLE_LOCATION='loss')
+    model = emphases.Model().cuda().train()
+    features, frame_lengths, bounds, word_lengths, targets = batch
+    assert emphases.training.native_step_supported(model, features)
+
+    def step():
+        model.zero_grad(set_to_none=True)
+        model(features, frame_lengths, bounds, word_lengths).sum().backward()
+    for _ in range(3):
+        step()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(steps):
+            step()
+        torch.cuda.synchronize()
+    times = [e.device_time for e in prof.events()
+             if e.device_type == torch.autograd.DeviceType.CUDA and
+             'conv_weight_grad_mma_kernel' in e.name]
+    assert len(times) == steps, len(times)
+    # the native step keeps length + 1 rows per item (one frame layer, k = 3)
+    # and one separator row before and after each (csrc/train_step.cu, kept_rows)
+    frames = features.shape[2]
+    rows = 1 + sum(min(frames, int(t) + 1) + 1 for t in frame_lengths)
+    return sum(times) / steps, rows
+
+
 def main():
     parser = argparse.ArgumentParser()
     parser.add_argument(
@@ -71,9 +133,17 @@ def main():
         '--dropout', type=float, default=None,
         help='DROPOUT of the convolution model (the reference sweeps 0.05 and 0.1); '
              'default None: no dropout modules')
+    parser.add_argument('--channels', type=int, default=None, help='CHANNELS (64, 80, 128)')
+    parser.add_argument('--layers', type=int, default=None, help='LAYERS')
+    parser.add_argument('--encoder-kernel', type=int, default=None, help='ENCODER_KERNEL_SIZE')
+    parser.add_argument('--decoder-kernel', type=int, default=None, help='DECODER_KERNEL_SIZE')
     args = parser.parse_args()
-    if args.dropout is not None and args.architecture != 'convolution':
-        parser.error('--dropout sets DROPOUT, which only the convolution model reads')
+    shape = {key: value for key, value in (
+        ('CHANNELS', args.channels), ('LAYERS', args.layers),
+        ('ENCODER_KERNEL_SIZE', args.encoder_kernel),
+        ('DECODER_KERNEL_SIZE', args.decoder_kernel)) if value is not None}
+    if args.architecture != 'convolution' and (args.dropout is not None or shape):
+        parser.error('--dropout and the shape options configure the convolution model')
     rank = int(os.environ.get('RANK', 0))
     local = int(os.environ.get('LOCAL_RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -84,7 +154,7 @@ def main():
         dist.init_process_group('nccl', device_id=device)
     import emphases_b200 as emphases
     emphases.reset_configuration()
-    emphases.configure(ARCHITECTURE=args.architecture)
+    emphases.configure(ARCHITECTURE=args.architecture, **shape)
     if args.dropout is not None:
         emphases.configure(DROPOUT=args.dropout)
     torch.manual_seed(0)
@@ -134,10 +204,26 @@ def main():
         ms, reduce_ms, frames_total = worst[0].item(), worst[1].item(), total[2].item()
     else:
         frames_total = frames
+    weight_grad = None
+    if rank == 0 and shape:
+        from emphases_b200 import engine
+        width = engine.kernel_width(emphases.CHANNELS)
+        starts, rows = engine.packed_starts([int(batch[0].shape[2])] * int(batch[0].shape[0]))
+        weight_grad = {}
+        for kernel in sorted({emphases.ENCODER_KERNEL_SIZE, emphases.DECODER_KERNEL_SIZE}):
+            us = time_weight_grad(emphases, width, kernel, rows)
+            weight_grad[f'{width}/k{kernel}'] = {
+                'us_per_layer': us, 'rows': rows,
+                'useful_tflops': 2 * kernel * width ** 2 * rows / (us * 1e-6) / 1e12}
+        us, native_rows = native_weight_grad(emphases, batch)
+        weight_grad['80/k3 native'] = {
+            'us_per_layer': us, 'rows': native_rows,
+            'useful_tflops': 2 * 3 * 80 ** 2 * native_rows / (us * 1e-6) / 1e12}
     if rank == 0:
         name, power_limit = card()
         print(json.dumps({
-            'architecture': args.architecture, 'dropout': args.dropout,
+            'architecture': args.architecture, 'dropout': args.dropout, 'shape': shape,
+            'weight_grad': weight_grad,
             'gpu': name, 'power_limit': power_limit,
             'metric': 'training step (config 5)', 'n_gpus': world,
             'ms_per_step': ms, 'allreduce_ms': reduce_ms,
