@@ -16,14 +16,25 @@
 // from L2 into a 3-stage smem ring with cp.async.bulk + mbarrier.  D is a
 // 128-lane x 80-column fp32 accumulator in TMEM.
 //
+// The CTAs run in clusters of two (a CTA pair on one TPC).  Every MMA is a
+// cta_group::2 M=256 instruction issued by rank 0: each CTA supplies the 128
+// rows of its own tile as A and holds half of the weights (40 output columns)
+// as B, and each CTA's TMEM receives its own 128 x 80 accumulator.  Per SM that
+// is the same math as an M=128 MMA with half of the B bytes to fetch from
+// shared memory; one such pair MMA costs 47 clk against 102 clk for each of
+// the two cta_group::1 MMAs it replaces (profiles/r06_umma_2cta_microbench.md).
+// Pair tile p is tiles 2p (rank 0) and 2p + 1 (rank 1).
+//
 // Warp roles (persistent CTA, one per SM, kSlots tiles in flight):
 //   warps 4s .. 4s+3 : epilogue group of tile slot s (TMEM lane quadrant =
 //                      warp % 4): tcgen05.ld -> +bias -> activation ->
 //                      separator-row zeroing -> bf16 -> back into the slot's
 //                      A buffer (next layer's operand), fp32 to HBM after the
 //                      last layer
-//   warp 4*kSlots    : MMA issuer (one elected lane issues tcgen05.mma)
-//   warp 4*kSlots+1  : weight producer (cp.async.bulk)
+//   warp 4*kSlots    : rank 0: MMA issuer for the pair (one elected lane
+//                      issues tcgen05.mma); rank 1: tells rank 0 when its
+//                      half of a ring stage has landed
+//   warp 4*kSlots+1  : weight producer (cp.async.bulk of this CTA's half)
 // While the tensor core works on slot s, the epilogue groups of the other
 // slots drain their accumulators, so MMA and epilogue overlap.
 #include <cuda_bf16.h>
@@ -51,11 +62,15 @@ constexpr int RB = M + 2;             // buffer rows (one pad row each side)
 constexpr int kStages = 3;            // weight ring
 constexpr int kMaxLayers = 16;
 constexpr int ACT_BYTES = KG * RB * 16;           // 20,800 per slot
-constexpr int W_TAP_BYTES = KG * C * 16;          // 12,800
+constexpr int CH = C / 2;             // output columns of the weight half one CTA holds
+constexpr int W_TAP_BYTES = KG * C * 16;          // 12,800 (both halves)
+constexpr int W_HALF_TAP_BYTES = KG * CH * 16;    // 6,400
 constexpr int W_BIAS_BYTES = 2 * C * 16;          // bias chunk: 2 k-groups, 2,560
 // per kernel size (3: the conv stacks; 1: the per-row linear maps of the
-// Transformer variant): bytes of one ring entry
+// Transformer variant): bytes of one blob entry, and of the half of its taps
+// that one CTA of a pair loads into a ring stage
 __host__ __device__ constexpr int conv_bytes(int ks) { return ks * W_TAP_BYTES; }                  // 38,400 at k = 3
+__host__ __device__ constexpr int half_bytes(int ks) { return ks * W_HALF_TAP_BYTES; }             // 19,200 at k = 3
 __host__ __device__ constexpr int layer_bytes(int ks) { return conv_bytes(ks) + W_BIAS_BYTES; }    // 40,960 at k = 3
 constexpr int kTmemCols = 512;
 
@@ -92,11 +107,12 @@ template <int PARTS, int KSIZE>
 struct __align__(128) Smem {
     static constexpr int kSlots = Config<PARTS>::kSlots;
     uint8_t act[kSlots][Config<PARTS>::kParts][ACT_BYTES + 64];   // +64 keeps 128-B alignment
-    uint8_t w[Config<PARTS>::kRing][layer_bytes(KSIZE)];
+    uint8_t w[Config<PARTS>::kRing][half_bytes(KSIZE)];   // this CTA's weight half
     float bias[kMaxLayers][C];                // fp32 bias, added by the epilogue
-    uint64_t w_full[kStages];
-    uint64_t w_empty[kStages];
-    uint64_t act_ready[kSlots];
+    uint64_t w_full[kStages];                 // this CTA's half landed
+    uint64_t peer_full[kStages];              // rank 0 only: rank 1's half landed
+    uint64_t w_empty[kStages];                // the pair's MMAs are done with the stage
+    uint64_t act_ready[kSlots];               // rank 0 only: both tiles' operands stored
     uint64_t mma_done[kSlots];
     uint32_t tmem_base;
 };
@@ -141,12 +157,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) {
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
 }
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile(
-        "{\n\t.reg .b64 state;\n\t"
-        "mbarrier.arrive.shared::cta.b64 state, [%0];\n\t}"
-        ::"r"(smem_u32(bar)) : "memory");
-}
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
     asm volatile(
         "{\n\t.reg .b64 state;\n\t"
@@ -163,6 +173,45 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
             "selp.u32 %0, 1, 0, p;\n\t}"
             : "=r"(done) : "r"(addr), "r"(parity) : "memory");
     } while (!done);
+}
+// wait with acquire at cluster scope: the barrier's arrivals come from the
+// peer CTA too
+__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
+    uint32_t done;
+    const uint32_t addr = smem_u32(bar);
+    do {
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t"
+            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
+            "selp.u32 %0, 1, 0, p;\n\t}"
+            : "=r"(done) : "r"(addr), "r"(parity) : "memory");
+    } while (!done);
+}
+// arrive on the barrier at the same offset in CTA 0 of the cluster.
+// This knowingly departs from the PTX memory model: the arrive uses the
+// default .release.cta semantics, and a cta-scope release in rank 1 is not
+// morally strong with rank 0's cluster-scope acquire.  The hand-off of rank
+// 1's operand stores to the MMA that rank 0 issues therefore rests on the
+// hardware's causality order, the same as the remote arrives of CUTLASS's
+// cluster pipelines (ClusterBarrier::arrive(cta_id)).  The .release.cluster
+// form is the one the model covers; it made every epilogue hand-off slower
+// (frame stack 1.37 against 1.27 ms on one B200, 1000 W).
+__device__ __forceinline__ void mbar_arrive_rank0(uint64_t* bar) {
+    asm volatile(
+        "{\n\t.reg .b32 remote;\n\t"
+        "mapa.shared::cluster.u32 remote, %0, 0;\n\t"
+        "mbarrier.arrive.shared::cluster.b64 _, [remote];\n\t}"
+        ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ uint32_t cluster_rank() {
+    uint32_t rank;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+    return rank;
+}
+// every thread of both CTAs
+__device__ __forceinline__ void cluster_sync() {
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\t"
+                 "barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 __device__ __forceinline__ void fence_barrier_init() {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -181,25 +230,28 @@ __device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t b
         "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
         ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
+// TMEM of a CTA pair: one warp of each CTA allocates (the same columns in both)
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
                  ::"r"(smem_u32(dst)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
 }
 __device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
 }
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-                 ::"r"(smem_u32(bar)) : "memory");
+// arrive on the barrier at this offset in both CTAs once the pair's MMAs issued
+// so far are complete
+__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                 ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
 }
-// D[tmem] (+)= A[smem] * B[smem], bf16 x bf16 -> fp32
+// D[tmem] (+)= A[smem] * B[smem], bf16 x bf16 -> fp32, M = 256 over the pair
 __device__ __forceinline__ void umma_bf16(
     uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
     asm volatile(
         "{\n\t.reg .pred p;\n\t"
         "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
         ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
 }
 // No-swizzle K-major smem matrix descriptor (cute::UMMA::SmemDescriptor):
@@ -274,9 +326,9 @@ __device__ __forceinline__ bool elect_one() {
 
 // instruction descriptor (cute::UMMA::InstrDescriptor): D fp32 [4,6) = 1,
 // A bf16 [7,10) = 1, B bf16 [10,13) = 1, A and B K-major, N >> 3 at [17,23),
-// M >> 4 at [24,29)
+// M >> 4 at [24,29); M = 256 rows over the CTA pair
 constexpr uint32_t kInstrDesc =
-    (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(C >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+    (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(C >> 3) << 17) | ((uint32_t)(2 * M >> 4) << 24);
 
 // two values -> PARTS bf16x2 words: hi, then the bf16 of what is left, ...
 template <int PARTS>
@@ -335,10 +387,10 @@ __device__ __noinline__ void epilogue_generic(
 }
 
 template <int PARTS, int KSIZE>
-__global__ void __launch_bounds__(Config<PARTS>::kThreads, 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Config<PARTS>::kThreads, 1)
 conv_stack_tc_kernel(
     const float* __restrict__ x, const int32_t* __restrict__ row_seq, int total_rows,
-    const uint8_t* __restrict__ weights,   // ring entries: [tap][kg][n][8] bf16 + bias chunk
+    const uint8_t* __restrict__ weights,   // blob entries: [half][tap][kg][40 n][8] bf16 + bias chunk
     Acts acts, int n_layers, int tile_rows, int n_tiles, float* __restrict__ y,
     PoolArgs pool) {
     constexpr int kSlots = Config<PARTS>::kSlots;
@@ -349,12 +401,20 @@ conv_stack_tc_kernel(
     extern __shared__ __align__(128) uint8_t smem_raw[];
     Smem<PARTS, KSIZE>& sm = *reinterpret_cast<Smem<PARTS, KSIZE>*>(smem_raw);
     constexpr int W_CONV_BYTES = conv_bytes(KSIZE);
+    constexpr int W_HALF_BYTES = half_bytes(KSIZE);
     constexpr int W_LAYER_BYTES = layer_bytes(KSIZE);
     constexpr int HALF = (KSIZE - 1) / 2;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int halo = n_layers * HALF;
-    const int rounds = (n_tiles + gridDim.x * kSlots - 1) / (gridDim.x * kSlots);
+    const int rank = (int)cluster_rank();
+    const int cluster = blockIdx.x >> 1, n_clusters = gridDim.x >> 1;
+    // pair tile p = tiles 2p and 2p + 1; a pair whose second tile is past the
+    // end still runs both CTAs: rank 1 may load a few real rows into its halo,
+    // but every row it would store lies at or past total_rows, so it stores
+    // nothing
+    const int n_pairs = (n_tiles + 1) >> 1;
+    const int rounds = (n_pairs + n_clusters * kSlots - 1) / (n_clusters * kSlots);
 
     // ---- one-time setup ----
     // pad rows (buffer rows 0 and RB-1) of every k-group stay zero forever
@@ -377,9 +437,10 @@ conv_stack_tc_kernel(
         for (int i = 0; i < kRing; ++i) {
             mbar_init(&sm.w_full[i], 1);
             mbar_init(&sm.w_empty[i], 1);
+            mbar_init(&sm.peer_full[i], 1);
         }
         for (int s = 0; s < kSlots; ++s) {
-            mbar_init(&sm.act_ready[s], 4);     // one elected lane per epilogue warp
+            mbar_init(&sm.act_ready[s], 8);     // one elected lane per epilogue warp of the pair
             mbar_init(&sm.mma_done[s], 1);
         }
         fence_barrier_init();
@@ -387,7 +448,7 @@ conv_stack_tc_kernel(
     if (warp == kSlots * 4) tmem_alloc(&sm.tmem_base, kTmemCols);
     fence_proxy_async();
     tc_fence_before();
-    __syncthreads();
+    cluster_sync();     // no arrive from the peer may meet an uninitialized barrier
     tc_fence_after();
     const uint32_t tmem_base = sm.tmem_base;
 
@@ -440,14 +501,15 @@ conv_stack_tc_kernel(
             }
         };
         {
-            const int first = blockIdx.x * kSlots + slot;
-            if (first < n_tiles) fetch_tile(first);
+            const int first = cluster * kSlots + slot;
+            if (first < n_pairs) fetch_tile(2 * first + rank);
         }
 
         for (int round = 0; round < rounds; ++round) {
-            const int tile = (round * gridDim.x + blockIdx.x) * kSlots + slot;
-            if (tile >= n_tiles) break;
-            const int next_tile = tile + gridDim.x * kSlots;
+            const int pair = (round * n_clusters + cluster) * kSlots + slot;
+            if (pair >= n_pairs) break;
+            const int tile = 2 * pair + rank;
+            const int next_tile = tile + 2 * n_clusters * kSlots;
             const int row0 = tile * tile_rows - halo;   // global row of local row 0
             const int g = row0 + row;
             const bool in_range = g >= 0 && g < total_rows;
@@ -475,7 +537,7 @@ conv_stack_tc_kernel(
             fence_proxy_async();        // generic-proxy writes -> visible to the tensor core
             tc_fence_before();          // orders the previous round's TMEM reads too
             __syncwarp();
-            if (lane == 0) mbar_arrive(&sm.act_ready[slot]);
+            if (lane == 0) mbar_arrive_rank0(&sm.act_ready[slot]);
 
             // pull the next round's tile of this slot into L2 while this one computes
             if (next_tile < n_tiles) {
@@ -561,7 +623,7 @@ conv_stack_tc_kernel(
                 fence_proxy_async();
                 tc_fence_before();
                 __syncwarp();
-                if (lane == 0) mbar_arrive(&sm.act_ready[slot]);
+                if (lane == 0) mbar_arrive_rank0(&sm.act_ready[slot]);
                 if (tid == 0) TRACE(3, round * n_layers + layer);
             }
 
@@ -698,11 +760,26 @@ conv_stack_tc_kernel(
                 }
             }
         }
+    } else if (warp == kSlots * 4 && rank == 1) {
+        // ===================== rank 1: ring stage relay ======================
+        // rank 0 issues the pair's MMAs only once this CTA's weight half is in
+        if (lane == 0) {
+            int stage = 0;
+            uint32_t full_parity = 0;
+            for (int round = 0; round < rounds; ++round) {
+                if ((round * n_clusters + cluster) * kSlots >= n_pairs) break;
+                for (int entry = 0; entry < n_layers * kEntries; ++entry) {
+                    mbar_wait(&sm.w_full[stage], full_parity);
+                    mbar_arrive_rank0(&sm.peer_full[stage]);
+                    if (++stage == kRing) { stage = 0; full_parity ^= 1; }
+                }
+            }
+        }
     } else if (warp == kSlots * 4) {
-        // ============================ MMA issuer ============================
+        // ====================== rank 0: MMA issuer ======================
         // The whole warp runs this loop (warp-uniform control flow keeps the
         // descriptors in uniform registers); one elected lane issues.  A
-        // measured tcgen05.mma of this shape costs ~100 clk, so every
+        // measured pair tcgen05.mma of this shape costs ~47 clk, so every
         // instruction saved in the issue path counts.
         uint32_t ready_parity = 0;                   // bit s = parity of slot s
         int stage = 0;
@@ -712,21 +789,22 @@ conv_stack_tc_kernel(
         for (int s = 0; s < kSlots; ++s) d_act[s] = make_desc(smem_u32(sm.act[s][0]), RB * 16, 128);
         constexpr uint64_t kLoPart = (ACT_BYTES + 64) >> 4;      // hi -> lo operand buffer
         for (int round = 0; round < rounds; ++round) {
-            const int tile0 = (round * gridDim.x + blockIdx.x) * kSlots;
-            if (tile0 >= n_tiles) break;
-            const int active = min(kSlots, n_tiles - tile0);
+            const int pair0 = (round * n_clusters + cluster) * kSlots;
+            if (pair0 >= n_pairs) break;
+            const int active = min(kSlots, n_pairs - pair0);
             for (int layer = 0; layer < n_layers; ++layer) {
 #pragma unroll
                 for (int entry = 0; entry < kEntries; ++entry) {
-                    // entry e: weight part e (entry 0 also carries the bias chunk)
+                    // entry e: weight part e, both halves
                     mbar_wait(&sm.w_full[stage], full_parity);
-                    const uint64_t d_w = make_desc(smem_u32(sm.w[stage]), C * 16, 128);
+                    mbar_wait_cluster(&sm.peer_full[stage], full_parity);
+                    const uint64_t d_w = make_desc(smem_u32(sm.w[stage]), CH * 16, 128);
 #pragma unroll
                     for (int s = 0; s < kSlots; ++s) {
                         if (s < active) {
                             if (entry == 0) {
                                 if (s == 0 && lane == 0) TRACE(4, round * n_layers + layer);
-                                mbar_wait(&sm.act_ready[s], (ready_parity >> s) & 1);
+                                mbar_wait_cluster(&sm.act_ready[s], (ready_parity >> s) & 1);
                                 if (s == 0 && lane == 0) TRACE(5, round * n_layers + layer);
                                 ready_parity ^= 1u << s;
                                 tc_fence_after();
@@ -747,7 +825,7 @@ conv_stack_tc_kernel(
                                                     d_act[s] + part * kLoPart +
                                                         // tap t reads buffer row r + t + 1 - HALF
                                                         (uint64_t)(((2 * kk) * RB * 16 + (tap + 1 - HALF) * 16) >> 4),
-                                                    d_w + (uint64_t)((tap * W_TAP_BYTES + (2 * kk) * C * 16) >> 4),
+                                                    d_w + (uint64_t)((tap * W_HALF_TAP_BYTES + (2 * kk) * CH * 16) >> 4),
                                                     kInstrDesc,
                                                     // a class is opened by its entry-0 MMA
                                                     (entry | tap | kk) != 0);
@@ -755,14 +833,14 @@ conv_stack_tc_kernel(
                                         }
                                     }
                                 }
-                                if (entry == kEntries - 1) umma_commit(&sm.mma_done[s]);
+                                if (entry == kEntries - 1) umma_commit_pair(&sm.mma_done[s]);
                             }
                             __syncwarp();
                             if (s == 0 && lane == 0) TRACE(6, round * n_layers + layer);
                             if (s == kSlots - 1 && lane == 0) TRACE(7, round * n_layers + layer);
                         }
                     }
-                    if (elect_one()) umma_commit(&sm.w_empty[stage]);   // ring entry consumed
+                    if (elect_one()) umma_commit_pair(&sm.w_empty[stage]);   // ring stage consumed
                     __syncwarp();
                     if (++stage == kRing) { stage = 0; full_parity ^= 1; }
                 }
@@ -774,32 +852,40 @@ conv_stack_tc_kernel(
             int stage = 0;
             uint32_t empty_parity = 1;       // first pass over the ring never waits
             for (int round = 0; round < rounds; ++round) {
-                const int tile0 = (round * gridDim.x + blockIdx.x) * kSlots;
-                if (tile0 >= n_tiles) break;
+                if ((round * n_clusters + cluster) * kSlots >= n_pairs) break;
                 for (int entry = 0; entry < n_layers * kEntries; ++entry) {
                     mbar_wait(&sm.w_empty[stage], empty_parity);
-                    mbar_arrive_expect_tx(&sm.w_full[stage], W_LAYER_BYTES);
-                    bulk_load(sm.w[stage], weights + (size_t)entry * W_LAYER_BYTES,
-                              W_LAYER_BYTES, &sm.w_full[stage]);
+                    mbar_arrive_expect_tx(&sm.w_full[stage], W_HALF_BYTES);
+                    bulk_load(sm.w[stage], weights + (size_t)entry * W_LAYER_BYTES + rank * W_HALF_BYTES,
+                              W_HALF_BYTES, &sm.w_full[stage]);
                     if (++stage == kRing) { stage = 0; empty_parity ^= 1; }
                 }
+            }
+            // producer tail: wait until the pair's MMAs release every stage, so
+            // that the last w_empty commits (multicast to both CTAs) have landed
+            // before this CTA passes the teardown barrier.  A stage never loaded
+            // passes at once (parity 1 of a fresh barrier).
+            for (int i = 0; i < kRing; ++i) {
+                mbar_wait(&sm.w_empty[stage], empty_parity);
+                if (++stage == kRing) { stage = 0; empty_parity ^= 1; }
             }
         }
     }
 
     // ---- teardown ----
     tc_fence_before();
-    __syncthreads();
+    cluster_sync();     // neither CTA leaves while the pair's MMAs or arrivals can reach it
     if (warp == kSlots * 4) {
         tc_fence_after();
         tmem_dealloc(tmem_base, kTmemCols);
     }
 }
 
-// fp32 weights [L][tap][in][out] + bias [L][out] -> ring entries of
-// W_LAYER_BYTES: bf16 [tap][kg][out][8 in] followed by the bias chunk bf16
-// [2][out][8] (k-group 0 holds the fp32 bias as three bf16 parts (hi, mid, lo,
-// 0, ...), k-group 1 is zero).
+// fp32 weights [L][tap][in][out] + bias [L][out] -> blob entries of
+// W_LAYER_BYTES: bf16 [half][tap][kg][40 out][8 in] (half h = output columns
+// 40h .. 40h+39, the ring stage of CTA h of a pair) followed by the bias chunk
+// bf16 [2][out][8] (k-group 0 holds the fp32 bias as three bf16 parts (hi,
+// mid, lo, 0, ...), k-group 1 is zero; the kernel reads it once at setup).
 // parts = 2 / 3: that many entries per layer -- (W_hi, bias chunk), (W_mid, zeros)
 // (, (W_lo, zeros)) with W_hi = bf16(W), W_mid = bf16(W - W_hi), W_lo = bf16 of
 // what is still left.
@@ -821,9 +907,10 @@ __device__ __forceinline__ void pack_weights_tc_body(
         if (local < conv) {
             const int e = local & 7;
             int rest = local >> 3;
-            const int n = rest % C; rest /= C;
-            const int kg = rest % KG;
-            const int tap = rest / KG;
+            const int nh = rest % CH; rest /= CH;
+            const int kg = rest % KG; rest /= KG;
+            const int tap = rest % ks;
+            const int n = (rest / ks) * CH + nh;
             const int ci = kg * 8 + e;
             const float value =
                 source == 0 ? w[((size_t)(layer * ks + tap) * C + ci) * C + n]
@@ -884,9 +971,31 @@ static int launch_tc(
                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
         "conv_tc smem attribute");
     if (s != EMPH_OK) return s;
+    // CTA pairs the device can keep resident (a pair needs two SMs of one TPC
+    // with room for this CTA): the persistent grid never exceeds it.  Cached
+    // per device; callers on several threads at once store the same value.
+    constexpr int kMaxDevices = 64;
+    static int max_clusters_of[kMaxDevices] = {};
+    int device = 0;
+    s = check_cuda(cudaGetDevice(&device), "conv_tc device");
+    if (s != EMPH_OK) return s;
+    EMPH_REQUIRE(device < kMaxDevices, "emph_conv_stack(tc): device %d out of range", device);
+    int max_clusters = max_clusters_of[device];
+    if (max_clusters == 0) {
+        cudaLaunchConfig_t config = {};
+        config.gridDim = dim3(2 * sm_count());
+        config.blockDim = dim3(tc::Config<PARTS>::kThreads);
+        config.dynamicSmemBytes = smem;
+        s = check_cuda(cudaOccupancyMaxActiveClusters(
+                           &max_clusters, (void*)tc::conv_stack_tc_kernel<PARTS, KSIZE>, &config),
+                       "conv_tc cluster occupancy");
+        if (s != EMPH_OK) return s;
+        EMPH_REQUIRE(max_clusters > 0, "emph_conv_stack(tc): no CTA pair fits on the device");
+        max_clusters_of[device] = max_clusters;
+    }
     const int n_tiles = (total_rows + tile_rows - 1) / tile_rows;
-    const int want = (n_tiles + kSlots - 1) / kSlots;
-    const int grid = want < sm_count() ? want : sm_count();
+    const int want = ((n_tiles + 1) / 2 + kSlots - 1) / kSlots;
+    const int grid = 2 * (want < max_clusters ? want : max_clusters);
     tc::conv_stack_tc_kernel<PARTS, KSIZE><<<grid, tc::Config<PARTS>::kThreads, smem, stream>>>(
         x, row_seq, total_rows, reinterpret_cast<const uint8_t*>(weights), acts,
         n_layers, tile_rows, n_tiles, y, pool);

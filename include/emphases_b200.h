@@ -190,8 +190,9 @@ int emph_conv_stack(
  * Weights for precision == EMPH_PREC_BF16_TC / _BF16X3_TC / _BF16X6_TC (the
  * split modes pack 2 / 3 bf16 blobs per layer: hi, (mid,) lo): fp32 weights
  * [n_layers][k][in][out] (the layout above) and bias [n_layers][out] -> per
- * layer a bf16 blob in the UMMA shared-memory operand layout [k][in / 8][out][8]
- * followed by a bias chunk (the bias as three bf16 parts, rebuilt exactly to
+ * layer a bf16 blob in the UMMA shared-memory operand layout, split in two
+ * halves of the output channels, [2][k][in / 8][out / 2][8] (one half per CTA
+ * of the kernel's CTA pairs), followed by a bias chunk (the bias as three bf16 parts, rebuilt exactly to
  * fp32 and added by the kernel's epilogue).  emph_conv_weights_tc_bytes gives the blob size (0 if
  * the configuration is not compiled in).  Pass the blob as `weights` of
  * emph_conv_stack; `bias` is then unused.
