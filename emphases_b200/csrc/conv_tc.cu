@@ -4,17 +4,21 @@
 //
 // Replaces input_layer + frame_encoder (emphases/model/core.py:92-94,
 // emphases/model/layers/convolution.py:13-37), i.e. the 7 frame-resolution
-// Conv1d(80 -> 80, k=3, 'same') layers that hold 99 % of the model FLOPs.
+// Conv1d(80 -> 80, k, 'same') layers that hold 99 % of the model FLOPs, and
+// the word decoder; kernel sizes 1, 3 (the default), 5 and 7 (the reference's
+// hyper-parameter sweep) at 80 channels.
 //
 // GEMM view of one layer on a tile of 128 packed rows:
 //     D[128 rows][80 out] = sum_{tap} A_tap[128 rows][80 in] * W_tap[80 in][80 out]
 // A lives in smem as bf16 in the no-swizzle K-major "interleaved" UMMA layout
 // [k-group of 8 channels][row][8 channels] with all rows of a k-group
-// contiguous (SBO = 128 B), so the +-1 row shift of the three taps is just a
-// 16-byte offset of the descriptor start address: the same buffer feeds all
-// three taps.  B (weights) uses the same layout per tap, streamed per layer
-// from L2 into a 3-stage smem ring with cp.async.bulk + mbarrier.  D is a
-// 128-lane x 80-column fp32 accumulator in TMEM.
+// contiguous (SBO = 128 B), so the row shift of tap t is just a 16-byte
+// multiple added to the descriptor start address: the same buffer feeds all
+// k taps.  Each k-group carries (k - 1) / 2 zero pad rows at each end (one at
+// k = 1), so the shifted reads stay inside it.  B (weights) uses the same
+// layout per tap, streamed per layer from L2 into a 2- or 3-stage smem ring
+// with cp.async.bulk + mbarrier.  D is a 128-lane x 80-column fp32
+// accumulator in TMEM.
 //
 // The CTAs run in clusters of two (a CTA pair on one TPC).  Every MMA is a
 // cta_group::2 M=256 instruction issued by rank 0: each CTA supplies the 128
@@ -58,16 +62,24 @@ __device__ long long g_trace[8][512];
 constexpr int C = 80;                 // channels (in = out)
 constexpr int KG = C / 8;             // k-groups of 8 channels
 constexpr int M = 128;                // rows per tile = UMMA M
-constexpr int RB = M + 2;             // buffer rows (one pad row each side)
 constexpr int kStages = 3;            // weight ring
 constexpr int kMaxLayers = 16;
-constexpr int ACT_BYTES = KG * RB * 16;           // 20,800 per slot
+constexpr int kSmemLimit = 232448;    // dynamic shared memory one block may opt in to
+// Operand buffer of one slot and part, per kernel size: the tile's M rows
+// with pad_rows(k) zero rows at each end of every k-group, so that tap t of
+// row r reads buffer row r + t + pad_rows(k) - (k - 1) / 2 and never leaves
+// the k-group.  k = 1 keeps one pad row each side, as k = 3 does.
+__host__ __device__ constexpr int pad_rows(int ks) { return ks > 3 ? (ks - 1) / 2 : 1; }
+__host__ __device__ constexpr int buffer_rows(int ks) { return M + 2 * pad_rows(ks); }  // 130 / 132 / 134
+__host__ __device__ constexpr int act_bytes(int ks) { return KG * buffer_rows(ks) * 16; }  // 20,800 at k = 3
+// parts of a slot lie this far apart: act_bytes rounded up to 128-B alignment
+__host__ __device__ constexpr int act_stride(int ks) { return (act_bytes(ks) + 127) / 128 * 128; }
 constexpr int CH = C / 2;             // output columns of the weight half one CTA holds
 constexpr int W_TAP_BYTES = KG * C * 16;          // 12,800 (both halves)
 constexpr int W_HALF_TAP_BYTES = KG * CH * 16;    // 6,400
 constexpr int W_BIAS_BYTES = 2 * C * 16;          // bias chunk: 2 k-groups, 2,560
-// per kernel size (3: the conv stacks; 1: the per-row linear maps of the
-// Transformer variant): bytes of one blob entry, and of the half of its taps
+// per kernel size (3, 5, 7: the conv stacks; 1: the per-row linear maps of
+// the Transformer variant): bytes of one blob entry, and of the half of its taps
 // that one CTA of a pair loads into a ring stage
 __host__ __device__ constexpr int conv_bytes(int ks) { return ks * W_TAP_BYTES; }                  // 38,400 at k = 3
 __host__ __device__ constexpr int half_bytes(int ks) { return ks * W_HALF_TAP_BYTES; }             // 19,200 at k = 3
@@ -106,7 +118,7 @@ struct Config {
 template <int PARTS, int KSIZE>
 struct __align__(128) Smem {
     static constexpr int kSlots = Config<PARTS>::kSlots;
-    uint8_t act[kSlots][Config<PARTS>::kParts][ACT_BYTES + 64];   // +64 keeps 128-B alignment
+    uint8_t act[kSlots][Config<PARTS>::kParts][act_stride(KSIZE)];
     uint8_t w[Config<PARTS>::kRing][half_bytes(KSIZE)];   // this CTA's weight half
     float bias[kMaxLayers][C];                // fp32 bias, added by the epilogue
     uint64_t w_full[kStages];                 // this CTA's half landed
@@ -346,20 +358,21 @@ __device__ __forceinline__ void split_pack(float lo_v, float hi_v, uint32_t (&wo
 }
 
 // Store 8 consecutive channels of one row into the slot's A-operand buffer(s)
-template <int PARTS>
+template <int PARTS, int KSIZE>
 __device__ __forceinline__ void store_kgroup(uint8_t* act_hi, int kg, int buffer_row, const float (&v)[8]) {
     uint32_t words[4][PARTS];
 #pragma unroll
     for (int j = 0; j < 4; ++j) split_pack<PARTS>(v[2 * j], v[2 * j + 1], words[j]);
 #pragma unroll
     for (int p = 0; p < PARTS; ++p)
-        *reinterpret_cast<uint4*>(act_hi + p * (ACT_BYTES + 64) + (kg * RB + buffer_row) * 16) =
+        *reinterpret_cast<uint4*>(act_hi + p * act_stride(KSIZE) +
+                                  (kg * buffer_rows(KSIZE) + buffer_row) * 16) =
             make_uint4(words[0][p], words[1][p], words[2][p], words[3][p]);
 }
 
 // Rare path: activations other than ReLU / identity.  Out of line so the hot
 // loop stays small in the instruction cache.
-template <int PARTS>
+template <int PARTS, int KSIZE>
 __device__ __noinline__ void epilogue_generic(
     uint32_t taddr, uint8_t* act, int row, int a, bool valid, bool last, bool store,
     float* yrow, const float* bias) {
@@ -374,8 +387,8 @@ __device__ __noinline__ void epilogue_generic(
         if (!last) {
             const float (&first)[8] = *reinterpret_cast<const float(*)[8]>(&v[0]);
             const float (&second)[8] = *reinterpret_cast<const float(*)[8]>(&v[8]);
-            store_kgroup<PARTS>(act, c0 >> 3, row + 1, first);
-            store_kgroup<PARTS>(act, (c0 >> 3) + 1, row + 1, second);
+            store_kgroup<PARTS, KSIZE>(act, c0 >> 3, row + pad_rows(KSIZE), first);
+            store_kgroup<PARTS, KSIZE>(act, (c0 >> 3) + 1, row + pad_rows(KSIZE), second);
         } else if (store) {
             float4* dst = reinterpret_cast<float4*>(yrow + c0);
             dst[0] = make_float4(v[0], v[1], v[2], v[3]);
@@ -404,6 +417,9 @@ conv_stack_tc_kernel(
     constexpr int W_HALF_BYTES = half_bytes(KSIZE);
     constexpr int W_LAYER_BYTES = layer_bytes(KSIZE);
     constexpr int HALF = (KSIZE - 1) / 2;
+    constexpr int PAD = pad_rows(KSIZE);       // tile row r lives in buffer row r + PAD
+    constexpr int RB = buffer_rows(KSIZE);
+    constexpr int ACT_STRIDE = act_stride(KSIZE);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int halo = n_layers * HALF;
@@ -417,12 +433,13 @@ conv_stack_tc_kernel(
     const int rounds = (n_pairs + n_clusters * kSlots - 1) / (n_clusters * kSlots);
 
     // ---- one-time setup ----
-    // pad rows (buffer rows 0 and RB-1) of every k-group stay zero forever
-    for (int i = tid; i < kSlots * kParts * KG * 2 * 4; i += kThreads) {
-        const int buffer = i / (KG * 8), rem = i % (KG * 8);
-        const int kg = rem / 8, edge = (rem / 4) & 1, word = rem & 3;
+    // pad rows (buffer rows 0 .. PAD-1 and RB-PAD .. RB-1) of every k-group
+    // stay zero forever
+    for (int i = tid; i < kSlots * kParts * KG * PAD * 2 * 4; i += kThreads) {
+        const int buffer = i / (KG * PAD * 8), rem = i % (KG * PAD * 8);
+        const int kg = rem / (PAD * 8), pad = (rem / 8) % PAD, edge = (rem / 4) & 1, word = rem & 3;
         reinterpret_cast<uint32_t*>(
-            sm.act[buffer / kParts][buffer % kParts] + (kg * RB + (edge ? RB - 1 : 0)) * 16)[word] = 0u;
+            sm.act[buffer / kParts][buffer % kParts] + (kg * RB + (edge ? RB - 1 - pad : pad)) * 16)[word] = 0u;
     }
     // fp32 bias of every layer, rebuilt exactly from the three bf16 parts the
     // packed blob carries after each layer's taps; the epilogue adds it
@@ -520,18 +537,18 @@ conv_stack_tc_kernel(
             for (int it = 0; it < 20; ++it) {
                 const int i = gtid + 128 * it;
                 const int r = i / (C / 4), c4 = i % (C / 4);
-                uint8_t* dst = act + ((c4 >> 1) * RB + r + 1) * 16 + (c4 & 1) * 8;
+                uint8_t* dst = act + ((c4 >> 1) * RB + r + PAD) * 16 + (c4 & 1) * 8;
                 if constexpr (kKeepRaw) {
                     uint32_t a[PARTS], b[PARTS];
                     split_pack<PARTS>(raw_rows[it].x, raw_rows[it].y, a);
                     split_pack<PARTS>(raw_rows[it].z, raw_rows[it].w, b);
 #pragma unroll
                     for (int p = 0; p < PARTS; ++p)
-                        *reinterpret_cast<uint2*>(dst + p * (ACT_BYTES + 64)) = make_uint2(a[p], b[p]);
+                        *reinterpret_cast<uint2*>(dst + p * ACT_STRIDE) = make_uint2(a[p], b[p]);
                 } else {
 #pragma unroll
                     for (int p = 0; p < PARTS; ++p)
-                        *reinterpret_cast<uint2*>(dst + p * (ACT_BYTES + 64)) = pk[p][it];
+                        *reinterpret_cast<uint2*>(dst + p * ACT_STRIDE) = pk[p][it];
                 }
             }
             fence_proxy_async();        // generic-proxy writes -> visible to the tensor core
@@ -588,7 +605,7 @@ conv_stack_tc_kernel(
                         }
                     }
                     if constexpr (PARTS == 1) {
-                        uint8_t* dst = act + (row + 1) * 16;
+                        uint8_t* dst = act + (row + PAD) * 16;
 #pragma unroll
                         for (int kg = 0; kg < KG; ++kg) {
                             uint32_t p[4];
@@ -612,11 +629,11 @@ conv_stack_tc_kernel(
                                 if (relu) w[j] = fmaxf(w[j], 0.f);
                                 if (zero) w[j] = 0.f;
                             }
-                            store_kgroup<PARTS>(act, kg, row + 1, w);
+                            store_kgroup<PARTS, KSIZE>(act, kg, row + PAD, w);
                         }
                     }
                 } else {
-                    epilogue_generic<PARTS>(
+                    epilogue_generic<PARTS, KSIZE>(
                         taddr, act, row, a, valid, false, false, y, sm.bias[layer]);
                 }
                 if (tid == 0) TRACE(2, round * n_layers + layer);
@@ -661,11 +678,12 @@ conv_stack_tc_kernel(
                         starts = __ballot_sync(0xffffffffu, lane < 2 || before != wid);
                         ends = __ballot_sync(0xffffffffu, lane >= 30 || after != wid);
                     }
-                    // scratch of this warp: the interior (rows 1 .. 128) of k-group
-                    // `quad` of the slot's operand buffer = 2048 contiguous bytes =
-                    // [32 rows][16 floats]; the last layer's MMAs are done with it, and
-                    // the slot's warps meet at a barrier before the next tile is stored
-                    float* scratch = reinterpret_cast<float*>(act + (quad * RB + 1) * 16);
+                    // scratch of this warp: the interior (rows PAD .. PAD + 127) of
+                    // k-group `quad` of the slot's operand buffer = 2048 contiguous
+                    // bytes = [32 rows][16 floats]; the last layer's MMAs are done with
+                    // it, and the slot's warps meet at a barrier before the next tile is
+                    // stored
+                    float* scratch = reinterpret_cast<float*>(act + (quad * RB + PAD) * 16);
                     const size_t word_base = (size_t)(wid >= 0 ? wid : 0) * C;
 #pragma unroll 1
                     for (int c0 = 0; c0 < C; c0 += 16) {
@@ -752,7 +770,7 @@ conv_stack_tc_kernel(
                     if (pool.mode == kPoolSum || pool.mode == kPoolMax)
                         asm volatile("bar.sync %0, 128;" ::"r"(slot + 1) : "memory");
                 } else {
-                    epilogue_generic<PARTS>(
+                    epilogue_generic<PARTS, KSIZE>(
                         taddr, act, row, a, valid, true,
                         in_range && row >= halo && row < M - halo,
                         y + (size_t)(in_range ? g : 0) * C, sm.bias[layer]);
@@ -787,7 +805,7 @@ conv_stack_tc_kernel(
         uint64_t d_act[kSlots];
 #pragma unroll
         for (int s = 0; s < kSlots; ++s) d_act[s] = make_desc(smem_u32(sm.act[s][0]), RB * 16, 128);
-        constexpr uint64_t kLoPart = (ACT_BYTES + 64) >> 4;      // hi -> lo operand buffer
+        constexpr uint64_t kLoPart = ACT_STRIDE >> 4;            // hi -> lo operand buffer
         for (int round = 0; round < rounds; ++round) {
             const int pair0 = (round * n_clusters + cluster) * kSlots;
             if (pair0 >= n_pairs) break;
@@ -823,8 +841,9 @@ conv_stack_tc_kernel(
                                                 umma_bf16(
                                                     d0 + (entry + part) * Config<PARTS>::kClassStride,
                                                     d_act[s] + part * kLoPart +
-                                                        // tap t reads buffer row r + t + 1 - HALF
-                                                        (uint64_t)(((2 * kk) * RB * 16 + (tap + 1 - HALF) * 16) >> 4),
+                                                        // tap t reads buffer row r + t + PAD - HALF
+                                                        // (r + t for k >= 3)
+                                                        (uint64_t)(((2 * kk) * RB * 16 + (tap + PAD - HALF) * 16) >> 4),
                                                     d_w + (uint64_t)((tap * W_HALF_TAP_BYTES + (2 * kk) * CH * 16) >> 4),
                                                     kInstrDesc,
                                                     // a class is opened by its entry-0 MMA
@@ -958,6 +977,8 @@ static int launch_tc(
     const float* x, const int32_t* row_seq, int32_t total_rows, const float* weights,
     const int32_t* acts_host, int32_t n_layers, float* y, cudaStream_t stream,
     tc::PoolArgs pool = tc::PoolArgs{nullptr, nullptr, nullptr, tc::kPoolNone}) {
+    static_assert(sizeof(tc::Smem<PARTS, KSIZE>) + 128 <= tc::kSmemLimit,
+                  "conv_tc: the slots and the weight ring do not fit shared memory");
     EMPH_REQUIRE(n_layers <= tc::kMaxLayers, "emph_conv_stack(tc): too many layers");
     const int halo = n_layers * ((KSIZE - 1) / 2);
     const int tile_rows = tc::M - 2 * halo;
@@ -1004,19 +1025,37 @@ static int launch_tc(
     return EMPH_OK;
 }
 
+// kernel sizes the tensor-core stack is compiled for (at 80 channels)
+static bool tc_kernel_size(int kernel_size) {
+    return kernel_size == 1 || kernel_size == 3 || kernel_size == 5 || kernel_size == 7;
+}
+
+template <int PARTS>
+static int launch_tc_ks(
+    const float* x, const int32_t* row_seq, int32_t total_rows, const float* weights,
+    const int32_t* acts_host, int32_t n_layers, int32_t kernel_size, float* y, cudaStream_t stream,
+    tc::PoolArgs pool = tc::PoolArgs{nullptr, nullptr, nullptr, tc::kPoolNone}) {
+    switch (kernel_size) {
+        case 1: return launch_tc<PARTS, 1>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream, pool);
+        case 3: return launch_tc<PARTS, 3>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream, pool);
+        case 5: return launch_tc<PARTS, 5>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream, pool);
+        case 7: return launch_tc<PARTS, 7>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream, pool);
+    }
+    set_error("emph_conv_stack(tc): kernel_size=%d not compiled in", kernel_size);
+    return EMPH_ENOSYS;
+}
+
 int conv_stack_bf16_tc(
     const float* x, const int32_t* row_seq, int32_t total_rows,
     const float* weights, const float* bias, const int32_t* acts_host,
     int32_t n_layers, int32_t channels, int32_t kernel_size, float* y,
     cudaStream_t stream) {
-    if (channels != tc::C || (kernel_size != 3 && kernel_size != 1)) {
+    if (channels != tc::C || !tc_kernel_size(kernel_size)) {
         set_error("emph_conv_stack(bf16 tc): channels=%d kernel_size=%d not compiled in",
                   channels, kernel_size);
         return EMPH_ENOSYS;
     }
-    if (kernel_size == 1)
-        return launch_tc<1, 1>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream);
-    return launch_tc<1, 3>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream);
+    return launch_tc_ks<1>(x, row_seq, total_rows, weights, acts_host, n_layers, kernel_size, y, stream);
 }
 
 int conv_stack_bf16x3_tc(
@@ -1024,14 +1063,12 @@ int conv_stack_bf16x3_tc(
     const float* weights, const int32_t* acts_host,
     int32_t n_layers, int32_t channels, int32_t kernel_size, float* y,
     cudaStream_t stream) {
-    if (channels != tc::C || (kernel_size != 3 && kernel_size != 1)) {
+    if (channels != tc::C || !tc_kernel_size(kernel_size)) {
         set_error("emph_conv_stack(bf16x3 tc): channels=%d kernel_size=%d not compiled in",
                   channels, kernel_size);
         return EMPH_ENOSYS;
     }
-    if (kernel_size == 1)
-        return launch_tc<2, 1>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream);
-    return launch_tc<2, 3>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream);
+    return launch_tc_ks<2>(x, row_seq, total_rows, weights, acts_host, n_layers, kernel_size, y, stream);
 }
 
 int conv_stack_bf16x6_tc(
@@ -1039,24 +1076,23 @@ int conv_stack_bf16x6_tc(
     const float* weights, const int32_t* acts_host,
     int32_t n_layers, int32_t channels, int32_t kernel_size, float* y,
     cudaStream_t stream) {
-    if (channels != tc::C || (kernel_size != 3 && kernel_size != 1)) {
+    if (channels != tc::C || !tc_kernel_size(kernel_size)) {
         set_error("emph_conv_stack(bf16x6 tc): channels=%d kernel_size=%d not compiled in",
                   channels, kernel_size);
         return EMPH_ENOSYS;
     }
-    if (kernel_size == 1)
-        return launch_tc<3, 1>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream);
-    return launch_tc<3, 3>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream);
+    return launch_tc_ks<3>(x, row_seq, total_rows, weights, acts_host, n_layers, kernel_size, y, stream);
 }
 
-// The k = 3 tensor-core stack with word pooling fused into the last layer's
-// epilogue (see tc::PoolArgs); y may be null (frame rows are then not written)
+// The tensor-core stack of kernel size 3, 5 or 7 with word pooling fused into
+// the last layer's epilogue (see tc::PoolArgs); y may be null (frame rows are
+// then not written)
 int conv_stack_tc_pool(
     const float* x, const int32_t* row_seq, int32_t total_rows,
     const float* weights, const int32_t* acts_host, int32_t n_layers, int32_t channels,
     int32_t kernel_size, int32_t precision, const int32_t* row_word, int32_t pool_mode,
     long long* fixed, float* out, float* y, cudaStream_t stream) {
-    if (channels != tc::C || kernel_size != 3) {
+    if (channels != tc::C || (kernel_size != 3 && kernel_size != 5 && kernel_size != 7)) {
         set_error("emph_conv_stack_pool: channels=%d kernel_size=%d not compiled in",
                   channels, kernel_size);
         return EMPH_ENOSYS;
@@ -1068,11 +1104,14 @@ int conv_stack_tc_pool(
     }
     const tc::PoolArgs pool{row_word, fixed, out, pool_mode};
     if (precision == EMPH_PREC_BF16_TC)
-        return launch_tc<1, 3>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream, pool);
+        return launch_tc_ks<1>(x, row_seq, total_rows, weights, acts_host, n_layers, kernel_size, y,
+                               stream, pool);
     if (precision == EMPH_PREC_BF16X3_TC)
-        return launch_tc<2, 3>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream, pool);
+        return launch_tc_ks<2>(x, row_seq, total_rows, weights, acts_host, n_layers, kernel_size, y,
+                               stream, pool);
     if (precision == EMPH_PREC_BF16X6_TC)
-        return launch_tc<3, 3>(x, row_seq, total_rows, weights, acts_host, n_layers, y, stream, pool);
+        return launch_tc_ks<3>(x, row_seq, total_rows, weights, acts_host, n_layers, kernel_size, y,
+                               stream, pool);
     set_error("emph_conv_stack_pool: precision %d has no tensor-core kernel", precision);
     return EMPH_ENOSYS;
 }
@@ -1087,7 +1126,7 @@ extern "C" int emph_conv_trace_read(long long* host) {
 
 extern "C" int emph_conv_weights_tc_bytes(
     int32_t n_layers, int32_t channels, int32_t kernel_size, int32_t precision) {
-    if (channels != emph::tc::C || (kernel_size != 3 && kernel_size != 1) || n_layers <= 0) return 0;
+    if (channels != emph::tc::C || !emph::tc_kernel_size(kernel_size) || n_layers <= 0) return 0;
     const int entry = emph::tc::layer_bytes(kernel_size);
     if (precision == EMPH_PREC_BF16X3_TC) return 2 * n_layers * entry;
     if (precision == EMPH_PREC_BF16X6_TC) return 3 * n_layers * entry;
@@ -1098,7 +1137,7 @@ extern "C" int emph_conv_weights_tc_bytes(
 extern "C" int emph_pack_conv_weights_tc(
     const float* weights, const float* bias, int32_t n_layers, int32_t channels,
     int32_t kernel_size, int32_t precision, void* packed, void* stream) {
-    if (channels != emph::tc::C || (kernel_size != 3 && kernel_size != 1)) {
+    if (channels != emph::tc::C || !emph::tc_kernel_size(kernel_size)) {
         emph::set_error("emph_pack_conv_weights_tc: channels=%d kernel_size=%d not compiled in",
                         channels, kernel_size);
         return EMPH_ENOSYS;

@@ -74,7 +74,9 @@ static bool plan_single_chunk(
     plan.chunk_start = (int32_t)lo;
     plan.chunk_len = (int32_t)length;
     plan.n_rows = (int32_t)n_rows;
-    plan.total_rows = (int32_t)n_rows + 2;           // one separator row each side
+    // one separator row each side: enough at kernel sizes 5 and 7 too, since
+    // both conv kernels read rows before 0 and from total_rows on as zeros
+    plan.total_rows = (int32_t)n_rows + 2;
     plan.total_word_rows = n_words + 2;
     plan.word_lo.assign(plan.total_word_rows, 0);
     plan.word_hi.assign(plan.total_word_rows, 0);

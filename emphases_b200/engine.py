@@ -537,7 +537,9 @@ def fuse_pooling(precision):
 
 
 def tensor_core_shape(stack):
-    return stack.channels == KERNEL_CHANNELS and stack.kernel_size in (1, 3)
+    """Conv stacks the tcgen05 kernel is compiled for: 80 channels, kernel
+    size 1, 3, 5 or 7 (128 channels run on the FFMA kernel)"""
+    return stack.channels == KERNEL_CHANNELS and stack.kernel_size in (1, 3, 5, 7)
 
 
 def linear_precision(stack):
@@ -747,7 +749,7 @@ class Engine:
         last = int(stack.acts[-1])
         if (
             precision == _lib.PREC_FP32 or not tensor_core_shape(stack) or
-            stack.kernel_size != 3 or x.shape[1] != stack.channels or
+            stack.kernel_size == 1 or x.shape[1] != stack.channels or
             not (last == _lib.ACT_RELU or (last == _lib.ACT_NONE and method != 'max'))
         ):
             return None

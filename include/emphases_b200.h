@@ -178,7 +178,12 @@ int emph_logmel_resampled_i16(
  *              produced by emph_pack_conv_weights_tc for that precision
  *   bias       [n_layers][channels]
  *   acts       [n_layers] EMPH_ACT_* codes (host pointer)
- *   precision  EMPH_PREC_*
+ *   precision  EMPH_PREC_*: EMPH_PREC_FP32 runs channels 80 and 128 at kernel
+ *              sizes 1 / 3 / 5 / 7; the tensor-core precisions run channels 80
+ *              at kernel sizes 1 / 3 / 5 / 7 (anything else: EMPH_ENOSYS).
+ *              Every precision needs (kernel_size - 1) / 2 * n_layers <= 48:
+ *              the halo of a 128-row tile leaves at least 32 rows (and the
+ *              tensor-core precisions take at most 16 layers)
  */
 int emph_conv_stack(
     const float* x, const int32_t* row_seq, int32_t total_rows,
@@ -204,7 +209,7 @@ int emph_pack_conv_weights_tc(
     int32_t kernel_size, int32_t precision, void* packed, void* stream);
 
 /*
- * emph_conv_stack (tensor-core precisions, channels 80, kernel size 3) with
+ * emph_conv_stack (tensor-core precisions, channels 80, kernel size 3, 5 or 7) with
  * the frame -> word pooling of emph_pool_words fused into the last layer's
  * epilogue: emphases/model/core.py:92-101 (frame_encoder followed by
  * downsample at the 'intermediate' location) in one pass, the frame rows never
