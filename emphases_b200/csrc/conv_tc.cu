@@ -45,6 +45,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace emph {
@@ -52,8 +54,11 @@ namespace emph {
 namespace tc {
 
 #ifdef EXP_TRACE
-// timeline of CTA 0 (tuning builds only): [event][index] clock64 values
-__device__ long long g_trace[8][512];
+// timeline of CTA 0 (tuning builds only): [event][index] clock64 values;
+// events 8 + s: the epilogue group of slot s sees mma_done[s]; 12 .. 16
+// (slot 0, index = round): tile boundary, see tools/conv_trace.py
+constexpr int kTraceEvents = 17;
+__device__ long long g_trace[kTraceEvents][512];
 #define TRACE(ev, idx) do { if (blockIdx.x == 0 && (idx) < 512) g_trace[ev][idx] = clock64(); } while (0)
 #else
 #define TRACE(ev, idx) do {} while (0)
@@ -551,10 +556,12 @@ conv_stack_tc_kernel(
                         *reinterpret_cast<uint2*>(dst + p * ACT_STRIDE) = pk[p][it];
                 }
             }
+            if (tid == 0) TRACE(13, round);
             fence_proxy_async();        // generic-proxy writes -> visible to the tensor core
             tc_fence_before();          // orders the previous round's TMEM reads too
             __syncwarp();
             if (lane == 0) mbar_arrive_rank0(&sm.act_ready[slot]);
+            if (tid == 0) TRACE(16, round);
 
             // pull the next round's tile of this slot into L2 while this one computes
             if (next_tile < n_tiles) {
@@ -577,6 +584,7 @@ conv_stack_tc_kernel(
                 if (tid == 0) TRACE(0, round * n_layers + layer);
                 mbar_wait(&sm.mma_done[slot], done_parity);
                 if (tid == 0) TRACE(1, round * n_layers + layer);
+                if (gtid == 0) TRACE(8 + slot, round * n_layers + layer);
                 done_parity ^= 1;
                 tc_fence_after();
                 if (simple) {
@@ -657,7 +665,9 @@ conv_stack_tc_kernel(
                 // (unconditional -- rows past the end load nothing -- so the
                 // registers are provably dead during the earlier layers)
                 if (simple) fetch_tile(next_tile);
+                if (tid == 0) TRACE(12, round);
                 mbar_wait(&sm.mma_done[slot], done_parity);
+                if (gtid == 0) TRACE(8 + slot, round * n_layers + layer);
                 done_parity ^= 1;
                 tc_fence_after();
                 if (simple) {
@@ -716,7 +726,6 @@ conv_stack_tc_kernel(
                             // values (float4 slot q of row r at q ^ ((r & 7) >> 1):
                             // conflict-free both ways), then lane = (parity, column)
                             // walks its 16 rows and keeps one running value per run
-                            const bool is_sum = pool.mode == kPoolSum;
                             __syncwarp();
 #pragma unroll
                             for (int q = 0; q < 4; ++q)
@@ -724,33 +733,88 @@ conv_stack_tc_kernel(
                                     scratch + lane * 16 + 4 * (q ^ ((lane & 7) >> 1))) =
                                     make_float4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
                             __syncwarp();
-                            const int parity = lane >> 4, column = lane & 15;
-                            float run = 0.f;
+                            if constexpr (PARTS == 1) {
+                                const int parity = lane >> 4, column = lane & 15;
+                                // this lane's 16 values first, so that the run below is
+                                // a chain of adds rather than of shared-memory loads (row
+                                // r = 2k + parity, (r & 7) >> 1 = k & 3)
+                                float v[16];
+#pragma unroll
+                                for (int k = 0; k < 16; ++k)
+                                    v[k] = scratch[(2 * k + parity) * 16 + 4 * ((column >> 2) ^ (k & 3)) +
+                                                   (column & 3)];
+                                const uint32_t my_starts = starts >> parity, my_ends = ends >> parity;
+                                // the loop once per pooling mode: all 16 rows unrolled with
+                                // compile-time bit tests.  This epilogue runs in all four
+                                // slots at once at every tile boundary, while the tensor
+                                // pipe waits for slot 0's next operands, so its
+                                // instruction count is the boundary's length
+                                auto reduce = [&](auto sum_mode) {
+                                    constexpr bool kSum = decltype(sum_mode)::value;
+                                    float run = 0.f;
+#pragma unroll
+                                    for (int k = 0; k < 16; ++k) {
+                                        const bool opens = (my_starts >> (2 * k)) & 1u;
+                                        run = kSum ? (opens ? v[k] : run + v[k])
+                                                   : (opens ? fmaxf(v[k], 0.f) : fmaxf(run, v[k]));
+                                        if ((ends >> (2 * k)) & 3u) {          // warp-uniform
+                                            const int word = __shfl_sync(0xffffffffu, wid, 2 * k + parity);
+                                            if (((my_ends >> (2 * k)) & 1u) && word >= 0) {
+                                                const size_t at = (size_t)word * C + c0 + column;
+                                                if constexpr (kSum) {
+                                                    // <= 16 rows per piece: 2^23 * 2^28 = 2^51,
+                                                    // and 2^12 pieces of it fit int64
+                                                    const float clamped = fminf(
+                                                        fmaxf(run, -16.f * kPoolFixedClamp),
+                                                        16.f * kPoolFixedClamp);
+                                                    atomicAdd(
+                                                        reinterpret_cast<unsigned long long*>(pool.fixed + at),
+                                                        (unsigned long long)__float2ll_rn(
+                                                            clamped * kPoolFixedScale));
+                                                } else {
+                                                    atomicMax(reinterpret_cast<int*>(pool.out + at),
+                                                              __float_as_int(run));
+                                                }
+                                            }
+                                        }
+                                    }
+                                };
+                                if (pool.mode == kPoolSum) reduce(std::true_type{});
+                                else reduce(std::false_type{});
+                            } else {
+                                // the split modes fuse the pooling only on request
+                                // (DESIGN 4.2) and keep the compact loop: the unrolled
+                                // one made their kernels' code larger and the bf16x6
+                                // step slower
+                                const bool is_sum = pool.mode == kPoolSum;
+                                const int parity = lane >> 4, column = lane & 15;
+                                float run = 0.f;
 #pragma unroll 4
-                            for (int k = 0; k < 16; ++k) {
-                                const int r = 2 * k + parity;
-                                const float v = scratch[r * 16 + 4 * ((column >> 2) ^ ((r & 7) >> 1)) +
-                                                        (column & 3)];
-                                const bool opens = (starts >> r) & 1u;
-                                run = is_sum ? (opens ? v : run + v)
-                                             : (opens ? fmaxf(v, 0.f) : fmaxf(run, v));
-                                if ((ends >> (2 * k)) & 3u) {          // warp-uniform
-                                    const int word = __shfl_sync(0xffffffffu, wid, r);
-                                    if (((ends >> r) & 1u) && word >= 0) {
-                                        const size_t at = (size_t)word * C + c0 + column;
-                                        if (is_sum) {
-                                            // <= 16 rows per piece: 2^23 * 2^28 = 2^51, and
-                                            // 2^12 pieces of it fit int64
-                                            const float clamped = fminf(
-                                                fmaxf(run, -16.f * kPoolFixedClamp),
-                                                16.f * kPoolFixedClamp);
-                                            atomicAdd(
-                                                reinterpret_cast<unsigned long long*>(pool.fixed + at),
-                                                (unsigned long long)__float2ll_rn(
-                                                    clamped * kPoolFixedScale));
-                                        } else {
-                                            atomicMax(reinterpret_cast<int*>(pool.out + at),
-                                                      __float_as_int(run));
+                                for (int k = 0; k < 16; ++k) {
+                                    const int r = 2 * k + parity;
+                                    const float v = scratch[r * 16 + 4 * ((column >> 2) ^ ((r & 7) >> 1)) +
+                                                            (column & 3)];
+                                    const bool opens = (starts >> r) & 1u;
+                                    run = is_sum ? (opens ? v : run + v)
+                                                 : (opens ? fmaxf(v, 0.f) : fmaxf(run, v));
+                                    if ((ends >> (2 * k)) & 3u) {          // warp-uniform
+                                        const int word = __shfl_sync(0xffffffffu, wid, r);
+                                        if (((ends >> r) & 1u) && word >= 0) {
+                                            const size_t at = (size_t)word * C + c0 + column;
+                                            if (is_sum) {
+                                                // <= 16 rows per piece: 2^23 * 2^28 = 2^51, and
+                                                // 2^12 pieces of it fit int64
+                                                const float clamped = fminf(
+                                                    fmaxf(run, -16.f * kPoolFixedClamp),
+                                                    16.f * kPoolFixedClamp);
+                                                atomicAdd(
+                                                    reinterpret_cast<unsigned long long*>(pool.fixed + at),
+                                                    (unsigned long long)__float2ll_rn(
+                                                        clamped * kPoolFixedScale));
+                                            } else {
+                                                atomicMax(reinterpret_cast<int*>(pool.out + at),
+                                                          __float_as_int(run));
+                                            }
                                         }
                                     }
                                 }
@@ -767,8 +831,10 @@ conv_stack_tc_kernel(
                     }
                     // the scratch lives in the operand buffer the slot's four warps
                     // fill together for the next tile: nobody stores before all are done
+                    if (tid == 0) TRACE(14, round);
                     if (pool.mode == kPoolSum || pool.mode == kPoolMax)
                         asm volatile("bar.sync %0, 128;" ::"r"(slot + 1) : "memory");
+                    if (tid == 0) TRACE(15, round);
                 } else {
                     epilogue_generic<PARTS, KSIZE>(
                         taddr, act, row, a, valid, true,
@@ -1120,7 +1186,7 @@ int conv_stack_tc_pool(
 
 #ifdef EXP_TRACE
 extern "C" int emph_conv_trace_read(long long* host) {
-    return (int)cudaMemcpyFromSymbol(host, emph::tc::g_trace, sizeof(long long) * 8 * 512);
+    return (int)cudaMemcpyFromSymbol(host, emph::tc::g_trace, sizeof(emph::tc::g_trace));
 }
 #endif
 
