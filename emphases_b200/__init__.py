@@ -108,3 +108,5 @@ from . import model  # noqa: E402,F401
 from . import training  # noqa: E402,F401
 from .scheduler import PackedAudio, pack_audio  # noqa: E402,F401
 from .training import loss  # noqa: E402,F401
+# the training loop; `emphases_b200.train` is the function, as in the reference
+from .train import train  # noqa: E402,F401

@@ -98,6 +98,7 @@ SIGNATURES = {
         _P, _P, _P, _P, _P, _I, _I, _U64, _U32, _F, _P, _P, _P, _P, _P, _P],
     'emph_word_metric_sums': [
         _P, _P, _P, _P, _I, _I, _I, ctypes.c_double, ctypes.c_double, _P, _P],
+    'emph_gather_batch': [_P, _I, _P, _P, _P, _P, _P, _I, _P, _I, _I, _I, _P, _P, _P],
 }
 
 class UtteranceStack(ctypes.Structure):

@@ -50,6 +50,12 @@ UPSAMPLE_METHOD = 'linear'
 BUCKETS = 2
 LOSS = 'bce'
 MAX_TRAINING_FRAMES = 75000
+# Training loop (emphases_b200.train).  The reference's emphases/train/core.py
+# is not in this repository; these are the values SURVEY.md section 2, row 8
+# records for it
+NUM_STEPS = 6000
+EVALUATION_INTERVAL = 100
+LEARNING_RATE = 1e-3
 
 # emphases_b200 extensions (not in the reference)
 # 'bf16x6' (default): tcgen05 tensor-core conv stacks with hi/mid/lo-split bf16

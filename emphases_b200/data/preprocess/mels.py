@@ -1,5 +1,4 @@
 """Mirror of emphases/data/preprocess/mels.py:16-59 (`from_audio`)"""
-import numpy as np
 import torch
 
 import emphases_b200 as emphases
@@ -13,32 +12,11 @@ def from_audio(audio, gpu=None):
     the reference's reflect pad raises (emphases/core.py:413-415 relies on it).
     """
     length = audio.shape[-1]
-    if length <= engine.PADDING:
-        raise RuntimeError(
-            'Padding size should be less than the corresponding input '
-            f'dimension, but got: padding ({engine.PADDING}, {engine.PADDING}) '
-            f'at dimension 1 of input of length {length}')
+    plan = engine.feature_plan([length])
     device = emphases.resolve_device(gpu, audio)
     eng = emphases.get_engine(device)
     with torch.cuda.device(device):
         frames = length // emphases.HOPSIZE
-        # A chunk that is its own utterance: surround it with the 432 zeros
-        # the chunk slice would see, i.e. chunk_start = 432 in padded coords
-        plan = engine.Plan(
-            n_seq=1, total_rows=frames + 2, total_word_rows=1,
-            utterance=np.zeros(1, np.int64), word_first=np.zeros(1, np.int64),
-            audio_off=np.zeros(1, np.int64),
-            audio_len=np.array([length], np.int32),
-            chunk_start=np.array([engine.PADDING], np.int32),
-            chunk_len=np.array([length], np.int32),
-            row_start=np.array([1], np.int32),
-            n_rows=np.array([frames], np.int32),
-            word_row_start=np.zeros(0, np.int32), n_words=np.zeros(0, np.int32),
-            word_seq=np.full(1, -1, np.int32), word_lo=np.zeros(1, np.int32),
-            word_hi=np.zeros(1, np.int32), audio_samples=length,
-            audio_offsets=np.zeros(1, np.int64))
-        plan.word_row_start = np.array([1], np.int32)
-        plan.n_words = np.array([0], np.int32)
         samples = audio[0].detach().to(device, torch.float32).contiguous()
         views = eng.upload_plan(plan)
         row_seq = eng.row_index(

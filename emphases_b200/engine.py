@@ -368,6 +368,47 @@ def _assemble_plan(
         audio_offsets=np.asarray(offsets, dtype=np.int64))
 
 
+def feature_plan(lengths, names=None):
+    """Plan of the training framing (emphases/data/preprocess/mels.py
+    `from_audio` on whole files): every file is one chunk that is its own
+    utterance, reflect-padded by 432 at its own edges, T = L // 160 frames.
+    In zero-padded coordinates that is chunk_start = 432, chunk_len = L.
+    Files are packed at AUDIO_ALIGN offsets (scheduler.PackedAudio.layout),
+    frame rows one separator row apart.  Only the log-mel fields are filled:
+    the plan has no words.
+
+    Raises RuntimeError, naming names[i] when given, for a file of <= 432
+    samples, where the reference's reflect pad raises."""
+    lengths = np.asarray(lengths, dtype=np.int64).reshape(-1)
+    short = np.nonzero(lengths <= PADDING)[0]
+    if len(short):
+        i = int(short[0])
+        where = f'{names[i]}: ' if names is not None else ''
+        raise RuntimeError(
+            f'{where}Padding size should be less than the corresponding input '
+            f'dimension, but got: padding ({PADDING}, {PADDING}) '
+            f'at dimension 1 of input of length {int(lengths[i])}')
+    n = len(lengths)
+    aligned = align_samples(lengths)
+    offsets = np.concatenate([[0], np.cumsum(aligned[:-1])]).astype(np.int64) \
+        if n else np.zeros(0, dtype=np.int64)
+    n_rows = lengths // HOPSIZE
+    row_start, total_rows = packed_starts(n_rows, gap=1)
+    if total_rows >= 2 ** 31:
+        raise ValueError('corpus too large for one log-mel launch')
+    return Plan(
+        n_seq=n, total_rows=total_rows, total_word_rows=1,
+        utterance=np.arange(n, dtype=np.int64), word_first=np.zeros(n, np.int64),
+        audio_off=offsets, audio_len=lengths.astype(np.int32),
+        chunk_start=np.full(n, PADDING, np.int32),
+        chunk_len=lengths.astype(np.int32),
+        row_start=row_start.astype(np.int32), n_rows=n_rows.astype(np.int32),
+        word_row_start=np.ones(n, np.int32), n_words=np.zeros(n, np.int32),
+        word_seq=np.full(1, -1, np.int32), word_lo=np.zeros(1, np.int32),
+        word_hi=np.zeros(1, np.int32),
+        audio_samples=max(int(aligned.sum()), AUDIO_ALIGN), audio_offsets=offsets)
+
+
 def validate_bounds(bounds, frames, method):
     """Raise where the reference raises (SURVEY.md A.4, torch indexing)"""
     lo = np.minimum(np.maximum(bounds[:, 0], 0), frames)
@@ -788,6 +829,23 @@ class Engine:
             _lib.ptr(word_hi), total_word_rows, _lib.POOL[method], _lib.ptr(y),
             _lib.stream_ptr())
         return y
+
+    def gather_batch(self, rows, row_start, n_rows, word_targets, word_start,
+                     n_words, items, tmax, wmax, ws=None):
+        """Padded (B, C, Tmax) features and (B, 1, Wmax) targets of corpus
+        items `items` (int32 device tensor) from resident packed frame rows and
+        word targets (emph_gather_batch)"""
+        batch, channels = items.numel(), rows.shape[1]
+        features = _empty(
+            ws, 'batch_features', (batch, channels, tmax), torch.float32, self.device)
+        targets = _empty(
+            ws, 'batch_targets', (batch, 1, wmax), torch.float32, self.device)
+        _lib.call(
+            'emph_gather_batch', _lib.ptr(rows), channels, _lib.ptr(row_start),
+            _lib.ptr(n_rows), _lib.ptr(word_targets), _lib.ptr(word_start),
+            _lib.ptr(n_words), row_start.numel(), _lib.ptr(items), batch, tmax,
+            wmax, _lib.ptr(features), _lib.ptr(targets), _lib.stream_ptr())
+        return features, targets
 
     def head(self, x, row_seq, weights: ModelWeights, mode, want_logits=True,
              want_scores=True, ws=None):

@@ -740,6 +740,30 @@ int emph_word_metric_sums(
     double* sums, void* stream);
 
 /*
+ * On-device collate of a training batch from a resident corpus
+ * (emphases/data/collate.py:11-77, features and targets):
+ *   rows            [*][channels] fp32 frame rows in the packed row layout
+ *                   (item i owns rows row_start[i] .. + n_rows[i])
+ *   word_targets    fp32 per-word targets, packed (item i owns word_start[i]
+ *                   .. + n_words[i])
+ *   items           DEVICE array of the batch's `batch` corpus indices
+ *                   (0 .. n_items - 1; an index outside that range yields an
+ *                   all-zero item)
+ *   features        (batch, channels, tmax): features[b][c][t] =
+ *                   rows[row_start[items[b]] + t][c] for t < n_rows, else 0
+ *   targets         (batch, 1, wmax): the item's targets, 0 for w >= n_words
+ * One launch; every output element is written (no memset needed).  The
+ * transpose runs through 32 x 32 shared-memory tiles, so loads along channels
+ * and stores along time are both coalesced.
+ */
+int emph_gather_batch(
+    const float* rows, int32_t channels,
+    const int32_t* row_start, const int32_t* n_rows,
+    const float* word_targets, const int32_t* word_start, const int32_t* n_words,
+    int32_t n_items, const int32_t* items, int32_t batch, int32_t tmax, int32_t wmax,
+    float* features, float* targets, void* stream);
+
+/*
  * Polyphase windowed-sinc resampling (emphases/core.py:613-619 `resample`, which
  * is torchaudio.transforms.Resample): y[q * new + p] = sum_k kernel[p][k] *
  * xpad[q * orig + k], xpad = zeros(width) ++ x ++ zeros(width + orig).
